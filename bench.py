@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: top-k queries/sec of the retrieval hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload at every N: BASELINE.json configs[1] — batched IR evaluation, 10,000 queries against the
 49,688 x 384 fp32 catalog, top-100 (one "step" = one pass over one 10,000-query batch). With N > 1 every
@@ -159,7 +159,8 @@ def run_reference(args, rank: int):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline, e2e and kernel-timing loops; the sharded, c1, c3 and ir_eval objects keep their own fixed counts")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--dtype", default="f32", choices=["f32", "bf16"], help="catalog storage dtype (headline: f32, the reference's)")
@@ -167,7 +168,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sharded", action="store_true", help="skip the row-sharded strong-scaling object (configs 4 and 5)")
     ap.add_argument("--no-side", action="store_true", help="skip the c1 / c3 / ir_eval side objects")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's result of the last timed step of the headline path (DeviceCatalog.topk on the seeded C2 inputs) "
+                         "as DIR/topk_values.npy (float32 [Q, k]) and DIR/topk_ids.npy (float64 [Q, k]), to compare two builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -245,15 +251,16 @@ def main():
         barrier()
         for s in range(steps):
             flush.zero_()  # evict L2 between timed iterations (not timed)
+            out = None  # the previous step's result is freed before the next one allocates, as when no result is kept
             starts[s].record()
-            fn()
+            out = fn()
             stops[s].record()
         barrier()
         ms = [a.elapsed_time(b) for a, b in zip(starts, stops)]
         total = torch.tensor([sum(ms)], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(total, op=dist.ReduceOp.MAX)
-        return total.item(), ms
+        return total.item(), ms, out
 
     def timed_in_flight(steps, depth=3):
         """Host-to-host batches kept in flight: the upload of batch s+1 overlaps the kernels of batch s and the download of batch
@@ -287,14 +294,22 @@ def main():
         step_device()
     launches_per_step = ops.last_launch_count()
     with ClockSampler(local_rank) as clocks:  # spans every timed region below
-        total_ms, per_step = timed(step_device, args.steps)
+        total_ms, per_step, last_out = timed(step_device, args.steps)
         for _ in range(3):
             step_e2e()
-        e2e_sync_ms, _ = timed(step_e2e, args.steps)
+        e2e_sync_ms, _, _ = timed(step_e2e, args.steps)
         timed_in_flight(min(args.steps, 4))
         e2e_ms = timed_in_flight(args.steps)
         # ---- dominant kernel alone (CUDA events recorded by the library around that kernel's launches) ---------
         kt = ops.kernel_timing(step_device, args.steps, flush=flush)
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        values, ids = last_out
+        np.save(out_dir / "topk_values.npy", values.float().cpu().numpy())
+        np.save(out_dir / "topk_ids.npy", ids.double().cpu().numpy())  # float64 holds every row id exactly
     peaks = _peaks()
     flops = 2.0 * Q * N * D
     if kt["kernel"] == "gemm_topk":
