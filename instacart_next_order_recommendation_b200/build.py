@@ -18,7 +18,7 @@ NVCC_FLAGS = [
     "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC",
     "--expt-relaxed-constexpr",
-] + os.environ.get("ICR_NVCC_DEFS", "").split()  # e.g. ICR_NVCC_DEFS="-DICR_EPI_WARPS=4" for tuning experiments
+] + os.environ.get("ICR_NVCC_DEFS", "").split()  # e.g. ICR_NVCC_DEFS="-DICR_HS_WARPS=6" for tuning experiments
 
 
 def _nvcc() -> str:

@@ -20,17 +20,19 @@
 //    (select.cu) folds the survivors into the running top-k and publishes the new tau. If a thread's
 //    candidate segment fills up anyway (adversarially ordered catalogs), its warp sorts the segment in
 //    shared memory, keeps the k best and raises that thread's tau: exact for any input.
-//  * fp32 catalogs keep fp32 parity on fp16 tensor cores: rows are L2-normalised, scaled by 2^8 and split
-//    into fp16 hi + lo planes (prep.cu); hi*hi + hi*lo + lo*hi accumulated in fp32 reproduces the fp32 dot
-//    product to ~1e-6 relative (profiles/r01_split_precision.txt). Each pipeline stage holds the four
-//    plane tiles of one 64-wide K block, so no plane is fetched twice. bf16 catalogs take one MMA term on
-//    the raw rows and multiply by the two inverse norms in the epilogue.
+//  * fp32 catalogs are swept with ONE MMA term on fp16 screening planes: rows are L2-normalised, scaled by 2^8 and
+//    rounded to fp16 (prep.cu). Screened scores are within a known band of the exact ones (select_args.cuh), so the
+//    thresholds sit that band below the k-th best, and the last select re-scores the rows inside it exactly in fp32
+//    (rescore_rank_kernel). bf16 catalogs take one MMA term on the raw rows and multiply by the two inverse norms in
+//    the epilogue.
+//  * The dense K2' path (DENSE, icr_cos_sim_dense) keeps fp32 parity for fp32 inputs: rows are split into fp16
+//    hi + lo planes, and hi*hi + hi*lo + lo*hi accumulated in fp32 reproduces the fp32 dot product to ~1e-6 relative
+//    (profiles/r01_split_precision.txt). Each pipeline stage holds the four plane tiles of one 64-wide K block, so no
+//    plane is fetched twice.
 //
 // Replaces cos_sim [Q,N] -> torch.topk(100) -> Python heap of sentence-transformers'
 // InformationRetrievalEvaluator (built at reference src/training/train_sbert.py:197-202) and the
 // cos_sim -> np.argsort loops of src/baselines/content_based.py:54-63.
-#include <cstdio>
-
 #include "select_args.cuh"
 #include "select_lean.cuh"
 #include "select_finish.cuh"
@@ -42,12 +44,6 @@ constexpr int kRingBytes = 192 * 1024;
 constexpr int kSegCapMax = 512;      // candidate keys per (query, chunk, column half) segment: 256 for k <= 128, else 512
 // warp 0 TMA, warp 1 MMA, warp 2 TMEM alloc, warp 3 idle, warps 4.. epilogue. With 8 epilogue warps (two per
 // scheduler) warps 4-7 filter accumulator columns 0-127 and warps 8-11 columns 128-255 of the same 128 queries.
-// Measured (profiles/r01_notes.md): once scores are screened 8 at a time (filter32) four warps are enough and
-// leave the MMA-issuing and TMA threads more issue slots: C5 shard 1039 vs 929 TFLOP/s, C4 Q=1024 1373 vs 1232;
-// eight warps only win where survivors are dense (C2 bf16: 694 vs 610). Default 4.
-#ifndef ICR_EPI_WARPS
-#define ICR_EPI_WARPS 4
-#endif
 // Epilogue warps per CTA, in sets of four (a warp may only read the TMEM lane quarter warp_id % 4); with two sets each
 // filters half of a tile's columns. Measured (profiles/r01_notes.md): the three-term kernel is tensor-bound and does
 // best with four (fewer segments for the select); the one-term kernels are epilogue-latency-bound and want two warps
@@ -309,7 +305,7 @@ __device__ __forceinline__ void k2_grid_barrier(unsigned int* counter, unsigned 
   asm volatile("bar.sync 2, %0;" ::"r"(ewarps * 32) : "memory");
 }
 
-// MODE = 3: fp16 hi/lo planes, three MMA terms (fp32 parity of every score: the dense K2' path);
+// MODE = 3: fp16 hi/lo planes, three MMA terms (fp32 parity of every score): instantiated for the dense K2' path only;
 // MODE = 1: raw bf16 rows, one term, inverse norms applied in the epilogue;
 // MODE = 2: one fp16 plane of the normalised fp32 rows, one term: SCREENING scores (select_args.cuh), the survivors
 //           of the whole sweep are re-scored exactly by the last select.
@@ -893,19 +889,17 @@ template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kSwapThreads, 1)
 gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant__ CUtensorMap tma_c, const GemmArgs g,
                  const __grid_constant__ HistSelectArgs sel) {
-  constexpr int TERMS = (MODE == 3) ? 3 : 1;
   constexpr bool BF16 = (MODE == 1);
-  constexpr int CT = (TERMS == 3) ? 2 : 1;  // catalog tiles per stage: hi | lo plane
-  constexpr int kStageBytes = CT * kTileBytes;
+  constexpr int kStageBytes = kTileBytes;
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   const int KB = g.kb_per_term;
   const int QH = g.qpad >> 1;              // query rows held by each CTA of the pair
   const int qtile_bytes = QH * 128;        // one 64-element K block of them (multiple of 2 KB)
-  const int res_bytes = CT * KB * qtile_bytes;
+  const int res_bytes = KB * qtile_bytes;
   int stages = (kRingBytes - res_bytes) / kStageBytes;
   if (stages > kSwapMaxStages) stages = kSwapMaxStages;
-  unsigned char* q_res = smem;  // block (plane * KB + kb) at q_res + block * qtile_bytes
+  unsigned char* q_res = smem;  // K block kb at q_res + kb * qtile_bytes
   unsigned char* stage_base = smem + res_bytes;
   float* tau_s = reinterpret_cast<float*>(smem + kRingBytes);  // [256] per-query thresholds (raw units)
   int* cnt_s = reinterpret_cast<int*>(tau_s + 256);             // [256] keys in this CTA's segment of each query
@@ -949,9 +943,8 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
     // ================= TMA producer =================
     const uint32_t qb = smem_u32(qfull_bar);
     if (rank == 0) mbar_expect_tx(qb, 2 * res_bytes);
-    for (int pl = 0; pl < CT; ++pl)
-      for (int kb = 0; kb < KB; ++kb)
-        tma_load_2d_pair(smem_u32(q_res + (pl * KB + kb) * qtile_bytes), &tma_q, pl * g.plane_stride + kb * BK, static_cast<int>(rank) * QH, qb);
+    for (int kb = 0; kb < KB; ++kb)
+      tma_load_2d_pair(smem_u32(q_res + kb * qtile_bytes), &tma_q, kb * BK, static_cast<int>(rank) * QH, qb);
     int stage = 0;
     uint32_t phase = 0;
     for (int w = pair; w < items; w += npairs) {
@@ -965,7 +958,6 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
           if (rank == 0) mbar_expect_tx(fb, 2 * kStageBytes);
           const uint32_t sa = smem_u32(stage_base + stage * kStageBytes);
           tma_load_2d_pair(sa, &tma_c, kb * BK, crow, fb);
-          if (TERMS == 3) tma_load_2d_pair(sa + kTileBytes, &tma_c, g.plane_stride + kb * BK, crow, fb);
           if (++stage == stages) {
             stage = 0;
             phase ^= 1;
@@ -979,7 +971,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
     const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (static_cast<uint32_t>(g.qpad >> 3) << 17) | (static_cast<uint32_t>(BN >> 4) << 24);
     const uint64_t qd0 = smem_desc_sw128(smem_u32(q_res));
     const uint64_t cd0 = smem_desc_sw128(smem_u32(stage_base));
-    constexpr uint64_t kTileUnits = kTileBytes >> 4, kStageUnits = kStageBytes >> 4;
+    constexpr uint64_t kStageUnits = kStageBytes >> 4;
     const uint64_t qunits = static_cast<uint64_t>(qtile_bytes >> 4);
     mbar_wait(smem_u32(qfull_bar), 0);
     tc_fence_after();
@@ -996,18 +988,13 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
         for (int kb = 0; kb < KB; ++kb) {
           mbar_wait(smem_u32(&full_bar[stage]), phase);
           tc_fence_after();
-          const uint64_t c_hi = cd0 + static_cast<uint64_t>(stage) * kStageUnits;
-          const uint64_t q_hi = qd0 + static_cast<uint64_t>(kb) * qunits;
+          const uint64_t cdesc = cd0 + static_cast<uint64_t>(stage) * kStageUnits;
+          const uint64_t qdesc = qd0 + static_cast<uint64_t>(kb) * qunits;
           if (elect_one()) {
 #pragma unroll
             for (int k4 = 0; k4 < BK / 16; ++k4) {
               const uint64_t o = static_cast<uint64_t>(k4 * 2);
-              umma_f16_pair(d_tmem, c_hi + o, q_hi + o, idesc, (kb | k4) != 0 ? 1u : 0u);
-              if (TERMS == 3) {
-                const uint64_t c_lo = c_hi + kTileUnits, q_lo = q_hi + static_cast<uint64_t>(KB) * qunits;
-                umma_f16_pair(d_tmem, c_hi + o, q_lo + o, idesc, 1u);
-                umma_f16_pair(d_tmem, c_lo + o, q_hi + o, idesc, 1u);
-              }
+              umma_f16_pair(d_tmem, cdesc + o, qdesc + o, idesc, (kb | k4) != 0 ? 1u : 0u);
             }
             umma_commit_pair(smem_u32(&empty_bar[stage]));
             if (kb == KB - 1) umma_commit_pair(smem_u32(&tfull_bar[acc]));
@@ -1222,14 +1209,8 @@ static_assert(kGemmSmemBytes <= 232448, "exceeds the 227 KB of shared memory a C
 constexpr size_t kSwapSmemBytes = static_cast<size_t>(kRingBytes) + 2 * 256 * 4 + 16 + (2 * kSwapMaxStages + 6) * sizeof(uint64_t) + 16 + kSwapBootBytes + 1024;
 static_assert(kSwapSmemBytes <= 232448, "exceeds the 227 KB of shared memory a CTA may use");
 
-// the swapped kernel applies when one block of queries is small enough to stay resident next to a useful ring
-// fp32 catalogs: MODE 2 (one-term screening + exact re-scoring of the survivors) unless ICR_F32_EXACT3 asks for the
-// round-1 path (three MMA terms on hi|lo planes built per call) - kept as an A/B switch for benchmarks and tests
-static bool f32_exact3() {
-  static const bool on = getenv("ICR_F32_EXACT3") != nullptr;
-  return on;
-}
-static int mode_for(int dtype) { return dtype == ICR_BF16 ? 1 : (f32_exact3() ? 3 : 2); }
+// top-k path: MODE 1 on bf16 catalogs, MODE 2 (one-term screening + exact re-scoring of the survivors) on fp32 ones
+static int mode_for(int dtype) { return dtype == ICR_BF16 ? 1 : 2; }
 // keys carried per query between phases: k exact keys, or k + room for the screening band (select_args.cuh)
 static int carry_cap(int k, int mode) {
   if (mode != 2) return k;
@@ -1237,13 +1218,13 @@ static int carry_cap(int k, int mode) {
   return kc < 512 ? kc : 512;
 }
 
-static bool swap_applies(int64_t Q, int64_t N, int64_t D, int dtype) {
-  static const bool disabled = getenv("ICR_NO_SWAP") != nullptr;  // A/B switch for benchmarks
-  if (disabled || Q > 256) return false;
+// the swapped kernel applies when one block of queries is small enough to stay resident next to a useful ring
+static bool swap_applies(int64_t Q, int64_t N, int64_t D) {
+  if (Q > 256) return false;
   const int64_t qpad = (Q + 31) / 32 * 32;
   const int64_t kb = (D + BK - 1) / BK;
-  const int64_t res = (mode_for(dtype) == 3 ? 2 : 1) * kb * (qpad / 2) * 128;
-  const int64_t sweep_bytes = N * ((D + BK - 1) / BK * BK) * 2 * (mode_for(dtype) == 3 ? 2 : 1);
+  const int64_t res = kb * (qpad / 2) * 128;
+  const int64_t sweep_bytes = N * ((D + BK - 1) / BK * BK) * 2;
   return res <= (sweep_bytes <= kSmallCatalogBytes ? kSwapResidentMaxSmallCatalog : kSwapResidentMax);
 }
 
@@ -1255,20 +1236,18 @@ struct Phase {
 // so a phase that multiplies the rows seen by g admits ~k*ln(g) (at most ~k*(g-1)) survivors per query.
 // swapped kernel: its epilogue work is small (128 x Q scores per tile), so it affords denser survivors in exchange
 // for fewer phases - every phase costs a launch of the GEMM and of the select (~25 us for a small batch)
+constexpr int kSwapGrowth = 32;
+constexpr int kK2First = 4, kSwapFirst = 8;  // tiles of the first phase, at least
 static int plan_phases(int64_t N, int qblocks, int k, Phase* out, int max_phases, bool swap, int begin0 = 0) {
   const int T = static_cast<int>((N + BN - 1) / BN);
-  static const int swap_growth = getenv("ICR_SWAP_GROWTH") ? atoi(getenv("ICR_SWAP_GROWTH")) : 32;  // tuning hook
-  // tuning hook; default 8, or 32 for ONE query block on a catalog that streams from HBM: there every phase costs ~35-45 us of
-  // small GEMM + select beside a stream of a few hundred us, and 3 sparse phases beat 4 (profiles/r02_c4_phase_sweep.txt)
-  static const int k2_growth_env = getenv("ICR_K2_GROWTH") ? atoi(getenv("ICR_K2_GROWTH")) : 0;
-  const int k2_growth = k2_growth_env > 0 ? k2_growth_env : ((qblocks == 1 && T >= 2048) ? 32 : 8);
-  const int growth = swap ? swap_growth : k2_growth;
+  // K2: 8, or 32 for ONE query block on a catalog that streams from HBM: there every phase costs ~35-45 us of small
+  // GEMM + select beside a stream of a few hundred us, and 3 sparse phases beat 4 (profiles/r02_c4_phase_sweep.txt)
+  const int k2_growth = (qblocks == 1 && T >= 2048) ? 32 : 8;
+  const int growth = swap ? kSwapGrowth : k2_growth;
   const int npairs = kNumSMs / 2;
-  static const int k2_first = getenv("ICR_K2_FIRST") ? atoi(getenv("ICR_K2_FIRST")) : 4;  // tuning hook
   int first = (2 * k + BN - 1) / BN;
-  if (first < k2_first) first = k2_first;
-  static const int swap_first = getenv("ICR_SWAP_FIRST") ? atoi(getenv("ICR_SWAP_FIRST")) : 8;  // tuning hook
-  if (swap && first < swap_first) first = swap_first;
+  if (first < kK2First) first = kK2First;
+  if (swap && first < kSwapFirst) first = kSwapFirst;
   int n = 0, begin = 0, end = first < T ? first : T;
   if (begin0 > 0) {  // rows of tiles [0, begin0) were scored densely: the sparse phases start behind them
     begin = begin0;
@@ -1311,22 +1290,14 @@ static int plan_phases(int64_t N, int qblocks, int k, Phase* out, int max_phases
 }
 
 constexpr int kMaxPhases = 16;
-// rows 0..1023 (4 tiles) are scored densely in the first phase of the (non-swapped) top-k path; ICR_K2_DENSE0 / ICR_K2_GROWTH:
-// tuning hooks (profiles/r01_notes.md)
-static const int kDense0Env = getenv("ICR_K2_DENSE0") ? atoi(getenv("ICR_K2_DENSE0")) : 0;
+// Rows of the first tiles are scored densely in the first phase of the (non-swapped) top-k path (profiles/r01_notes.md):
 // 4 tiles, or 16 for one query block on a catalog that streams from HBM (one sparse phase less, see plan_phases)
-static int dense0_tiles(int64_t Q, int64_t N) {
-  if (kDense0Env > 0) return kDense0Env;
-  return (Q <= 2 * BM && (N + BN - 1) / BN >= 2048) ? 16 : 4;
-}
+static int dense0_tiles(int64_t Q, int64_t N) { return (Q <= 2 * BM && (N + BN - 1) / BN >= 2048) ? 16 : 4; }
 
-// kernel variants: 0 = fp16 hi|lo planes (3 terms), 1 = bf16 streaming both operands, 2 = bf16 with resident queries,
-// 3 / 4 = swapped kernel (small batches) on planes / bf16, 5 / 6 = fp16 screen plane streaming / resident queries,
-// 7 = swapped kernel on the screen plane
-static int variant_terms(int which) { return (which == 0 || which == 3) ? 3 : 1; }
-
+// kernel variants: 1 = bf16 streaming both operands, 2 = bf16 with resident queries, 5 / 6 = fp16 screen plane streaming /
+// resident queries, 4 / 7 = swapped kernel (small batches) on bf16 / the screen plane; DENSE only: 0 = fp16 hi|lo planes,
+// three MMA terms (K2' on fp32 inputs)
 #define ICR_GEMM_VARIANTS(X, DENSE)            \
-  X(0, (gemm_topk_kernel<3, false, DENSE>))    \
   X(1, (gemm_topk_kernel<1, false, DENSE>))    \
   X(2, (gemm_topk_kernel<1, true, DENSE>))     \
   X(5, (gemm_topk_kernel<2, false, DENSE>))    \
@@ -1338,9 +1309,8 @@ static int variant_terms(int which) { return (which == 0 || which == 3) ? 3 : 1;
 // refuses the attribute on a cluster kernel gets the plain launch (the grid is sized to one CTA per SM either way).
 template <typename... KArgs, typename... Args>
 static void launch_gemm_grid(void (*kernel)(KArgs...), int grid, int threads, size_t smem, cudaStream_t st, bool coop, Args&&... args) {
-  static const bool no_coop = getenv("ICR_NO_COOP") != nullptr;  // A/B switch for benchmarks
   static thread_local bool refused = false;
-  if (coop && !no_coop && !refused) {
+  if (coop && !refused) {
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(static_cast<unsigned>(grid));
     cfg.blockDim = dim3(static_cast<unsigned>(threads));
@@ -1358,7 +1328,6 @@ static void launch_gemm_grid(void (*kernel)(KArgs...), int grid, int threads, si
       return;  // left for ICR_LAUNCH_CHECK
     (void)cudaGetLastError();
     if (e != cudaErrorCooperativeLaunchTooLarge) refused = true;
-    if (getenv("ICR_DEBUG_COOP")) fprintf(stderr, "icr: cooperative launch refused (%s), plain launch used\n", cudaGetErrorName(e));
   }
   kernel<<<grid, threads, smem, st>>>(KArgs(args)...);
 }
@@ -1371,13 +1340,16 @@ static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, co
 #define ICR_SET(ID, K) \
   if (which == ID) rc = ensure_dyn_smem(cache[ID], K, kGemmSmemBytes);
   ICR_GEMM_VARIANTS(ICR_SET, DENSE)
+  if constexpr (DENSE) ICR_SET(0, (gemm_topk_kernel<3, false, true>))
 #undef ICR_SET
   if (rc) return rc;
-  profile_begin(kKernelGemm, variant_terms(which), st);
-  const int threads = 128 + epi_warps(variant_terms(which)) * 32;
+  const int terms = which == 0 ? 3 : 1;
+  profile_begin(kKernelGemm, terms, st);
+  const int threads = 128 + epi_warps(terms) * 32;
 #define ICR_RUN(ID, K) \
   if (which == ID) launch_gemm_grid(K, grid, threads, kGemmSmemBytes, st, g.boot > 0, map_a, map_b, g);
   ICR_GEMM_VARIANTS(ICR_RUN, DENSE)
+  if constexpr (DENSE) ICR_RUN(0, (gemm_topk_kernel<3, false, true>))
 #undef ICR_RUN
   profile_end(st);
   ICR_LAUNCH_CHECK();
@@ -1386,24 +1358,17 @@ static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, co
 
 static int launch_swap_variant(int which, int grid, const CUtensorMap& map_q, const CUtensorMap& map_c, const GemmArgs& g, cudaStream_t st,
                                const HistSelectArgs& sel = HistSelectArgs{}) {
-  static thread_local SmemAttrCache cache[3];
+  static thread_local SmemAttrCache cache[2];
   int rc = ICR_OK;
-  if (which == 3) rc = ensure_dyn_smem(cache[0], gemm_swap_kernel<3>, kSwapSmemBytes);
-  if (which == 4) rc = ensure_dyn_smem(cache[1], gemm_swap_kernel<1>, kSwapSmemBytes);
-  if (which == 7) rc = ensure_dyn_smem(cache[2], gemm_swap_kernel<2>, kSwapSmemBytes);
+  if (which == 4) rc = ensure_dyn_smem(cache[0], gemm_swap_kernel<1>, kSwapSmemBytes);
+  if (which == 7) rc = ensure_dyn_smem(cache[1], gemm_swap_kernel<2>, kSwapSmemBytes);
   if (rc) return rc;
-  profile_begin(kKernelGemm, variant_terms(which), st);
-  if (which == 3) launch_gemm_grid(gemm_swap_kernel<3>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
+  profile_begin(kKernelGemm, 1, st);
   if (which == 4) launch_gemm_grid(gemm_swap_kernel<1>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
   if (which == 7) launch_gemm_grid(gemm_swap_kernel<2>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
   profile_end(st);
   ICR_LAUNCH_CHECK();
   return ICR_OK;
-}
-
-static bool dense0_applies(int64_t Q, int64_t N, int64_t D, int dtype) {
-  static const bool disabled = getenv("ICR_NO_DENSE0") != nullptr;  // A/B switch for benchmarks
-  return !disabled && !swap_applies(Q, N, D, dtype);
 }
 
 struct GemmWs {
@@ -1417,19 +1382,18 @@ struct GemmWs {
 
 // Single-launch mode of K2: one phase over the whole catalog, `chunks` tile ranges per query block, the first `tiles` tiles of
 // every work item scored twice (once for the block maxima the thresholds come from). The bootstrap rows are chosen so that
-// ~ICR_K2_BOOT_TARGET keys per query pass the threshold (N * k / rows); the mode needs 2k..kK2BootCap block maxima per query and
+// ~kK2BootTarget keys per query pass the threshold (N * k / rows); the mode needs 2k..kK2BootCap block maxima per query and
 // re-streams at most a quarter of a chunk - i.e. it serves catalogs of up to a few hundred thousand rows, where the phased
 // path spends a third of its time on the two bootstrap phases and their selects; larger catalogs keep the phased path.
-static int k2_boot_plan(int64_t Q, int64_t N, int64_t D, int dtype, int k, int* chunks_out, int* coarse_out = nullptr) {
+constexpr int kK2BootTarget = 550;  // profiles/r02_k2_boot_target_sweep_*.txt
+static int k2_boot_plan(int64_t Q, int64_t N, int64_t D, int k, int* chunks_out, int* coarse_out = nullptr) {
   if (coarse_out) *coarse_out = 0;
-  static const bool disabled = getenv("ICR_NO_BOOT_K2") != nullptr;  // A/B switch for benchmarks
-  static const int target = getenv("ICR_K2_BOOT_TARGET") ? atoi(getenv("ICR_K2_BOOT_TARGET")) : 550;
-  if (disabled || mode_for(dtype) == 3 || swap_applies(Q, N, D, dtype)) return 0;
+  if (swap_applies(Q, N, D)) return 0;
   const int T = static_cast<int>((N + BN - 1) / BN);
   const int qblocks = static_cast<int>((Q + 2 * BM - 1) / (2 * BM));
   const int npairs = kNumSMs / 2;
   int c0 = (2 * npairs + qblocks - 1) / qblocks;
-  const int by_load = (target + 71) / 72;  // survivors spread over 2 * chunks segments, kept under a quarter of their capacity
+  const int by_load = (kK2BootTarget + 71) / 72;  // survivors spread over 2 * chunks segments, kept under a quarter of their capacity
   if (c0 < by_load) c0 = by_load;
   if (c0 > T) c0 = T;
   int best = c0;
@@ -1442,7 +1406,7 @@ static int k2_boot_plan(int64_t Q, int64_t N, int64_t D, int dtype, int k, int* 
       best = c;
     }
   }
-  const int64_t want_rows = N * k / (target > 0 ? target : 1);
+  const int64_t want_rows = N * k / kK2BootTarget;
   int tiles = static_cast<int>((want_rows + static_cast<int64_t>(BN) * best - 1) / (static_cast<int64_t>(BN) * best));
   if (tiles < 1) tiles = 1;
   while (best * tiles * (BN / 32) < 2 * k) ++tiles;
@@ -1455,8 +1419,7 @@ static int k2_boot_plan(int64_t Q, int64_t N, int64_t D, int dtype, int k, int* 
     const int qblocks1 = static_cast<int>((Q + 2 * BM - 1) / (2 * BM));
     int ct = kK2BootCap / (best * eh);
     if (ct > tiles) ct = tiles;
-    static const bool no_coarse = getenv("ICR_NO_BOOT_COARSE") != nullptr;  // A/B switch for benchmarks
-    if (no_coarse || qblocks1 != 1 || T < 2048 || mode_for(dtype) == 3 || ct < 1 || best * ct * eh < 2 * k) return 0;
+    if (qblocks1 != 1 || T < 2048 || ct < 1 || best * ct * eh < 2 * k) return 0;
     if (static_cast<double>(N) * k / (static_cast<double>(BN) * best * ct) > 2500.0) return 0;  // survivors per query the segments and the select take in their stride
     if (ct * 4 > T / best) return 0;
     if (coarse_out) *coarse_out = 1;
@@ -1477,9 +1440,8 @@ static int k2_boot_plan(int64_t Q, int64_t N, int64_t D, int dtype, int k, int* 
 // The bootstrap threshold lets ~N * k / (rows scored in the bootstrap) keys per query through: the number of bootstrap tiles per
 // chunk is chosen so that this stays near 4,000 (cheap for the select, far from the segments' capacity), and the mode is
 // refused when that would re-stream more than a quarter of a chunk.
-static int boot_pairs_for(int64_t Q, int64_t N, int64_t D, int dtype, int k, int* boot_tiles) {
-  static const bool disabled = getenv("ICR_NO_BOOT") != nullptr;  // A/B switch for benchmarks
-  if (disabled || !swap_applies(Q, N, D, dtype)) return 0;
+static int boot_pairs_for(int64_t Q, int64_t N, int64_t D, int k, int* boot_tiles) {
+  if (!swap_applies(Q, N, D)) return 0;
   const int64_t T = (N + BN - 1) / BN;
   const int pairs = static_cast<int>(T < kNumSMs / 2 ? T : kNumSMs / 2);
   const int groups = 8 * pairs;  // 2 CTAs x 4 epilogue warps
@@ -1498,30 +1460,30 @@ static GemmWs gemm_ws_layout(int64_t Q, int64_t N, int64_t D, int dtype, int k, 
   const int mode = mode_for(dtype);
   const int qblocks = static_cast<int>((Q + 2 * BM - 1) / (2 * BM));
   Phase ph[kMaxPhases];
-  const bool dense0 = dense0_applies(Q, N, D, dtype);
-  const int np = plan_phases(N, qblocks, k, ph, kMaxPhases, swap_applies(Q, N, D, dtype), dense0 ? dense0_tiles(Q, N) : 0);
+  const bool swap = swap_applies(Q, N, D);
+  const bool dense0 = !swap;  // K2 scores its first tiles densely (see launch_gemm_topk)
+  const int np = plan_phases(N, qblocks, k, ph, kMaxPhases, swap, dense0 ? dense0_tiles(Q, N) : 0);
   int maxc = 1;
   for (int i = 0; i < np; ++i) maxc = ph[i].chunks > maxc ? ph[i].chunks : maxc;
   w.boot_tiles = 0;
-  w.boot_pairs = boot_pairs_for(Q, N, D, dtype, k, &w.boot_tiles);
+  w.boot_pairs = boot_pairs_for(Q, N, D, k, &w.boot_tiles);
   if (w.boot_pairs > maxc) maxc = w.boot_pairs;
   w.k2_boot_chunks = 0;
   w.k2_boot_coarse = 0;
-  w.k2_boot_tiles = k2_boot_plan(Q, N, D, dtype, k, &w.k2_boot_chunks, &w.k2_boot_coarse);
+  w.k2_boot_tiles = k2_boot_plan(Q, N, D, k, &w.k2_boot_chunks, &w.k2_boot_coarse);
   if (w.k2_boot_chunks > maxc) maxc = w.k2_boot_chunks;
   w.max_chunks = maxc;
-  const int64_t dp = (D + 63) / 64 * 64;
-  const int64_t plane_elems = mode == 3 ? 2 * dp : dp;  // hi|lo planes, or the screen plane
+  const int64_t dp = (D + 63) / 64 * 64;  // elements of a screen-plane row
   size_t off = 0;
   auto take = [&](size_t bytes) {
     const size_t o = off;
     off += align_up(bytes, 1024);
     return o;
   };
-  w.q_planes = take(mode != 1 ? static_cast<size_t>(Q) * plane_elems * 2 : 0);
-  w.c_planes = take((mode == 3 || (mode == 2 && !have_planes)) ? static_cast<size_t>(N) * plane_elems * 2 : 0);
-  w.qinv = take(mode != 3 ? static_cast<size_t>(Q) * 4 : 0);
-  w.cinv = take((mode != 3 && !have_cinv) ? static_cast<size_t>(N) * 4 : 0);
+  w.q_planes = take(mode == 2 ? static_cast<size_t>(Q) * dp * 2 : 0);
+  w.c_planes = take((mode == 2 && !have_planes) ? static_cast<size_t>(N) * dp * 2 : 0);
+  w.qinv = take(static_cast<size_t>(Q) * 4);
+  w.cinv = take(!have_cinv ? static_cast<size_t>(N) * 4 : 0);
   w.tau = take(static_cast<size_t>(Q) * 4);
   w.overflow = take(static_cast<size_t>(Q) * 4 + 32);  // + the grid-barrier counters of the boot mode (zeroed with the flags)
   w.kc = carry_cap(k, mode);
@@ -1530,7 +1492,7 @@ static GemmWs gemm_ws_layout(int64_t Q, int64_t N, int64_t D, int dtype, int k, 
     w.carry_cnt[i] = take(static_cast<size_t>(Q) * 4);
   }
   w.seg_cap = seg_cap_for(k);
-  const int halves = swap_applies(Q, N, D, dtype) ? 2 : epi_warps(mode == 3 ? 3 : 1) / 4;
+  const int halves = swap ? 2 : epi_warps(1) / 4;
   w.cand = take(static_cast<size_t>(Q) * maxc * halves * w.seg_cap * 8);
   w.cand_cnt = take(static_cast<size_t>(Q) * maxc * halves * 4);
   w.scratch = take(static_cast<size_t>(kNumSMs) * kEpiWarps * kSegCapMax * 8);  // in-kernel compaction scratch
@@ -1553,16 +1515,6 @@ bool gemm_topk_supported(int64_t Q, int64_t N, int64_t D, int dtype, int k, cons
 size_t gemm_topk_workspace_bytes(int64_t Q, int64_t N, int64_t D, int dtype, int k, int have_planes) {
   // sized without cached inverse norms so that one figure covers both cases
   return gemm_ws_layout(Q, N, D, dtype, k, have_planes, 0).total;
-}
-
-// tau = -inf (phase 0 admits every row), overflow flags cleared
-__global__ void init_phase_state_kernel(float* tau, unsigned int* overflow, int64_t n) {
-  const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (i < n) {
-    tau[i] = -INFINITY;
-    overflow[i] = 0u;
-  }
-  if (i < 8) overflow[n + i] = 0u;  // the grid-barrier counters kept behind the flags
 }
 
 int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* catalog, int64_t N, int64_t ldc, int64_t D,
@@ -1601,26 +1553,14 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
   sa.id_offset = row_offset;
   sa.raw_keys = 1;  // the only producer of segments is the GEMM epilogue
   CUtensorMap map_a, map_b;
-  bool state_ready = false;
   const void* q_operand = queries;  // what the TMA map of the swapped kernel is built over
   int64_t q_cols = D, q_ld = ldq;
-  if (mode == 3) {
-    uint16_t* qp = reinterpret_cast<uint16_t*>(base + L.q_planes);
-    uint16_t* cp = reinterpret_cast<uint16_t*>(base + L.c_planes);
-    if ((rc = launch_split_planes(static_cast<const float*>(queries), Q, D, ldq, qp, st))) return rc;
-    if ((rc = launch_split_planes(static_cast<const float*>(catalog), N, D, ldc, cp, st))) return rc;
-    if ((rc = make_map(&map_a, qp, Q, 2 * dp, 2 * dp, false))) return rc;
-    if ((rc = make_map(&map_b, cp, N, 2 * dp, 2 * dp, false))) return rc;
-    g.kb_per_term = static_cast<int>(dp / BK);
-    g.plane_stride = static_cast<int>(dp);
-    g.acc_scale = 1.0f / 65536.0f;
-    q_operand = qp;
-    q_cols = q_ld = 2 * dp;
-  } else if (mode == 2) {
+  // the query-side preparation kernels also initialise tau (-inf: phase 0 admits every row), the overflow flags and the
+  // grid-barrier counters behind them
+  if (mode == 2) {
     uint16_t* qp = reinterpret_cast<uint16_t*>(base + L.q_planes);
     float* qinv = reinterpret_cast<float*>(base + L.qinv);
     if ((rc = launch_screen_plane(static_cast<const float*>(queries), Q, D, ldq, qp, qinv, st, const_cast<float*>(g.tau), g.overflow))) return rc;
-    state_ready = true;
     const uint16_t* cp = cat_planes;
     const float* cinv = cat_inv_norms;
     if (!cp) {
@@ -1656,7 +1596,6 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
   } else {
     float* qinv = reinterpret_cast<float*>(base + L.qinv);
     if ((rc = launch_row_inv_norms(queries, Q, D, ldq, dtype, qinv, st, const_cast<float*>(g.tau), g.overflow))) return rc;
-    state_ready = true;
     const float* cinv = cat_inv_norms;
     if (!cinv) {
       float* built = reinterpret_cast<float*>(base + L.cinv);
@@ -1673,19 +1612,14 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
   }
   sa.out_scale = g.acc_scale;
   sa.out_qscale = g.qinv;
-  const int terms = mode == 3 ? 3 : 1;
-  const bool swap = swap_applies(Q, N, D, dtype);
-  const bool astat = terms == 1 && g.kb_per_term <= kAStatMaxKB;
+  const bool swap = swap_applies(Q, N, D);
+  const bool astat = g.kb_per_term <= kAStatMaxKB;
   int which;
-  if (swap) which = mode == 3 ? 3 : (mode == 1 ? 4 : 7);
-  else which = mode == 3 ? 0 : (mode == 1 ? (astat ? 2 : 1) : (astat ? 6 : 5));
+  if (swap) which = mode == 1 ? 4 : 7;
+  else which = mode == 1 ? (astat ? 2 : 1) : (astat ? 6 : 5);
   if (swap) {
     g.qpad = static_cast<int>((Q + 31) / 32 * 32);
     if ((rc = make_map(&map_a, q_operand, Q, q_cols, q_ld, mode == 1, g.qpad / 2))) return rc;
-  }
-  if (!state_ready) {  // the query-side preparation kernels of the one-term paths initialise tau / overflow themselves
-    init_phase_state_kernel<<<static_cast<unsigned>((Q + 255) / 256), 256, 0, st>>>(const_cast<float*>(g.tau), g.overflow, Q);
-    ICR_LAUNCH_CHECK();
   }
 
   if (L.boot_pairs > 0) {
@@ -1706,13 +1640,11 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
     // k-th largest of `groups` maxima of 32 rows each, so ~N * k / (32 * groups * boot_tiles) rows pass it (plus the screening
     // band's share): that has to stay under a third of the tail's buffer (a query that overflows it anyway is still exact). Larger cases (catalogs that
     // stream from HBM, where the select is a few percent of the call) keep the separate select launch.
-    static const bool no_fuse = getenv("ICR_NO_FUSED_SELECT") != nullptr;  // A/B switch for benchmarks and tests
     const double expect = static_cast<double>(N) * k / (256.0 * L.boot_pairs * L.boot_tiles);
     // One CTA finishes one query at a time: more queries than CTAs means rounds, which only short lists (k <= 32) afford
     // (Q = 256 on the 49,688-row catalog: k = 10 75 us against 89 us with the select launch, k = 100 134 against 118).
     const bool one_round = Q <= 2 * L.boot_pairs || k <= 32;
-    g.fuse_select = (!no_fuse && mode != 3 && one_round && sp.nseg <= kTailSegs && expect <= kTailCap / 3 &&
-                     (mode != 2 || D % 4 == 0)) ? 1 : 0;
+    g.fuse_select = (one_round && sp.nseg <= kTailSegs && expect <= kTailCap / 3 && (mode != 2 || D % 4 == 0)) ? 1 : 0;
     if ((rc = launch_swap_variant(which, 2 * L.boot_pairs, map_a, map_b, g, st, sp))) return rc;
     if (g.fuse_select) return ICR_OK;
     return run_select(sp, Q, st);
@@ -1731,7 +1663,7 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
     const int pairs = items < kNumSMs / 2 ? items : kNumSMs / 2;
     if ((rc = launch_gemm_variant<false>(which, 2 * pairs, map_a, map_b, g, st))) return rc;
     HistSelectArgs sp = sa;
-    sp.nseg = g.chunks * (epi_warps(terms) / 4);
+    sp.nseg = g.chunks * (epi_warps(1) / 4);
     sp.carry_out = mode == 2 ? reinterpret_cast<uint64_t*>(base + L.carry[0]) : nullptr;
     sp.carry_cnt_out = mode == 2 ? reinterpret_cast<int*>(base + L.carry_cnt[0]) : nullptr;
     sp.out_scores = out_scores;
@@ -1744,7 +1676,7 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
   // score matrix instead (full 128-byte lines) and the select builds its keys from that.
   Phase ph[kMaxPhases];
   const int T = static_cast<int>((N + BN - 1) / BN);
-  const bool dense0 = dense0_applies(Q, N, D, dtype);
+  const bool dense0 = !swap;  // K2 only
   int done_phases = 0;
   if (dense0) {
     const int kDense0Tiles = dense0_tiles(Q, N);
@@ -1792,7 +1724,7 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
     const bool last = (pp == np - 1);
     const int cur = p & 1, prev = cur ^ 1;
     HistSelectArgs sp = sa;
-    sp.nseg = g.chunks * (swap ? 2 : epi_warps(terms) / 4);
+    sp.nseg = g.chunks * (swap ? 2 : epi_warps(1) / 4);
     sp.carry_in = p > 0 ? reinterpret_cast<uint64_t*>(base + L.carry[prev]) : nullptr;
     sp.carry_cnt_in = p > 0 ? reinterpret_cast<int*>(base + L.carry_cnt[prev]) : nullptr;
     const bool keep = !last || mode == 2;

@@ -12,8 +12,6 @@
 //
 // Replaces sentence_transformers.losses.MultipleNegativesRankingLoss.forward + autograd
 // (constructed at reference src/training/train_sbert.py:182-185).
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace icr {
@@ -323,9 +321,8 @@ static int launch_mnrl_tm(const MnrlArgs& g, bool bwd, cudaStream_t st) {
 template <typename T, int NCV>
 static int launch_mnrl(const MnrlArgs& g, bool bwd, cudaStream_t st) {
   using C = MnrlCfg<T, NCV>;
-  // fewer CTAs than SMs with the default tile: spread the batch over 2-row tiles (ICR_MNRL_TM=0 keeps the default, for A/B runs)
-  static const int tm_env = getenv("ICR_MNRL_TM") ? atoi(getenv("ICR_MNRL_TM")) : 2;
-  if (C::TM > 2 && tm_env == 2 && (g.B + C::TM - 1) / C::TM < 148) return launch_mnrl_tm<T, NCV, 2>(g, bwd, st);
+  // fewer CTAs than SMs with the default tile: spread the batch over 2-row tiles
+  if (C::TM > 2 && (g.B + C::TM - 1) / C::TM < 148) return launch_mnrl_tm<T, NCV, 2>(g, bwd, st);
   return launch_mnrl_tm<T, NCV, 0>(g, bwd, st);
 }
 

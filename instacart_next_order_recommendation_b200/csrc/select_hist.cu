@@ -11,8 +11,6 @@
 // Keys are distinct 64-bit values (score bits, ~row), so ties in score are resolved exactly by row and the
 // refinement always terminates. The final phase sorts the k selected keys; earlier phases only need the set
 // and its minimum (the new threshold tau).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "ptx.cuh"
 #include "select_args.cuh"
@@ -827,9 +825,8 @@ int launch_peer_exchange_merge(const float* scores, const int64_t* ids, int64_t 
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeCooperative;
   attr[0].val.cooperative = 1;
-  static const bool no_coop = getenv("ICR_NO_COOP") != nullptr;  // A/B switch (the grid is sized to be co-resident either way)
   cfg.attrs = attr;
-  cfg.numAttrs = no_coop ? 0 : 1;
+  cfg.numAttrs = 1;
   ICR_CUDA_CHECK(cudaLaunchKernelEx(&cfg, peer_exchange_merge_kernel, m));
   count_launch();
   return ICR_OK;
@@ -852,12 +849,14 @@ int launch_merge_lists(const float* cs, const int64_t* ci, int64_t Q, int G, int
   return run_select(a, Q, st);
 }
 
+// batches of up to this many queries take the block-per-query select, larger ones a warp per query
+constexpr int64_t kSelectBlockMaxQ = 512;
+
 int run_select(const HistSelectArgs& a, int64_t Q, cudaStream_t st) {
   static thread_local SmemAttrCache warp_cache, block_cache;  // per device
   int rc = ensure_dyn_smem(warp_cache, select_hist_kernel, sizeof(LsSmem));
   if (rc) return rc;
-  static const int block_max_q = getenv("ICR_SELECT_BLOCK_MAXQ") ? atoi(getenv("ICR_SELECT_BLOCK_MAXQ")) : 512;  // tuning hook
-  if (Q <= block_max_q) {
+  if (Q <= kSelectBlockMaxQ) {
     if ((rc = ensure_dyn_smem(block_cache, select_block_kernel, sizeof(BsSmem)))) return rc;
     select_block_kernel<<<static_cast<unsigned>(Q), kBsThreads, sizeof(BsSmem), st>>>(a);
     ICR_LAUNCH_CHECK();

@@ -15,8 +15,8 @@ and ``DeviceCatalog.from_index`` streams either one into HBM chunk by chunk thro
 buffers — for a whole catalog or for one rank's row block of a sharded one (SURVEY §8f row 3).
 
 ``DeviceCatalog`` is what the kernels read: the same rows resident in HBM (fp32, or bf16
-on request), plus — for fp32 — the fp16 (hi|lo) operand planes of the tensor-core path,
-built once at load instead of re-normalising the catalog on every request as
+on request), plus — for fp32 — the fp16 screening plane and the inverse row norms of the
+tensor-core path, built once at load instead of re-normalising the catalog on every request as
 ``sentence_transformers.util.cos_sim`` does (serve_recommendations.py:214).
 """
 
