@@ -134,6 +134,31 @@ int icr_cos_topk(const void* queries, int64_t Q, int64_t ldq,
                  float* out_scores, int64_t* out_ids,
                  void* workspace, size_t workspace_bytes, void* stream);
 
+/* Per-query exclusions: a bitmap `bits` uint32 [ceil(N/32)][Q] (device memory, 4-byte aligned). Row r of the catalog
+ * (a local row, before row_offset) is excluded for query q when bit r % 32 of bits[r / 32][q] is set. The word index
+ * is outermost: the 32 rows a kernel filters together share one word, and 32 consecutive queries read one 128-byte
+ * line. Q * ceil(N/32) * 4 bytes: 6.2 KB per query on a 49,688-row catalog.
+ *
+ * icr_query_exclusion_bits builds it from a CSR list (the convention of icr_ir_metrics): query q excludes
+ * rows[offsets[q] .. offsets[q+1]), in any order, duplicates allowed; rows outside [0, N) are ignored, as the
+ * reference skips excluded ids that are not in the catalog. offsets [Q + 1] and rows are device memory. One memset and
+ * one scatter kernel on `stream`; a caller that reuses an exclusion set across calls builds it once. */
+int icr_query_exclusion_bits(const int64_t* offsets, const int64_t* rows, int64_t Q, int64_t N,
+                             uint32_t* bits, void* stream);
+
+/* icr_cos_topk with per-query exclusions `excl_bits` (the bitmap above, for these Q queries and N rows; NULL = none,
+ * which is exactly icr_cos_topk). Given together with exclude_mask, a row is excluded when either says so. Same
+ * workspace (icr_cos_topk_workspace_bytes) and the same plan: the bitmap changes only which rows are eligible. If fewer
+ * than k rows are eligible for a query, its tail is (-inf, -1). Not available on the sharded entry. */
+int icr_cos_topk_excl(const void* queries, int64_t Q, int64_t ldq,
+                      const void* catalog, int64_t N, int64_t ldc,
+                      int64_t D, int dtype,
+                      const uint16_t* cat_planes, const float* cat_inv_norms,
+                      const uint8_t* exclude_mask, const uint32_t* excl_bits,
+                      int k, int64_t row_offset, int path,
+                      float* out_scores, int64_t* out_ids,
+                      void* workspace, size_t workspace_bytes, void* stream);
+
 /* number of kernel launches the last icr_cos_topk call on this thread enqueued */
 int icr_last_launch_count(void);
 

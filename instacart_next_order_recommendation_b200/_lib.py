@@ -53,6 +53,12 @@ SIGNATURES = {
         [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int64,
          c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
     ),
+    "icr_query_exclusion_bits": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
+    "icr_cos_topk_excl": (
+        c_int,
+        [c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
+         c_int64, c_int, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p],
+    ),
     "icr_cos_sim_dense_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int]),
     "icr_cos_sim_dense": (
         c_int,

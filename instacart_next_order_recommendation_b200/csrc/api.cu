@@ -64,7 +64,7 @@ int launch_peer_exchange(const float* scores, const int64_t* ids, int64_t n, int
                          int64_t n_max, cudaStream_t st);
 int gemv_grid(int64_t N);
 int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, const void* q, int64_t ldq, int Q,
-                     const uint8_t* mask, int k, uint64_t* part_keys, int* part_cnt, int grid, float* out_scores, int64_t* out_ids,
+                     const uint8_t* mask, const uint32_t* xbits, int64_t xld, int k, uint64_t* part_keys, int* part_cnt, int grid, float* out_scores, int64_t* out_ids,
                      int64_t id_offset, unsigned int* done_counter, cudaStream_t st, const float* cat_inv, const PeerTail* peer = nullptr,
                      float* fin_scores = nullptr, int64_t* fin_ids = nullptr);
 size_t select_scratch_bytes(int64_t Q, int nseg, int seg_cap, int k);
@@ -79,8 +79,8 @@ int launch_cos_sim_dense(const void* a, int64_t Qa, int64_t lda, const void* b, 
 // GEMM path (gemm_topk.cu)
 size_t gemm_topk_workspace_bytes(int64_t Q, int64_t N, int64_t D, int dtype, int k, int have_planes);
 int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* catalog, int64_t N, int64_t ldc, int64_t D,
-                     int dtype, const uint16_t* cat_planes, const float* cat_inv_norms, const uint8_t* mask, int k, int64_t row_offset,
-                     float* out_scores, int64_t* out_ids, void* ws, size_t ws_bytes, cudaStream_t st);
+                     int dtype, const uint16_t* cat_planes, const float* cat_inv_norms, const uint8_t* mask, const uint32_t* xbits, int k,
+                     int64_t row_offset, float* out_scores, int64_t* out_ids, void* ws, size_t ws_bytes, cudaStream_t st);
 bool gemm_topk_supported(int64_t Q, int64_t N, int64_t D, int dtype, int k, const uint8_t* mask);
 size_t gemm_dense_workspace_bytes(int64_t Qa, int64_t Nb, int64_t D, int dtype);
 int launch_gemm_dense(const void* a, int64_t Qa, int64_t lda, const void* b, int64_t Nb, int64_t ldb, int64_t D, int dtype, float* out,
@@ -97,6 +97,7 @@ int launch_scale2(const void* x0, const void* x1, int64_t n, int dtype, const fl
 bool mnrl_tc_applies(int64_t B, int64_t Bc, int64_t D);
 size_t mnrl_tc_workspace_bytes(int64_t B, int64_t Bc, int64_t D);
 int launch_mnrl_tc(const MnrlArgs& m, int dtype, int mode, void* ws, size_t ws_bytes, cudaStream_t st);
+int launch_query_exclusion_bits(const int64_t* offsets, const int64_t* rows, int64_t Q, int64_t N, uint32_t* bits, cudaStream_t st);
 int launch_ir_metrics(const int64_t* ids, int64_t Q, int K, int64_t ld, const int64_t* rel_offsets, const int64_t* rel_rows,
                       const int32_t* n_relevant, const int32_t* kinds, const int32_t* ks, int M, double* per_query, double* means,
                       cudaStream_t st);
@@ -270,8 +271,10 @@ size_t icr_cos_topk_workspace_bytes(int64_t Q, int64_t N, int64_t D, int dtype, 
 
 // `peer` != null (request-sized sharded call on the GEMV path, gemv_peer_tail_fits): the exchange and the global merge happen
 // in the tail of the scoring kernel; out_* then receive the GLOBAL top-k and stage_* hold the shard's own lists.
+// `excl_bits` (per-query exclusions, [ceil(N/32)][Q]) is null on the sharded entry.
 static int cos_topk_impl(const void* queries, int64_t Q, int64_t ldq, const void* catalog, int64_t N, int64_t ldc, int64_t D,
-                         int dtype, const uint16_t* cat_planes, const float* cat_inv_norms, const uint8_t* exclude_mask, int k,
+                         int dtype, const uint16_t* cat_planes, const float* cat_inv_norms, const uint8_t* exclude_mask,
+                         const uint32_t* excl_bits, int k,
                          int64_t row_offset, int path, float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
                          void* stream, const PeerTail* peer, float* stage_scores, int64_t* stage_ids) {
   int rc;
@@ -288,6 +291,10 @@ static int cos_topk_impl(const void* queries, int64_t Q, int64_t ldq, const void
   if (Q > 0 && (!out_scores || !out_ids)) {
     set_error("cos_topk: null output");
     return ICR_ERR_ARG;
+  }
+  if ((reinterpret_cast<uintptr_t>(excl_bits) & 3) != 0) {
+    set_error("cos_topk: excl_bits must be 4-byte aligned");
+    return ICR_ERR_ALIGN;
   }
   if ((rc = check_device())) return rc;
   if (Q == 0) return ICR_OK;
@@ -310,7 +317,7 @@ static int cos_topk_impl(const void* queries, int64_t Q, int64_t ldq, const void
                 (long long)N, (long long)D, k, exclude_mask != nullptr);
       return ICR_ERR_ARG;
     }
-    return launch_gemm_topk(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, k, row_offset,
+    return launch_gemm_topk(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, excl_bits, k, row_offset,
                             out_scores, out_ids, workspace, workspace_bytes, st);
   }
   if (N == 0) {
@@ -334,25 +341,47 @@ static int cos_topk_impl(const void* queries, int64_t Q, int64_t ldq, const void
   // the last CTA of every GEMV launch merges the per-CTA lists itself (no select launch on the latency path)
   if (!ws_resident) ICR_CUDA_CHECK(cudaMemsetAsync(done_counter, 0, 2 * sizeof(unsigned int), st));  // ticket + slab-chunk counter
   if (peer)  // the merging CTA of the one GEMV launch also exchanges and merges (gemv_topk.cu peer_tail_merge)
-    return launch_gemv_topk(catalog, N, ldc, static_cast<int>(D), dtype, queries, ldq, static_cast<int>(Q), exclude_mask, k, part_keys, part_cnt,
+    return launch_gemv_topk(catalog, N, ldc, static_cast<int>(D), dtype, queries, ldq, static_cast<int>(Q), exclude_mask, nullptr, 0, k, part_keys, part_cnt,
                             grid, stage_scores, stage_ids, row_offset, done_counter, st, cat_inv_norms, peer, out_scores, out_ids);
   for (int64_t q0 = 0; q0 < Q; q0 += qc) {
     const int nq = static_cast<int>(Q - q0 < qc ? Q - q0 : qc);
     const char* qptr = static_cast<const char*>(queries) + q0 * ldq * esz;
-    rc = launch_gemv_topk(catalog, N, ldc, static_cast<int>(D), dtype, qptr, ldq, nq, exclude_mask, k, part_keys, part_cnt, grid,
+    rc = launch_gemv_topk(catalog, N, ldc, static_cast<int>(D), dtype, qptr, ldq, nq, exclude_mask, excl_bits ? excl_bits + q0 : nullptr, Q, k,
+                          part_keys, part_cnt, grid,
                           out_scores + q0 * k, out_ids + q0 * k, row_offset, done_counter, st, cat_inv_norms);
     if (rc) return rc;
   }
   return ICR_OK;
 }
 
+int icr_cos_topk_excl(const void* queries, int64_t Q, int64_t ldq, const void* catalog, int64_t N, int64_t ldc, int64_t D,
+                      int dtype, const uint16_t* cat_planes, const float* cat_inv_norms, const uint8_t* exclude_mask,
+                      const uint32_t* excl_bits, int k, int64_t row_offset, int path, float* out_scores, int64_t* out_ids, void* workspace,
+                      size_t workspace_bytes, void* stream) {
+  g_launches = 0;
+  return cos_topk_impl(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, excl_bits, k, row_offset, path,
+                       out_scores, out_ids, workspace, workspace_bytes, stream, nullptr, nullptr, nullptr);
+}
+
 int icr_cos_topk(const void* queries, int64_t Q, int64_t ldq, const void* catalog, int64_t N, int64_t ldc, int64_t D,
                  int dtype, const uint16_t* cat_planes, const float* cat_inv_norms, const uint8_t* exclude_mask, int k,
                  int64_t row_offset, int path, float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
                  void* stream) {
+  return icr_cos_topk_excl(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, nullptr, k, row_offset, path,
+                           out_scores, out_ids, workspace, workspace_bytes, stream);
+}
+
+int icr_query_exclusion_bits(const int64_t* offsets, const int64_t* rows, int64_t Q, int64_t N, uint32_t* bits, void* stream) {
   g_launches = 0;
-  return cos_topk_impl(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, k, row_offset, path, out_scores,
-                       out_ids, workspace, workspace_bytes, stream, nullptr, nullptr, nullptr);
+  if (Q < 0 || N < 0 || N >= 0xffffffffll || (Q > 0 && !offsets) || (Q > 0 && N > 0 && !bits) || (reinterpret_cast<uintptr_t>(bits) & 3)) {
+    set_error("query_exclusion_bits: bad arguments Q=%lld N=%lld (offsets, and bits for N > 0, must be non-null; bits 4-byte aligned)",
+              (long long)Q, (long long)N);
+    return ICR_ERR_ARG;
+  }
+  int rc;
+  if ((rc = check_device())) return rc;
+  if (Q == 0 || N == 0) return ICR_OK;
+  return launch_query_exclusion_bits(offsets, rows, Q, N, bits, static_cast<cudaStream_t>(stream));
 }
 
 static int check_peer_args(const char* who, int64_t n, int rank, int world, const uint64_t* peer_buffers, uint32_t epoch, int64_t n_max) {
@@ -419,10 +448,10 @@ int icr_cos_topk_sharded(const void* queries, int64_t Q, int64_t ldq, const void
   const PeerTail tail = make_peer_tail(rank, world, peer_buffers, epoch, n_max);
   const int p = resolve_path(path & ~ICR_PATH_WS_RESIDENT, Q, N, D, dtype, k, exclude_mask);
   if (p == ICR_PATH_GEMV && gemv_peer_tail_fits(static_cast<int>(Q < 8 ? Q : 8), k, world))  // one launch for the whole sharded request
-    return cos_topk_impl(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, k, row_offset, path, out_scores, out_ids,
+    return cos_topk_impl(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, nullptr, k, row_offset, path, out_scores, out_ids,
                          workspace, local_ws, stream, &tail, stage_scores, stage_ids);
   // otherwise the shard's lists go to the staging area and the exchange + merge kernel writes the outputs
-  rc = cos_topk_impl(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, k, row_offset, path, stage_scores, stage_ids,
+  rc = cos_topk_impl(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, nullptr, k, row_offset, path, stage_scores, stage_ids,
                      workspace, local_ws, stream, nullptr, nullptr, nullptr);
   if (rc) return rc;
   return launch_peer_exchange_merge(stage_scores, stage_ids, Q, k, tail, out_scores, out_ids, static_cast<cudaStream_t>(stream));

@@ -98,6 +98,27 @@ __host__ __device__ __forceinline__ uint64_t make_key(float s, uint32_t row) {
 __host__ __device__ __forceinline__ float key_score(uint64_t k) { return unorder_bits(static_cast<uint32_t>(k >> 32)); }
 __host__ __device__ __forceinline__ uint32_t key_row(uint64_t k) { return ~static_cast<uint32_t>(k); }
 
+// ---- excluded rows ---------------------------------------------------------------------------
+// `shared`: one byte per catalog row, the same for every query of a call. `bits`: per-query bitmap [ceil(N/32)][ld]
+// (icr_query_exclusion_bits), row r excluded for query q when bit r % 32 of bits[r / 32][q] is set. The word index is
+// outermost because the 32 rows of one epilogue block always share a word: 32 consecutive queries then read one
+// 128-byte line (K2), and 32 consecutive rows of one query read one word (K2s, the selects).
+// The kernels that accept a bitmap are separate instantiations (template flag BITS): the others compile to the
+// shared-mask test alone.
+struct Exclusions {
+  const uint8_t* shared;
+  const uint32_t* bits;
+  int64_t ld;  // queries per word row of `bits`
+  __device__ __forceinline__ uint32_t word(int64_t q, int64_t row32) const { return __ldg(bits + row32 * ld + q); }
+  __device__ __forceinline__ bool bit(int64_t q, int64_t row) const { return (word(q, row >> 5) >> (row & 31)) & 1u; }
+  template <bool BITS>
+  __device__ __forceinline__ bool excluded(int64_t q, int64_t row) const {
+    if (shared && shared[row]) return true;
+    if constexpr (BITS) return bit(q, row);
+    return false;
+  }
+};
+
 // ---- vector loads -------------------------------------------------------------------------
 // streaming 128-bit load: read-only path, do not allocate in L1 (catalog rows are used once)
 __device__ __forceinline__ uint4 ldg_stream(const void* p) {

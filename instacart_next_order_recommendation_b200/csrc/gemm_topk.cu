@@ -91,6 +91,8 @@ struct GemmArgs {
   int boot_coarse;           // K2 single-launch mode: ONE maximum per (bootstrap tile, column group) instead of one per 32 scores
   float band;                // screened scores (MODE 2): tau already sits `band` below the k-th best; 0 = exact scores
   unsigned int* overflow;    // [Q] screened scores: set when a segment cannot be cut back without losing keys of the band
+  const uint32_t* xbits;     // per-query exclusions (Exclusions::bits, ld = xld): read by the XB instantiations only
+  int64_t xld;
 };
 
 // chunk c of a phase covers tiles [first(c), first(c+1)): sizes differ by at most one tile
@@ -171,6 +173,25 @@ __device__ __forceinline__ void append_if(SegState& s, float sc, float tau_f, ui
       : "l"(s.seg + s.cnt), "f"(sc), "f"(tau_f), "r"(nrow), "r"(__float_as_uint(sc))
       : "memory");
   s.cnt += static_cast<int>(inc);
+}
+
+// Per-query exclusions (XB kernels): the accumulators of the rows that this thread's bitmap word `w` excludes become -inf
+// before any filter, maximum or bound sees them. Every filter is a strict ">", which never admits -inf (not even against
+// the first phase's tau = -inf), so the fast paths stay as they are; a warp whose 32 words are all zero skips the selects.
+__device__ __forceinline__ void exclude32(uint32_t (&r)[32], uint32_t w) {
+  if (__any_sync(kFull, w != 0u)) {
+#pragma unroll
+    for (int j = 0; j < 32; ++j) r[j] = ((w >> j) & 1u) ? 0xff800000u : r[j];
+  }
+}
+
+// Bootstrap threshold from the k-th largest group maximum `ks` (order bits): one ulp below it, minus the screening band.
+// XB kernels: a query with fewer than k eligible groups (rows excluded) has a k-th maximum of -inf, and its threshold
+// is -inf rather than the NaN one ulp below -inf would give (which no score passes).
+template <bool XB>
+__device__ __forceinline__ float boot_tau(uint32_t ks, float band) {
+  if (XB && ks <= order_bits(-INFINITY)) return -INFINITY;
+  return unorder_bits(ks > 1u ? ks - 1u : ks) - band;
 }
 
 // Filter 32 accumulator columns (catalog rows rbase .. rbase+31) of this thread's query.
@@ -312,11 +333,13 @@ __device__ __forceinline__ void k2_grid_barrier(unsigned int* counter, unsigned 
 // ASTAT (bf16, D <= 384): the work item's 128 query rows stay resident in shared memory for all of its catalog
 // tiles ("A-stationary"), so the ring streams catalog tiles only: 31 instead of 62 B/cycle/SM of L2 traffic,
 // which is the difference between L2-bound and tensor-bound for one-term MMAs (profiles/r01_notes.md).
-template <int MODE, bool ASTAT, bool DENSE>
+// XB (filtering kernels only): the call excludes rows per query (GemmArgs::xbits).
+template <int MODE, bool ASTAT, bool DENSE, bool XB = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kGemmThreads, 1)
 gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, const GemmArgs g) {
   constexpr int TERMS = (MODE == 3) ? 3 : 1;
   static_assert(!ASTAT || TERMS == 1, "A-stationary is a one-term variant");
+  static_assert(!XB || !DENSE, "dense scores are filtered by the select");
   constexpr bool BF16 = (MODE == 1);
   constexpr int EW = epi_warps(TERMS), EH = EW / 4, ECOLS = BN / EH;  // epilogue warps, column groups, columns per warp
   constexpr int kStageTiles = ASTAT ? 1 : ((TERMS == 3) ? 4 : 2);  // B | A_hi A_lo B_hi B_lo | A B
@@ -502,6 +525,25 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     const int cap = g.seg_cap;
     int acc = 0;
     uint32_t acc_phase = 0;
+    // XB: this query's bitmap words, one per 32-row block of the ECOLS columns a tile gives this warp. The next tile's words
+    // are loaded while the current tile is filtered (xw) and staged at the start of each tile in this warp's share of the
+    // bootstrap's ranking buffer (idle outside the ranking): xs[u * 32 + lane] = word of block u.
+    uint32_t* xs = boot_s + (warp - 4) * (kK2BootCap + kHsBins);
+    uint32_t xw[ECOLS / 32];
+    auto load_words = [&](int q, bool live, int row0) {
+      if constexpr (XB) {
+#pragma unroll
+        for (int u = 0; u < ECOLS / 32; ++u)
+          xw[u] = (live && row0 + u * 32 < g.N) ? Exclusions{nullptr, g.xbits, g.xld}.word(q, (row0 >> 5) + u) : 0u;
+      }
+    };
+    auto stage_words = [&]() {
+      if constexpr (XB) {
+#pragma unroll
+        for (int u = 0; u < ECOLS / 32; ++u) xs[u * 32 + lane] = xw[u];
+        __syncwarp();
+      }
+    };
     if (!DENSE && g.boot > 0) {
       // ---- single-launch mode, pass 0: group maxima of the first g.boot tiles of every work item ----------------------
       // A thread owns one query and sees 32 catalog scores per TMEM load: the maximum of each such block is the score of
@@ -519,9 +561,12 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         const int q = qb * (2 * BM) + static_cast<int>(rank) * BM + ew * 32 + lane;
         const bool live = q < g.Q;
         float* gq = g.gmax + static_cast<int64_t>(live ? q : 0) * gstride + (chunk * g.boot * EH + half) * per_tile;
+        load_words(q, live, t0 * BN + half * ECOLS);
         for (int bt = 0; bt < g.boot; ++bt) {
           float m_tile = -INFINITY;
           const int row0 = (t0 + bt) * BN + half * ECOLS;
+          stage_words();
+          if (bt + 1 < g.boot) load_words(q, live, row0 + BN);
           if (BF16) {
             __syncwarp();
 #pragma unroll
@@ -540,6 +585,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             uint32_t r[32];
             tmem_ld32(taddr + cb * 32, r);
             tmem_ld_wait(r);
+            if (XB) exclude32(r, xs[cb * 32 + lane]);  // an excluded row must not be a block's maximum: the k-th maximum stays a lower bound
             float m = -INFINITY;
             if (plain) {
 #pragma unroll
@@ -575,7 +621,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         uint32_t ks, kr;
         ls_kth(bsc, bsc, gstride, g.k, bhist, lane, ks, kr);  // only the k-th VALUE matters: the tie-break word is the value itself
         // the filter is a strict ">" and the bootstrap rows are filtered again in pass 1: one ulp below the k-th maximum
-        if (lane == 0) const_cast<float*>(g.tau)[j] = unorder_bits(ks > 1u ? ks - 1u : ks) - g.band;
+        if (lane == 0) const_cast<float*>(g.tau)[j] = boot_tau<XB>(ks, g.band);
         __syncwarp();
       }
       k2_grid_barrier(g.gsync + 1, gridDim.x, warp - 4, EW);
@@ -592,10 +638,13 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
       constexpr bool dense = DENSE;  // compile-time: the top-k instantiation keeps its register budget
       s.tau_ob = (live && !dense) ? order_bits(__ldcg(g.tau + q)) : 0xFFFFFFFFu;
       float* out_q = dense ? g.dense_out + static_cast<int64_t>(live ? q : 0) * g.dense_ld : nullptr;
+      load_words(q, live, t0 * BN + half * ECOLS);
       const float qscale = dense ? (g.dense_raw ? 1.0f : g.acc_scale * ((BF16 && live) ? g.qinv[q] : 1.0f)) : 0.f;
       const bool vec_ok = dense && (g.dense_ld % 4 == 0) && ((reinterpret_cast<uintptr_t>(g.dense_out) & 15) == 0);
       for (int tile = t0; tile < t1; ++tile) {
         const int row0 = tile * BN + half * ECOLS;
+        stage_words();
+        if (tile + 1 < t1) load_words(q, live, row0 + BN);
         float cmax_l = 1.f, cmin_l = 1.f;  // lane u: extremes of the inverse norms of 32-row block u
         if (BF16) {
           // stage this warp's catalog inverse norms once per tile (read back as shared-memory broadcasts), with
@@ -630,6 +679,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             if (live) dense_store32<BF16>(ra, out_q + row0 + cb * 32, qscale, cinv_s + cb * 32, g.N - (row0 + cb * 32), vec_ok);
           } else {
             compact_full_segments(s, scratch, cap, g.k, lane, g.band, g.overflow, q - lane);
+            if (XB) exclude32(ra, xs[cb * 32 + lane]);
             filter32<BF16>(ra, s, cinv_s + cb * 32, __shfl_sync(kFull, cmax_l, cb), __shfl_sync(kFull, cmin_l, cb), row0 + cb * 32, fast,
                            g.N, g.mask);
           }
@@ -639,6 +689,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             if (live) dense_store32<BF16>(rb, out_q + row0 + (cb + 1) * 32, qscale, cinv_s + (cb + 1) * 32, g.N - (row0 + (cb + 1) * 32), vec_ok);
           } else {
             compact_full_segments(s, scratch, cap, g.k, lane, g.band, g.overflow, q - lane);
+            if (XB) exclude32(rb, xs[(cb + 1) * 32 + lane]);
             filter32<BF16>(rb, s, cinv_s + (cb + 1) * 32, __shfl_sync(kFull, cmax_l, cb + 1), __shfl_sync(kFull, cmin_l, cb + 1),
                            row0 + (cb + 1) * 32, fast, g.N, g.mask);
           }
@@ -745,6 +796,7 @@ __device__ __forceinline__ void tail_order(const uint64_t* src, uint64_t* dst, i
   epi_sync();
 }
 
+template <bool XB>
 __device__ __noinline__ void swap_select_tail(unsigned int* gsync, const HistSelectArgs& a, unsigned char* ring, int ew, int lane, int et) {
   swap_grid_barrier(gsync, gridDim.x, et);
   uint64_t* kin = reinterpret_cast<uint64_t*>(ring);               // [kTailCap] gathered keys
@@ -831,7 +883,7 @@ __device__ __noinline__ void swap_select_tail(unsigned int* gsync, const HistSel
         }
       } else if (lost) {  // too many near-ties inside the band: rank the whole catalog for this query
         if (ew == 0) {
-          const int kr = ls_rank_catalog(sc, rw, kLsCap, hist, q, a, lane);
+          const int kr = ls_rank_catalog<XB>(sc, rw, kLsCap, hist, q, a, lane);
           ls_emit_ranked(sc, rw, kr, k, 1.0f, q, a, hist, lane);
         }
       } else {
@@ -874,7 +926,7 @@ __device__ __noinline__ void swap_select_tail(unsigned int* gsync, const HistSel
         kept = kc;
       }
       if (screened) {
-        if (lost || __ldcg(a.overflow + q) != 0u) kept = ls_rank_catalog(sc, rw, kLsCap, hist, q, a, lane);
+        if (lost || __ldcg(a.overflow + q) != 0u) kept = ls_rank_catalog<XB>(sc, rw, kLsCap, hist, q, a, lane);
         else ls_rescore<false>(sc, rw, kept, q, a, lane);
         ls_emit_ranked(sc, rw, kept, k, 1.0f, q, a, hist, lane);
       } else {
@@ -885,7 +937,41 @@ __device__ __noinline__ void swap_select_tail(unsigned int* gsync, const HistSel
   }
 }
 
-template <int MODE>
+// Per-query exclusions of the swapped kernel (XB): a warp's 32 rows share one bitmap word per query. Lane l loads the words
+// of queries l, l + 32, ... for the tile's row block (coalesced) into this warp's share of the bootstrap buffer, xs[query]
+// (idle outside the bootstrap's ranking); row `lane` of the warp is excluded for query j when bit `lane` of xs[j] is set
+// (broadcast reads).
+// The boot tiles load their words before the epilogue waits for the accumulator and store them after it; the filtering tiles
+// load the next tile's words while the current one is filtered.
+__device__ __forceinline__ void load_swap_words(uint32_t (&w)[8], const GemmArgs& g, int row32, int lane) {
+#pragma unroll
+  for (int b = 0; b < 8; ++b) {
+    const int q = b * 32 + lane;
+    w[b] = (b * 32 < g.qpad && q < g.Q && row32 * 32 < g.N) ? Exclusions{nullptr, g.xbits, g.xld}.word(q, row32) : 0u;
+  }
+}
+__device__ __forceinline__ void store_swap_words(uint32_t* xs, const uint32_t (&w)[8], int qpad, int lane) {
+  __syncwarp();
+#pragma unroll
+  for (int b = 0; b < 8; ++b)
+    if (b * 32 < qpad) xs[b * 32 + lane] = w[b];
+  __syncwarp();
+}
+// bit j: query jb + j excludes row `lane` of this warp
+__device__ __forceinline__ uint32_t swap_excluded32(const uint32_t* xs, int jb, int lane) {
+  uint32_t m = 0u;
+#pragma unroll
+  for (int j = 0; j < 32; j += 4) {
+    const uint4 w = *reinterpret_cast<const uint4*>(xs + jb + j);
+    m |= ((w.x >> lane) & 1u) << j;
+    m |= ((w.y >> lane) & 1u) << (j + 1);
+    m |= ((w.z >> lane) & 1u) << (j + 2);
+    m |= ((w.w >> lane) & 1u) << (j + 3);
+  }
+  return m;
+}
+
+template <int MODE, bool XB = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kSwapThreads, 1)
 gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant__ CUtensorMap tma_c, const GemmArgs g,
                  const __grid_constant__ HistSelectArgs sel) {
@@ -1016,6 +1102,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
     const int ew = warp & 3, et = threadIdx.x - 128;
     const int cap = g.seg_cap;
     uint64_t* scratch = g.compact_scratch + (static_cast<int64_t>(blockIdx.x) * kEpiWarps + ew) * kSegCapMax;
+    uint32_t* xs = boot_s + ew * (2 * kBootCap + kHsBins);  // XB: [qpad] staged bitmap words (see stage_swap_words)
     int acc = 0;
     uint32_t acc_phase = 0;
     for (int w = pair; w < items; w += npairs) {
@@ -1037,8 +1124,11 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
           const int row = (t0 + bt) * BN + static_cast<int>(rank) * BNH + ew * 32 + lane;
           const bool valid = row < g.N && !(g.mask && g.mask[row]);
           const float cinv_r = BF16 ? (row < g.N ? __ldg(g.cinv + row) : 0.f) : 1.0f;
+          uint32_t xw[8];
+          if (XB) load_swap_words(xw, g, (row - lane) >> 5, lane);
           mbar_wait(smem_u32(&tfull_bar[acc]), acc_phase);
           tc_fence_after();
+          if (XB) store_swap_words(xs, xw, g.qpad, lane);
           const uint32_t taddr = tmem_base + (static_cast<uint32_t>(ew * 32) << 16) + static_cast<uint32_t>(acc * 256);
 #pragma unroll
           for (int b = 0; b < 8; ++b) {
@@ -1047,8 +1137,9 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
               tmem_ld32(taddr + b * 32, r);
               tmem_ld_wait(r);
               float sc[32];
+              const uint32_t xm = XB ? swap_excluded32(xs, b * 32, lane) : 0u;  // excluded (row, query) pairs do not bound anything
 #pragma unroll
-              for (int j = 0; j < 32; ++j) sc[j] = valid ? __uint_as_float(r[j]) * cinv_r : -INFINITY;
+              for (int j = 0; j < 32; ++j) sc[j] = (valid && !((xm >> j) & 1u)) ? __uint_as_float(r[j]) * cinv_r : -INFINITY;
               warp_transpose_max<32>(sc, lane);  // lane l: the maximum over this warp's rows for query 32 * b + l
               best[b] = fmaxf(best[b], sc[0]);
             }
@@ -1078,7 +1169,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
           ls_kth(bsc, brw, gstride, g.k, bhist, lane, ks, kr);
           // the filter is a strict ">", and the bootstrap rows are filtered again: the threshold sits one ulp BELOW the k-th
           // group maximum so that the row it came from (and its exact ties) survive
-          if (lane == 0) const_cast<float*>(g.tau)[j] = unorder_bits(ks > 1u ? ks - 1u : ks) - g.band;
+          if (lane == 0) const_cast<float*>(g.tau)[j] = boot_tau<XB>(ks, g.band);
           __syncwarp();
         }
         swap_grid_barrier(g.gsync + 1, gridDim.x, et);
@@ -1089,11 +1180,18 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
       }
       if (et == 0) flag_s[0] = 0;
       epi_sync();
+      const int wrow0 = static_cast<int>(rank) * BNH + ew * 32;  // this warp's first row of a tile
+      uint32_t xw[8];  // XB: the words of the next tile, loaded while the current one is filtered
+      if (XB) load_swap_words(xw, g, (t0 * BN + wrow0) >> 5, lane);
       for (int tile = t0; tile < t1; ++tile) {
-        const int row = tile * BN + static_cast<int>(rank) * BNH + ew * 32 + lane;
+        const int row = tile * BN + wrow0 + lane;
         const bool valid = row < g.N && !(g.mask && g.mask[row]);
         const float cinv_r = BF16 ? (row < g.N ? __ldg(g.cinv + row) : 0.f) : 1.0f;
         const uint32_t nrow = ~static_cast<uint32_t>(row);
+        if (XB) {
+          store_swap_words(xs, xw, g.qpad, lane);
+          if (tile + 1 < t1) load_swap_words(xw, g, ((tile + 1) * BN + wrow0) >> 5, lane);
+        }
         mbar_wait(smem_u32(&tfull_bar[acc]), acc_phase);
         tc_fence_after();
         const uint32_t taddr = tmem_base + (static_cast<uint32_t>(ew * 32) << 16) + static_cast<uint32_t>(acc * 256);
@@ -1116,6 +1214,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
             m |= (sc[j + 3] > t4.w ? 1u : 0u) << (j + 3);
           }
           if (!valid) m = 0;
+          if (XB && __any_sync(kFull, xs[jb + lane] != 0u)) m &= ~swap_excluded32(xs, jb, lane);
           if (__any_sync(kFull, m != 0)) {
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
@@ -1180,7 +1279,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
       for (int j = et; j < g.Q; j += 128) g.cand_cnt[static_cast<int64_t>(j) * g.chunks * 2 + seg0] = min(cnt_s[j], cap);
       epi_sync();
     }
-    if (g.fuse_select) swap_select_tail(g.gsync + 2, sel, smem, ew, lane, et);
+    if (g.fuse_select) swap_select_tail<XB>(g.gsync + 2, sel, smem, ew, lane, et);
   }
 
   tc_fence_before();
@@ -1297,11 +1396,11 @@ static int dense0_tiles(int64_t Q, int64_t N) { return (Q <= 2 * BM && (N + BN -
 // kernel variants: 1 = bf16 streaming both operands, 2 = bf16 with resident queries, 5 / 6 = fp16 screen plane streaming /
 // resident queries, 4 / 7 = swapped kernel (small batches) on bf16 / the screen plane; DENSE only: 0 = fp16 hi|lo planes,
 // three MMA terms (K2' on fp32 inputs)
-#define ICR_GEMM_VARIANTS(X, DENSE)            \
-  X(1, (gemm_topk_kernel<1, false, DENSE>))    \
-  X(2, (gemm_topk_kernel<1, true, DENSE>))     \
-  X(5, (gemm_topk_kernel<2, false, DENSE>))    \
-  X(6, (gemm_topk_kernel<2, true, DENSE>))
+#define ICR_GEMM_VARIANTS(X, DENSE, XB)            \
+  X(1, (gemm_topk_kernel<1, false, DENSE, XB>))    \
+  X(2, (gemm_topk_kernel<1, true, DENSE, XB>))     \
+  X(5, (gemm_topk_kernel<2, false, DENSE, XB>))    \
+  X(6, (gemm_topk_kernel<2, true, DENSE, XB>))
 
 // Launch helper of the GEMM kernels. The single-launch modes (g.boot > 0) synchronise the whole grid through a counter in
 // global memory, which needs every CTA resident at once: those launches carry the cooperative attribute, so the driver
@@ -1332,14 +1431,15 @@ static void launch_gemm_grid(void (*kernel)(KArgs...), int grid, int threads, si
   kernel<<<grid, threads, smem, st>>>(KArgs(args)...);
 }
 
-// launches instantiation `which` of the queries-on-M kernel, DENSE (K2' / first phase) or filtering
-template <bool DENSE>
+// launches instantiation `which` of the queries-on-M kernel, DENSE (K2' / first phase) or filtering (XB: with per-query
+// exclusions)
+template <bool DENSE, bool XB = false>
 static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, const CUtensorMap& map_b, const GemmArgs& g, cudaStream_t st) {
   static thread_local SmemAttrCache cache[8];
   int rc = ICR_OK;
 #define ICR_SET(ID, K) \
   if (which == ID) rc = ensure_dyn_smem(cache[ID], K, kGemmSmemBytes);
-  ICR_GEMM_VARIANTS(ICR_SET, DENSE)
+  ICR_GEMM_VARIANTS(ICR_SET, DENSE, XB)
   if constexpr (DENSE) ICR_SET(0, (gemm_topk_kernel<3, false, true>))
 #undef ICR_SET
   if (rc) return rc;
@@ -1348,7 +1448,7 @@ static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, co
   const int threads = 128 + epi_warps(terms) * 32;
 #define ICR_RUN(ID, K) \
   if (which == ID) launch_gemm_grid(K, grid, threads, kGemmSmemBytes, st, g.boot > 0, map_a, map_b, g);
-  ICR_GEMM_VARIANTS(ICR_RUN, DENSE)
+  ICR_GEMM_VARIANTS(ICR_RUN, DENSE, XB)
   if constexpr (DENSE) ICR_RUN(0, (gemm_topk_kernel<3, false, true>))
 #undef ICR_RUN
   profile_end(st);
@@ -1356,16 +1456,17 @@ static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, co
   return ICR_OK;
 }
 
+template <bool XB = false>
 static int launch_swap_variant(int which, int grid, const CUtensorMap& map_q, const CUtensorMap& map_c, const GemmArgs& g, cudaStream_t st,
                                const HistSelectArgs& sel = HistSelectArgs{}) {
   static thread_local SmemAttrCache cache[2];
   int rc = ICR_OK;
-  if (which == 4) rc = ensure_dyn_smem(cache[0], gemm_swap_kernel<1>, kSwapSmemBytes);
-  if (which == 7) rc = ensure_dyn_smem(cache[1], gemm_swap_kernel<2>, kSwapSmemBytes);
+  if (which == 4) rc = ensure_dyn_smem(cache[0], gemm_swap_kernel<1, XB>, kSwapSmemBytes);
+  if (which == 7) rc = ensure_dyn_smem(cache[1], gemm_swap_kernel<2, XB>, kSwapSmemBytes);
   if (rc) return rc;
   profile_begin(kKernelGemm, 1, st);
-  if (which == 4) launch_gemm_grid(gemm_swap_kernel<1>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
-  if (which == 7) launch_gemm_grid(gemm_swap_kernel<2>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
+  if (which == 4) launch_gemm_grid(gemm_swap_kernel<1, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
+  if (which == 7) launch_gemm_grid(gemm_swap_kernel<2, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
   profile_end(st);
   ICR_LAUNCH_CHECK();
   return ICR_OK;
@@ -1517,9 +1618,16 @@ size_t gemm_topk_workspace_bytes(int64_t Q, int64_t N, int64_t D, int dtype, int
   return gemm_ws_layout(Q, N, D, dtype, k, have_planes, 0).total;
 }
 
+// the filtering GEMM launches of a call, with or without per-query exclusions
+static int launch_filter(bool swap, int which, int grid, const CUtensorMap& map_a, const CUtensorMap& map_b, const GemmArgs& g, cudaStream_t st,
+                         const HistSelectArgs& sel = HistSelectArgs{}) {
+  if (swap) return g.xbits ? launch_swap_variant<true>(which, grid, map_a, map_b, g, st, sel) : launch_swap_variant<false>(which, grid, map_a, map_b, g, st, sel);
+  return g.xbits ? launch_gemm_variant<false, true>(which, grid, map_a, map_b, g, st) : launch_gemm_variant<false, false>(which, grid, map_a, map_b, g, st);
+}
+
 int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* catalog, int64_t N, int64_t ldc, int64_t D,
-                     int dtype, const uint16_t* cat_planes, const float* cat_inv_norms, const uint8_t* mask, int k, int64_t row_offset,
-                     float* out_scores, int64_t* out_ids, void* ws, size_t ws_bytes, cudaStream_t st) {
+                     int dtype, const uint16_t* cat_planes, const float* cat_inv_norms, const uint8_t* mask, const uint32_t* xbits, int k,
+                     int64_t row_offset, float* out_scores, int64_t* out_ids, void* ws, size_t ws_bytes, cudaStream_t st) {
   const int mode = mode_for(dtype);
   const GemmWs L = gemm_ws_layout(Q, N, D, dtype, k, cat_planes != nullptr, cat_inv_norms != nullptr);
   if (ws_bytes < L.total) {
@@ -1536,6 +1644,8 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
   g.k = k;
   g.qblocks = qblocks;
   g.mask = mask;
+  g.xbits = xbits;
+  g.xld = Q;
   g.tau = reinterpret_cast<float*>(base + L.tau);
   g.overflow = reinterpret_cast<unsigned int*>(base + L.overflow);
   g.cand = reinterpret_cast<uint64_t*>(base + L.cand);
@@ -1552,6 +1662,8 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
   sa.seg_stride = sa.seg_cap = g.seg_cap;
   sa.id_offset = row_offset;
   sa.raw_keys = 1;  // the only producer of segments is the GEMM epilogue
+  sa.xbits = xbits;
+  sa.xld = Q;
   CUtensorMap map_a, map_b;
   const void* q_operand = queries;  // what the TMA map of the swapped kernel is built over
   int64_t q_cols = D, q_ld = ldq;
@@ -1645,7 +1757,7 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
     // (Q = 256 on the 49,688-row catalog: k = 10 75 us against 89 us with the select launch, k = 100 134 against 118).
     const bool one_round = Q <= 2 * L.boot_pairs || k <= 32;
     g.fuse_select = (one_round && sp.nseg <= kTailSegs && expect <= kTailCap / 3 && (mode != 2 || D % 4 == 0)) ? 1 : 0;
-    if ((rc = launch_swap_variant(which, 2 * L.boot_pairs, map_a, map_b, g, st, sp))) return rc;
+    if ((rc = launch_filter(true, which, 2 * L.boot_pairs, map_a, map_b, g, st, sp))) return rc;
     if (g.fuse_select) return ICR_OK;
     return run_select(sp, Q, st);
   }
@@ -1661,7 +1773,7 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
     g.chunks = L.k2_boot_chunks;
     const int items = qblocks * g.chunks;
     const int pairs = items < kNumSMs / 2 ? items : kNumSMs / 2;
-    if ((rc = launch_gemm_variant<false>(which, 2 * pairs, map_a, map_b, g, st))) return rc;
+    if ((rc = launch_filter(false, which, 2 * pairs, map_a, map_b, g, st))) return rc;
     HistSelectArgs sp = sa;
     sp.nseg = g.chunks * (epi_warps(1) / 4);
     sp.carry_out = mode == 2 ? reinterpret_cast<uint64_t*>(base + L.carry[0]) : nullptr;
@@ -1718,9 +1830,7 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
     const int items = qblocks * g.chunks;
     const int pairs = items < kNumSMs / 2 ? items : kNumSMs / 2;
     const int grid = 2 * pairs;  // whole CTA pairs (cluster dims 2x1x1)
-    if (swap) rc = launch_swap_variant(which, grid, map_a, map_b, g, st);
-    else rc = launch_gemm_variant<false>(which, grid, map_a, map_b, g, st);
-    if (rc) return rc;
+    if ((rc = launch_filter(swap, which, grid, map_a, map_b, g, st))) return rc;
     const bool last = (pp == np - 1);
     const int cur = p & 1, prev = cur ^ 1;
     HistSelectArgs sp = sa;

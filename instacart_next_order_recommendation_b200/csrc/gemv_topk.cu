@@ -94,6 +94,9 @@ struct GemvArgs {
   float* fin_scores;
   int64_t* fin_ids;
   PeerTail peer;
+  // per-query exclusions (XB kernels): Exclusions::bits of this call's queries, query a.q0 + t at column a.q0 + t
+  const uint32_t* xbits;
+  int64_t xld;
 };
 
 // barrier over the 256 compute threads: the whole CTA in the direct kernel, a named barrier in the ring kernel
@@ -204,7 +207,8 @@ __device__ __forceinline__ void fma_vector(const uint4 (&c)[RB], const float* qs
 
 // transposing reduction of the RB*(QT+1) partial sums, then threshold test and candidate append
 // NORMS: lane r (< RB) brings the precomputed inverse norm of row r0 + r in `inv_lane`
-template <int RB, int QT, bool NORMS = false>
+// XB: per-query exclusions, one scattered bitmap load for the (few) scores that beat the threshold
+template <int RB, int QT, bool NORMS = false, bool XB = false>
 __device__ __forceinline__ void reduce_and_append(float (&acc)[RB * (QT + (NORMS ? 0 : 1))], const GemvArgs& a, GemvSmem<QT>& sm, int nq, int64_t r0,
                                                   int64_t row_limit, int lane, float inv_lane = 0.f) {
   constexpr int V = RB * (QT + (NORMS ? 0 : 1));
@@ -219,7 +223,7 @@ __device__ __forceinline__ void reduce_and_append(float (&acc)[RB * (QT + (NORMS
   if (t < nq && (lane & ((1 << SH) - 1)) == 0 && row < row_limit) {
     const bool excluded = a.mask && a.mask[row];
     const float score = acc[0] * inv;
-    if (!excluded && score > sm.tau[t]) {
+    if (!excluded && score > sm.tau[t] && !(XB && Exclusions{nullptr, a.xbits, a.xld}.bit(a.q0 + t, row))) {
       const int pos = atomicAdd(&sm.ncand[t], 1);
       if (pos < GemvSmem<QT>::CAND) sm.cand[t * GemvSmem<QT>::CAND + pos] = make_key(score, static_cast<uint32_t>(row));
     }
@@ -649,7 +653,7 @@ __device__ __forceinline__ void emit_and_merge(const GemvArgs& a, GemvSmem<QT>& 
 // =====================================================================================================
 // direct-load kernel: RB rows per warp batch, QT queries per pass; V = RB * (QT + 1) in {16, 32}
 // =====================================================================================================
-template <typename T, int RB, int QT>
+template <typename T, int RB, int QT, bool XB = false>
 __global__ void __launch_bounds__(kGemvThreads) gemv_topk_kernel(GemvArgs a) {
   constexpr int VEC = Elem<T>::VEC;
   constexpr int V = RB * (QT + 1);
@@ -695,7 +699,7 @@ __global__ void __launch_bounds__(kGemvThreads) gemv_topk_kernel(GemvArgs a) {
           if (v < nvec) fma_vector<T, RB, QT>(c[u], sm.qs, dpad, v, acc);
         }
       }
-      reduce_and_append<RB, QT>(acc, a, sm, nq, r0, blk_end, lane);
+      reduce_and_append<RB, QT, false, XB>(acc, a, sm, nq, r0, blk_end, lane);
     }
     __syncthreads();
     refresh_thresholds<QT, false>(a, sm, nq, blk + kBlockRows >= row_end, kBlockRows, tid);
@@ -706,7 +710,7 @@ __global__ void __launch_bounds__(kGemvThreads) gemv_topk_kernel(GemvArgs a) {
 // =====================================================================================================
 // ring kernel: producer warp + bulk async copies into a shared-memory ring, 8 consumer warps
 // =====================================================================================================
-template <typename T, int QT, bool NORMS = false>
+template <typename T, int QT, bool NORMS = false, bool XB = false>
 __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) {
   static_assert(!NORMS || QT == 1, "precomputed norms: single-query kernel only (V must stay a power of two)");
   constexpr int VEC = Elem<T>::VEC;
@@ -875,7 +879,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) 
           c[r] = *reinterpret_cast<const uint4*>(slab + static_cast<size_t>(g * RB + r) * row_bytes + static_cast<size_t>(v) * 16);
         fma_vector<T, RB, QT, NORMS>(c, sm.qs, dpad, v, acc);
       }
-      reduce_and_append<RB, QT, NORMS>(acc, a, sm, nq, r0 + g * RB, a.N, lane, inv_lane);
+      reduce_and_append<RB, QT, NORMS, XB>(acc, a, sm, nq, r0 + g * RB, a.N, lane, inv_lane);
     }
     __syncwarp();
     if (lane == 0) ptx::mbar_arrive(ptx::smem_u32(&empty_bar[slot]));
@@ -902,16 +906,16 @@ __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) 
 // ---- host side --------------------------------------------------------------------------------------------
 constexpr size_t kSmemBudget = 227 * 1024 - 1024;
 
-template <typename T, int RB, int QT>
+template <typename T, int RB, int QT, bool XB>
 static int launch_direct(const GemvArgs& a, int grid, cudaStream_t st) {
   const size_t smem = GemvSmem<QT>::bytes(a.D);
   static thread_local SmemSizeCache configured;  // per device (ADVICE r1): a thread may serve several GPUs
   if (smem > 48 * 1024) {
-    const int rc = ensure_dyn_smem_size(configured, gemv_topk_kernel<T, RB, QT>, smem);
+    const int rc = ensure_dyn_smem_size(configured, gemv_topk_kernel<T, RB, QT, XB>, smem);
     if (rc) return rc;
   }
   profile_begin(kKernelGemv, 1, st);
-  gemv_topk_kernel<T, RB, QT><<<grid, kGemvThreads, smem, st>>>(a);
+  gemv_topk_kernel<T, RB, QT, XB><<<grid, kGemvThreads, smem, st>>>(a);
   profile_end(st);
   ICR_LAUNCH_CHECK();
   return ICR_OK;
@@ -934,7 +938,7 @@ static int ring_slots_for(int D) {
   return static_cast<int>(slots);
 }
 
-template <typename T, int QT, bool NORMS = false>
+template <typename T, int QT, bool NORMS, bool XB>
 static int launch_ring(GemvArgs a, int grid, cudaStream_t st) {
   a.ring_slots = ring_slots_for<T, QT>(a.D);
   {
@@ -951,11 +955,11 @@ static int launch_ring(GemvArgs a, int grid, cudaStream_t st) {
   const size_t smem = static_cast<size_t>(a.ring_slots) * (QT == 7 ? 4 : 8) * a.D * sizeof(T) + 3 * kMaxSlots * sizeof(uint64_t) + kMaxSlots * 8 * sizeof(float) + GemvSmem<QT>::bytes(a.D) + 128;
   static thread_local SmemSizeCache configured;  // per device
   {
-    const int rc = ensure_dyn_smem_size(configured, gemv_ring_kernel<T, QT, NORMS>, smem);
+    const int rc = ensure_dyn_smem_size(configured, gemv_ring_kernel<T, QT, NORMS, XB>, smem);
     if (rc) return rc;
   }
   profile_begin(kKernelGemv, 1, st);
-  gemv_ring_kernel<T, QT, NORMS><<<grid, kRingThreads, smem, st>>>(a);
+  gemv_ring_kernel<T, QT, NORMS, XB><<<grid, kRingThreads, smem, st>>>(a);
   profile_end(st);
   ICR_LAUNCH_CHECK();
   return ICR_OK;
@@ -994,9 +998,18 @@ int gemv_grid(int64_t N) {
   return static_cast<int>(g);
 }
 
+// one pass of qt (1, 3 or 7) queries
+template <typename T, bool XB>
+static int launch_gemv_pass(const GemvArgs& a, int qt, bool ring, int g, cudaStream_t st) {
+  if (qt == 1) return ring ? (a.cat_inv ? launch_ring<T, 1, true, XB>(a, g, st) : launch_ring<T, 1, false, XB>(a, g, st)) : launch_direct<T, 8, 1, XB>(a, g, st);
+  if (qt == 3) return ring ? launch_ring<T, 3, false, XB>(a, g, st) : launch_direct<T, 8, 3, XB>(a, g, st);
+  return ring ? launch_ring<T, 7, false, XB>(a, g, st) : launch_direct<T, 4, 7, XB>(a, g, st);
+}
+
 // Runs ceil(Q/7) passes (one for Q <= 7). part_keys/part_cnt sized [Q][grid][k] / [Q][grid].
+// xbits: per-query exclusions of these Q queries (Exclusions::bits with ld xld), or null.
 int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, const void* q, int64_t ldq, int Q,
-                     const uint8_t* mask, int k, uint64_t* part_keys, int* part_cnt, int grid, float* out_scores, int64_t* out_ids,
+                     const uint8_t* mask, const uint32_t* xbits, int64_t xld, int k, uint64_t* part_keys, int* part_cnt, int grid, float* out_scores, int64_t* out_ids,
                      int64_t id_offset, unsigned int* done_counter, cudaStream_t st, const float* cat_inv, const PeerTail* peer, float* fin_scores,
                      int64_t* fin_ids) {
   GemvArgs a{};
@@ -1008,7 +1021,6 @@ int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, 
   }
   // the ring kernel copies the inverse norms with 16-byte bulk copies; an unaligned array falls back to norms from the rows
   a.cat_inv = (reinterpret_cast<uintptr_t>(cat_inv) & 15) == 0 ? cat_inv : nullptr;
-  cat_inv = a.cat_inv;
   a.cat = cat;
   a.N = N;
   a.ldc = ldc;
@@ -1017,6 +1029,8 @@ int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, 
   a.ldq = ldq;
   a.Q = Q;
   a.mask = mask;
+  a.xbits = xbits;
+  a.xld = xld;
   a.k = k;
   a.part_keys = part_keys;
   a.part_cnt = part_cnt;
@@ -1034,17 +1048,8 @@ int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, 
     const int g = ring ? (grid < 148 ? grid : 148) : grid;
     a.rows_per_cta = (N + g - 1) / g;
     int rc;
-    if (dtype == ICR_F32) {
-      if (qt == 1) rc = ring ? (cat_inv ? launch_ring<float, 1, true>(a, g, st) : launch_ring<float, 1>(a, g, st)) : launch_direct<float, 8, 1>(a, g, st);
-      else if (qt == 3) rc = ring ? launch_ring<float, 3>(a, g, st) : launch_direct<float, 8, 3>(a, g, st);
-      else rc = ring ? launch_ring<float, 7>(a, g, st) : launch_direct<float, 4, 7>(a, g, st);
-    } else {
-      if (qt == 1)
-        rc = ring ? (cat_inv ? launch_ring<__nv_bfloat16, 1, true>(a, g, st) : launch_ring<__nv_bfloat16, 1>(a, g, st))
-                  : launch_direct<__nv_bfloat16, 8, 1>(a, g, st);
-      else if (qt == 3) rc = ring ? launch_ring<__nv_bfloat16, 3>(a, g, st) : launch_direct<__nv_bfloat16, 8, 3>(a, g, st);
-      else rc = ring ? launch_ring<__nv_bfloat16, 7>(a, g, st) : launch_direct<__nv_bfloat16, 4, 7>(a, g, st);
-    }
+    if (dtype == ICR_F32) rc = xbits ? launch_gemv_pass<float, true>(a, qt, ring, g, st) : launch_gemv_pass<float, false>(a, qt, ring, g, st);
+    else rc = xbits ? launch_gemv_pass<__nv_bfloat16, true>(a, qt, ring, g, st) : launch_gemv_pass<__nv_bfloat16, false>(a, qt, ring, g, st);
     if (rc != ICR_OK) return rc;
     q0 += qt;
   }

@@ -203,4 +203,27 @@ int launch_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, 
   return ICR_OK;
 }
 
+// ---- per-query exclusion bitmap (icr_query_exclusion_bits) ------------------------------------------------
+// One warp per query scatters its CSR list into bits[row / 32][q]; rows outside [0, N) are ignored, duplicates are harmless.
+__global__ void __launch_bounds__(256) query_exclusion_bits_kernel(const int64_t* __restrict__ offsets, const int64_t* __restrict__ rows,
+                                                                   int64_t Q, int64_t N, uint32_t* __restrict__ bits) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nwarps = static_cast<int64_t>(gridDim.x) * (blockDim.x >> 5);
+  for (int64_t q = static_cast<int64_t>(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5); q < Q; q += nwarps) {
+    const int64_t b = offsets[q], e = offsets[q + 1];
+    for (int64_t i = b + lane; i < e; i += 32) {
+      const int64_t r = rows[i];
+      if (r >= 0 && r < N) atomicOr(bits + (r >> 5) * Q + q, 1u << (r & 31));
+    }
+  }
+}
+
+int launch_query_exclusion_bits(const int64_t* offsets, const int64_t* rows, int64_t Q, int64_t N, uint32_t* bits, cudaStream_t st) {
+  ICR_CUDA_CHECK(cudaMemsetAsync(bits, 0, static_cast<size_t>((N + 31) / 32) * static_cast<size_t>(Q) * sizeof(uint32_t), st));
+  const int64_t blocks = (Q + 7) / 8;
+  query_exclusion_bits_kernel<<<static_cast<unsigned>(blocks < 148 * 8 ? blocks : 148 * 8), 256, 0, st>>>(offsets, rows, Q, N, bits);
+  ICR_LAUNCH_CHECK();
+  return ICR_OK;
+}
+
 }  // namespace icr

@@ -56,6 +56,11 @@ struct HistSelectArgs {
   int rs_D;
   const float* rs_qinv;     // [Q]
   const float* rs_cinv;     // [rs_N]
+  // per-query exclusions (Exclusions::bits, ld = Q): read by the dense front end and the whole-catalog rankings of the
+  // BITS instantiations only; the segments of the GEMM epilogue are already filtered
+  const uint32_t* xbits;
+  int64_t xld;
+  __device__ __forceinline__ Exclusions excl() const { return Exclusions{mask, xbits, xld}; }
 };
 
 int run_select(const HistSelectArgs& a, int64_t Q, cudaStream_t st);

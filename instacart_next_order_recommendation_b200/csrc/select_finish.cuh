@@ -151,6 +151,7 @@ __device__ __forceinline__ void ls_rescore(uint32_t* sc, const uint32_t* rw, int
 
 // Exact ranking of the WHOLE catalog for one query by one warp (only for queries whose screening band overflowed: more
 // near-ties around the k-th score than the carry holds). Leaves the k best exact keys in sc/rw, returns their number.
+template <bool XB = false>
 __device__ __forceinline__ int ls_rank_catalog(uint32_t* sc, uint32_t* rw, int buf_cap, uint32_t* hist, int64_t q, const HistSelectArgs& a, int lane) {
   const float* qrow = a.rs_q + q * a.rs_ldq;
   const float qi = a.rs_qinv[q];
@@ -166,7 +167,7 @@ __device__ __forceinline__ int ls_rank_catalog(uint32_t* sc, uint32_t* rw, int b
     score_rows8(qrow, rows, a.rs_D, acc, lane);
     warp_transpose_reduce<8>(acc, lane);
     const int64_t row = r0 + (lane >> 2);
-    bool ok = (lane & 3) == 0 && row < a.rs_N && !(a.mask && a.mask[row]);
+    bool ok = (lane & 3) == 0 && row < a.rs_N && !a.excl().excluded<XB>(q, row);
     uint32_t s1 = 0, r1 = 0;
     if (ok) {
       s1 = order_bits(acc[0] * qi * __ldg(a.rs_cinv + row));

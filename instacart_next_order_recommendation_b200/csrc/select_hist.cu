@@ -29,11 +29,12 @@ constexpr int kHsWarps = ICR_HS_WARPS;  // queries per CTA, 11 KB of shared memo
 constexpr int kHsSel = 512;       // >= 2 * ICR_MAX_K: the k results, or k + the band capacity of screened keys
 
 // flat candidate t of query q from the dense matrix or the shard lists -> key; false if there is none
+template <bool XB = false>
 __device__ __forceinline__ bool front_fetch(const HistSelectArgs& a, int64_t q, int t, int count, uint64_t& key) {
   key = 0ull;
   if (t >= count) return false;
   if (a.dense) {
-    if (a.mask && a.mask[t]) return false;
+    if (a.excl().excluded<XB>(q, t)) return false;
     key = make_key(__ldcs(a.dense + q * a.dense_ld + t), static_cast<uint32_t>(t));
     return true;
   }
@@ -54,6 +55,8 @@ struct LsSmem {
   uint32_t hist[kHsWarps][kHsBins];
 };
 
+// XB: the call excludes rows per query (HistSelectArgs::xbits); only the dense front end reads the bitmap
+template <bool XB>
 __global__ void __launch_bounds__(kHsWarps * 32, 24 / kHsWarps) select_hist_kernel(HistSelectArgs a) {
   extern __shared__ __align__(16) unsigned char hs_raw[];
   LsSmem& sm = *reinterpret_cast<LsSmem*>(hs_raw);
@@ -84,7 +87,7 @@ __global__ void __launch_bounds__(kHsWarps * 32, 24 / kHsWarps) select_hist_kern
       f[j] = t < a.dense_rows ? __ldcs(row + t) : 0.f;
     }
     int n = 0;
-    if (a.mask == nullptr) {  // key i = catalog row i
+    if (a.mask == nullptr && !XB) {  // key i = catalog row i
 #pragma unroll
       for (int j = 0; j < 32; ++j) {
         const int t = lane + 32 * j;
@@ -96,7 +99,7 @@ __global__ void __launch_bounds__(kHsWarps * 32, 24 / kHsWarps) select_hist_kern
 #pragma unroll
       for (int j = 0; j < 32; ++j) {
         const int t = lane + 32 * j;
-        const bool valid = t < a.dense_rows && !a.mask[t];
+        const bool valid = t < a.dense_rows && !a.excl().excluded<XB>(q, t);
         const unsigned m = __ballot_sync(kFull, valid);
         if (valid) {
           const int pos = n + __popc(m & lt);
@@ -139,7 +142,7 @@ __global__ void __launch_bounds__(kHsWarps * 32, 24 / kHsWarps) select_hist_kern
         uint64_t key[8];
         bool ok[8];
 #pragma unroll
-        for (int u = 0; u < 8; ++u) ok[u] = front_fetch(a, q, base + u * 32 + lane, count, key[u]);
+        for (int u = 0; u < 8; ++u) ok[u] = front_fetch<XB>(a, q, base + u * 32 + lane, count, key[u]);
 #pragma unroll
         for (int u = 0; u < 8; ++u) {
           const unsigned m = __ballot_sync(kFull, ok[u]);
@@ -289,6 +292,7 @@ struct RsSmem {
 #ifndef ICR_RS_WIDE
 #define ICR_RS_WIDE 1  // 1: 8 rows x 3 vectors = 24 loads per lane in flight (D = 384); 0: 4 x 3
 #endif
+template <bool XB>
 __global__ void __launch_bounds__(kHsWarps * 32, ICR_RS_MINB) rescore_rank_kernel(HistSelectArgs a) {
   __shared__ __align__(16) RsSmem sm;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -299,7 +303,7 @@ __global__ void __launch_bounds__(kHsWarps * 32, ICR_RS_MINB) rescore_rank_kerne
   int kept;
   ICR_ST_BEGIN();
   if (a.overflow[q]) {
-    kept = ls_rank_catalog(sc, rw, kRsCap, sm.hist[warp], q, a, lane);
+    kept = ls_rank_catalog<XB>(sc, rw, kRsCap, sm.hist[warp], q, a, lane);
   } else {
     kept = min(a.carry_cnt_in[q], a.kc);
     for (int i = lane; i < kept; i += 32) rw[i] = static_cast<uint32_t>(a.carry_in[q * a.kc + i]);
@@ -473,6 +477,7 @@ __device__ __forceinline__ uint64_t block_truncate(BsSmem& sm, int n, int kk, in
 
 // Exact ranking of the whole catalog for one query by one CTA (screening-band overflow only; see warp_rank_catalog).
 // Leaves the result keys in sm.sel[0..return value).
+template <bool XB>
 __device__ __forceinline__ int block_rank_catalog(BsSmem& sm, int64_t q, const HistSelectArgs& a, int tid) {
   const int warp = tid >> 5, lane = tid & 31;
   const float* qrow = a.rs_q + q * a.rs_ldq;
@@ -493,7 +498,7 @@ __device__ __forceinline__ int block_rank_catalog(BsSmem& sm, int64_t q, const H
     score_rows8(qrow, rows, a.rs_D, acc, lane);
     warp_transpose_reduce<8>(acc, lane);
     const int64_t row = w0 + (lane >> 2);
-    bool ok = (lane & 3) == 0 && row < a.rs_N && !(a.mask && a.mask[row]);
+    bool ok = (lane & 3) == 0 && row < a.rs_N && !a.excl().excluded<XB>(q, row);
     uint64_t key = 0ull;
     if (ok) {
       key = make_key(acc[0] * qi * __ldg(a.rs_cinv + row), static_cast<uint32_t>(row));
@@ -518,6 +523,7 @@ __device__ __forceinline__ int block_rank_catalog(BsSmem& sm, int64_t q, const H
   return n;
 }
 
+template <bool XB>
 __global__ void __launch_bounds__(kBsThreads) select_block_kernel(HistSelectArgs a) {
   extern __shared__ __align__(16) unsigned char bs_raw[];
   BsSmem& sm = *reinterpret_cast<BsSmem*>(bs_raw);
@@ -545,7 +551,7 @@ __global__ void __launch_bounds__(kBsThreads) select_block_kernel(HistSelectArgs
       uint64_t key[4];
       bool ok[4];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) ok[u] = front_fetch(a, q, base + u * kBsThreads + tid, count, key[u]);
+      for (int u = 0; u < 4; ++u) ok[u] = front_fetch<XB>(a, q, base + u * kBsThreads + tid, count, key[u]);
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
         const unsigned m = __ballot_sync(kFull, ok[u]);
@@ -665,7 +671,7 @@ __global__ void __launch_bounds__(kBsThreads) select_block_kernel(HistSelectArgs
       if (tid == 0) a.carry_cnt_out[q] = kept;
     }
     if (a.out_scores) {
-      if (a.overflow[q]) kept = block_rank_catalog(sm, q, a, tid);
+      if (a.overflow[q]) kept = block_rank_catalog<XB>(sm, q, a, tid);
       else warp_rescore(sm.sel, kept, warp, kBsThreads / 32, q, a, lane);
       __syncthreads();
       for (int i = tid; i < kept; i += kBsThreads) {  // kept <= kHsSel: rank counting, as below
@@ -852,18 +858,19 @@ int launch_merge_lists(const float* cs, const int64_t* ci, int64_t Q, int G, int
 // batches of up to this many queries take the block-per-query select, larger ones a warp per query
 constexpr int64_t kSelectBlockMaxQ = 512;
 
-int run_select(const HistSelectArgs& a, int64_t Q, cudaStream_t st) {
+template <bool XB>
+static int run_select_impl(const HistSelectArgs& a, int64_t Q, cudaStream_t st) {
   static thread_local SmemAttrCache warp_cache, block_cache;  // per device
-  int rc = ensure_dyn_smem(warp_cache, select_hist_kernel, sizeof(LsSmem));
+  int rc = ensure_dyn_smem(warp_cache, select_hist_kernel<XB>, sizeof(LsSmem));
   if (rc) return rc;
   if (Q <= kSelectBlockMaxQ) {
-    if ((rc = ensure_dyn_smem(block_cache, select_block_kernel, sizeof(BsSmem)))) return rc;
-    select_block_kernel<<<static_cast<unsigned>(Q), kBsThreads, sizeof(BsSmem), st>>>(a);
+    if ((rc = ensure_dyn_smem(block_cache, select_block_kernel<XB>, sizeof(BsSmem)))) return rc;
+    select_block_kernel<XB><<<static_cast<unsigned>(Q), kBsThreads, sizeof(BsSmem), st>>>(a);
     ICR_LAUNCH_CHECK();
     return ICR_OK;
   }
   const unsigned grid = static_cast<unsigned>((Q + kHsWarps - 1) / kHsWarps);
-  select_hist_kernel<<<grid, kHsWarps * 32, sizeof(LsSmem), st>>>(a);
+  select_hist_kernel<XB><<<grid, kHsWarps * 32, sizeof(LsSmem), st>>>(a);
   ICR_LAUNCH_CHECK();
   if (a.band > 0.f && a.out_scores) {
     // screened keys: the select left the candidates within the band in carry_out; re-score them exactly and rank
@@ -874,10 +881,14 @@ int run_select(const HistSelectArgs& a, int64_t Q, cudaStream_t st) {
     HistSelectArgs r = a;
     r.carry_in = a.carry_out;
     r.carry_cnt_in = a.carry_cnt_out;
-    rescore_rank_kernel<<<grid, kHsWarps * 32, 0, st>>>(r);
+    rescore_rank_kernel<XB><<<grid, kHsWarps * 32, 0, st>>>(r);
     ICR_LAUNCH_CHECK();
   }
   return ICR_OK;
+}
+
+int run_select(const HistSelectArgs& a, int64_t Q, cudaStream_t st) {
+  return a.xbits ? run_select_impl<true>(a, Q, st) : run_select_impl<false>(a, Q, st);
 }
 
 }  // namespace icr

@@ -463,10 +463,22 @@ class DeviceCatalog:
         cur.wait_stream(down)  # `down` waited on every piece of `rank`, which waited on every upload
         return vals_h, ids_h
 
-    def topk(self, queries, k: int, *, exclude_mask: torch.Tensor | None = None, path: int = ops.PATH_AUTO, peer=None):
+    # per-query exclusion bitmaps of one call stay below this; larger batches are split into query chunks
+    EXCLUSION_BITS_MAX_BYTES = 256 << 20
+
+    def topk(self, queries, k: int, *, exclude_mask: torch.Tensor | None = None, exclude_rows=None, path: int = ops.PATH_AUTO,
+             peer=None):
         """(values [Q,k], global ids [Q,k]) of the k most cosine-similar rows per query. With ``peer``
         (``PeerExchange.next_call()``; needs k <= len(self)) the rows are one rank's shard and the result is the global
-        top-k over all ranks' shards (``ops.cos_topk``)."""
+        top-k over all ranks' shards (``ops.cos_topk``).
+
+        ``exclude_mask`` (uint8/bool [len(self)]) drops rows for every query. ``exclude_rows`` gives one collection of
+        local rows per query (before ``row_offset``; out-of-range rows are ignored) that this query never returns: the
+        batch is searched in one fused call per chunk of queries whose exclusion bitmap (``ops.query_exclusion_bits``,
+        ceil(len(self)/32) words per query) fits EXCLUSION_BITS_MAX_BYTES. A query with fewer than k eligible rows gets a
+        (-inf, -1) tail."""
+        if exclude_rows is not None:
+            return self._topk_excluding(queries, k, exclude_rows, exclude_mask, path, peer)
         q = queries
         rows = self.rows
         if (exclude_mask is None and peer is None and isinstance(q, torch.Tensor) and q.dim() == 2 and 1 <= q.shape[0] <= 7 and q.is_cuda
@@ -484,6 +496,31 @@ class DeviceCatalog:
         ws = self._resident_workspace(q.shape[0], k, path, peer is not None) if q.shape[0] <= 8 else None
         return ops.cos_topk(q, self.rows, k, cat_planes=self.planes, cat_inv_norms=self.inv_norms, exclude_mask=exclude_mask,
                             row_offset=self.row_offset, path=path, workspace=ws, peer=peer)
+
+    def _topk_excluding(self, queries, k: int, exclude_rows, exclude_mask, path: int, peer):
+        if peer is not None:
+            raise ValueError("exclude_rows is not supported on a sharded call")
+        q = to_device_matrix(queries, device=self.device, dtype=self.dtype)
+        if q.dim() == 1:
+            q = q.unsqueeze(0)
+        Q = q.shape[0]
+        exclude_rows = list(exclude_rows)
+        if len(exclude_rows) != Q:
+            raise ValueError(f"exclude_rows has {len(exclude_rows)} entries for {Q} queries")
+        k = min(int(k), len(self))
+        if k < 1:
+            return (torch.empty(Q, 0, device=self.device), torch.empty(Q, 0, dtype=torch.int64, device=self.device))
+        per_query = 4 * ops.exclusion_words(len(self))
+        chunk = max(1, self.EXCLUSION_BITS_MAX_BYTES // per_query)
+        outs = []
+        for lo in range(0, Q, chunk):
+            hi = min(Q, lo + chunk)
+            bits = ops.query_exclusion_bits(exclude_rows[lo:hi], len(self), self.device)
+            outs.append(ops.cos_topk(q[lo:hi], self.rows, k, cat_planes=self.planes, cat_inv_norms=self.inv_norms,
+                                     exclude_mask=exclude_mask, exclude_bits=bits, row_offset=self.row_offset, path=path))
+        if len(outs) == 1:
+            return outs[0]
+        return torch.cat([v for v, _ in outs]), torch.cat([i for _, i in outs])
 
     def _resident_workspace(self, Q: int, k: int, path: int, sharded: bool = False) -> torch.Tensor:
         """Request-sized calls keep one zero-initialised workspace per (shape, stream): the library then skips the memset of

@@ -155,6 +155,48 @@ def convert_rows(x: torch.Tensor, out: torch.Tensor, *, normalize: bool = False)
     return out
 
 
+def exclusion_words(n_rows: int) -> int:
+    """Words per query of a per-query exclusion bitmap over `n_rows` catalog rows: ceil(n_rows / 32)."""
+    return (int(n_rows) + 31) // 32
+
+
+def query_exclusion_bits(rows_per_query, n_rows: int, device=None) -> torch.Tensor:
+    """Per-query exclusion bitmap uint32 [ceil(n_rows/32), Q] for ``cos_topk(..., exclude_bits=...)``.
+
+    `rows_per_query` is a sequence of Q iterables of catalog rows (local rows, before any row offset), or a CSR pair
+    ``(offsets [Q+1], rows)`` of int64 tensors. Any order, duplicates allowed; rows outside [0, n_rows) are ignored.
+    Row r is excluded for query q when bit r % 32 of ``bits[r // 32, q]`` is set. Built on the device
+    (``icr_query_exclusion_bits``); a bitmap can be reused by every call with the same queries' exclusions."""
+    import numpy as np
+
+    n_rows = int(n_rows)
+    if n_rows < 0:
+        raise ValueError("n_rows must be >= 0")
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    if dev.type != "cuda":
+        raise RuntimeError("the exclusion bitmap is built on a CUDA device (no CPU fallback)")
+    if isinstance(rows_per_query, tuple) and len(rows_per_query) == 2 and all(isinstance(t, torch.Tensor) for t in rows_per_query):
+        offsets, rows = rows_per_query
+        if offsets.dim() != 1 or offsets.numel() < 1 or rows.dim() != 1:
+            raise ValueError("CSR exclusions must be 1-D offsets [Q+1] and rows tensors")
+        offsets = offsets.to(device=dev, dtype=torch.int64).contiguous()
+        rows = rows.to(device=dev, dtype=torch.int64).contiguous()
+    else:
+        lists = [np.asarray(list(r) if not isinstance(r, np.ndarray) else r, dtype=np.int64).reshape(-1) for r in rows_per_query]
+        off = np.zeros(len(lists) + 1, dtype=np.int64)
+        if lists:
+            np.cumsum([len(r) for r in lists], out=off[1:])
+        flat = np.concatenate(lists) if lists and off[-1] > 0 else np.zeros(1, np.int64)
+        offsets = torch.from_numpy(off).to(dev)
+        rows = torch.from_numpy(flat).to(dev)
+    Q = offsets.numel() - 1
+    bits = torch.empty(exclusion_words(n_rows), Q, dtype=torch.uint32, device=dev)
+    lib = _lib.load()
+    with _on(dev):
+        _lib.check(lib.icr_query_exclusion_bits(offsets.data_ptr(), rows.data_ptr(), Q, n_rows, bits.data_ptr(), _stream(dev)))
+    return bits
+
+
 def cos_topk(
     queries: torch.Tensor,
     catalog: torch.Tensor,
@@ -163,6 +205,7 @@ def cos_topk(
     cat_planes: torch.Tensor | None = None,
     cat_inv_norms: torch.Tensor | None = None,
     exclude_mask: torch.Tensor | None = None,
+    exclude_bits: torch.Tensor | None = None,
     row_offset: int = 0,
     path: int = PATH_AUTO,
     out: tuple[torch.Tensor, torch.Tensor] | None = None,
@@ -170,6 +213,10 @@ def cos_topk(
     peer: tuple[int, int, int, int, int] | None = None,
 ):
     """(values f32 [Q,k] descending, ids int64 [Q,k]) == torch.topk(cos_sim(q, c), k, dim=1).
+
+    ``exclude_mask`` (uint8/bool [N]) drops rows for every query; ``exclude_bits`` (``query_exclusion_bits``, uint32
+    [ceil(N/32), Q]) drops rows per query. A row is dropped when either says so; queries with fewer than k eligible rows
+    get a (-inf, -1) tail.
 
     ``peer`` = (rank, world, address of the uint64 buffer-pointer array, epoch, n_max) from ``PeerExchange.next_call()``:
     `catalog` is this rank's row shard and the call also exchanges and merges the candidates of all ranks
@@ -191,6 +238,15 @@ def cos_topk(
         if exclude_mask.dtype not in (torch.uint8, torch.bool) or exclude_mask.numel() != N:
             raise ValueError("exclude_mask must be uint8/bool with one entry per catalog row")
         exclude_mask = exclude_mask.contiguous().view(torch.uint8)
+    if exclude_bits is not None:
+        _require_cuda("exclude_bits", exclude_bits)
+        if exclude_bits.dtype not in (torch.uint32, torch.int32) or tuple(exclude_bits.shape) != (exclusion_words(N), Q):
+            raise ValueError(f"exclude_bits must be uint32 [ceil(N/32), Q] = [{exclusion_words(N)}, {Q}] (query_exclusion_bits)")
+        if exclude_bits.device != catalog.device:
+            raise ValueError("exclude_bits must live on the catalog's device")
+        if peer is not None:
+            raise ValueError("per-query exclusions are not supported on the sharded call")
+        exclude_bits = exclude_bits.contiguous()
     if cat_planes is not None:
         if cat_planes.dtype != torch.float16 or cat_planes.shape != (N, lib.icr_screen_plane_row_elems(D)) or not cat_planes.is_contiguous():
             raise ValueError("cat_planes must be the contiguous plane returned by screen_plane(catalog)")
@@ -219,6 +275,15 @@ def cos_topk(
                     queries.data_ptr(), Q, _ld(queries), catalog.data_ptr(), N, _ld(catalog), D, dt, _ptr(cat_planes), _ptr(cat_inv_norms),
                     _ptr(exclude_mask), k, row_offset, path, rank, world, ptrs, epoch, n_max, vals.data_ptr(), ids.data_ptr(),
                     ws.data_ptr(), ws.numel(), _stream(dev),
+                )
+            )
+            return vals, ids
+        if exclude_bits is not None:
+            _lib.check(
+                lib.icr_cos_topk_excl(
+                    queries.data_ptr(), Q, _ld(queries), catalog.data_ptr(), N, _ld(catalog), D, dt, _ptr(cat_planes), _ptr(cat_inv_norms),
+                    _ptr(exclude_mask), exclude_bits.data_ptr(), k, row_offset, path, vals.data_ptr(), ids.data_ptr(), ws.data_ptr(),
+                    ws.numel(), _stream(dev),
                 )
             )
             return vals, ids

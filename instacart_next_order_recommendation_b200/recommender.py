@@ -5,7 +5,8 @@ Same constructor, attributes and ``recommend`` signatures as the reference
 on-disk index are unchanged. What changes is the tail: instead of
 ``cos_sim(query, catalog)[0]`` -> full ``argsort`` -> Python walk (:213-225, :250-262), one fused
 kernel scores the HBM-resident catalog and selects the top ``top_k + |excluded ∩ catalog|`` rows,
-and the walk runs over those few candidates — the observable result is identical.
+and the walk runs over those few candidates — the observable result is identical. ``recommend_batch``
+serves many requests in one encode and one fused top-k, each request with its own exclusion set.
 """
 
 from __future__ import annotations
@@ -170,6 +171,38 @@ class Recommender:
     def recommend(self, query: str, top_k: int = 10, exclude_product_ids: set[str] | None = None) -> list[tuple[str, float]]:
         """Return top-k (product_id, score) sorted by cosine similarity."""
         return self._rank(self._encode_query(query), top_k, exclude_product_ids)
+
+    def _encode_queries(self, queries: list[str]):
+        if self._query_on_device:
+            try:
+                return self.model.encode(queries, normalize_embeddings=True, convert_to_tensor=True)
+            except TypeError:
+                self._query_on_device = False
+        return self.model.encode(queries, normalize_embeddings=True)
+
+    def recommend_batch(self, queries: list[str], top_k: int = 10,
+                        exclude_product_ids: list[set[str] | None] | None = None) -> list[list[tuple[str, float]]]:
+        """``recommend`` for many requests at once: entry i equals ``recommend(queries[i], top_k, exclude_product_ids[i])``.
+
+        The queries are encoded in one ``encode`` call and ranked in one fused top-k over the resident catalog, each with
+        its own exclusion set applied on the device (``DeviceCatalog.topk(..., exclude_rows=...)``): no per-request
+        launches, and no limit on the size of an exclusion set. Unknown product ids are ignored; a request with fewer
+        eligible products than top_k gets a shorter list."""
+        queries = list(queries)
+        if exclude_product_ids is not None and len(exclude_product_ids) != len(queries):
+            raise ValueError(f"exclude_product_ids has {len(exclude_product_ids)} entries for {len(queries)} queries")
+        if not queries:
+            return []
+        n = len(self.product_ids)
+        if top_k <= 0 or n == 0:
+            return [[] for _ in queries]
+        if top_k > ops.MAX_K:
+            raise ValueError(f"top_k={top_k} exceeds the fused kernel limit {ops.MAX_K} (the reference API caps top_k at 100)")
+        excluded = [[self._pid_to_row[p] for p in (ex or ()) if p in self._pid_to_row] for ex in (exclude_product_ids or [None] * len(queries))]
+        embs = self._encode_queries(queries)
+        k = min(top_k, n)
+        vals, ids = self.catalog.topk(embs, k, exclude_rows=excluded if any(excluded) else None)
+        return [[(self.product_ids[r], float(s)) for s, r in zip(vr, ir) if r >= 0] for vr, ir in zip(vals.tolist(), ids.tolist())]
 
 
 class MonitoredRecommender(Recommender):
