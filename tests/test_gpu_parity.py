@@ -167,7 +167,7 @@ def test_dense_cos_sim_vs_oracle():
     assert (icr.cos_sim(a[0], a[1]).cpu() - oracle.cos_sim(a[0], a[1])).abs().max() < 1e-6
 
 
-@pytest.mark.parametrize("Qa,Nb,D", [(300, 5000, 384), (257, 5001, 384), (1000, 3000, 768), (64, 1024, 100)])
+@pytest.mark.parametrize("Qa,Nb,D", [(300, 5000, 384), (257, 5001, 384), (1000, 3000, 768), (64, 1024, 100), (300, 3000, 2048), (256, 2000, 4096)])
 def test_dense_cos_sim_tensor_core_path(Qa, Nb, D):
     """Large enough for the tcgen05 dense epilogue (K2'): fp32 keeps 1e-5 through the fp16 hi/lo planes."""
     a = oracle.synth_unnormalised(Qa, D, seed=13)
