@@ -46,7 +46,8 @@ typedef enum {
 typedef enum {
   ICR_F32 = 0,
   ICR_BF16 = 1,
-  ICR_F16 = 2 /* MNRL entry points only: embeddings as the reference's fp16-autocast training produces them (train_sbert.py:210,232) */
+  ICR_F16 = 2 /* embeddings as the reference's fp16-autocast training produces them (train_sbert.py:210,232); the MNRL entry
+                points, and catalogs of icr_cos_topk / icr_cos_sim_dense: 2 bytes per element like bf16, 8x finer rounding */
 } icr_dtype;
 
 /* which kernel family serves a cos_topk call */
@@ -70,7 +71,7 @@ int icr_device_supported(void);
  * Catalog preparation (once per index load; replaces the per-call re-normalisation that
  * sentence_transformers.util.cos_sim does on every /recommend,
  * reference src/inference/serve_recommendations.py:214,250).
- *   inv_norms[r] = 1 / max(||x_r||_2, 1e-12)            (F.normalize's eps)
+ *   inv_norms[r] = 1 / max(||x_r||_2, 1e-12)            (F.normalize's eps; x: ICR_F32, ICR_BF16 or ICR_F16)
  * ------------------------------------------------------------------------------------- */
 int icr_row_inv_norms(const void* x, int64_t rows, int64_t dim, int64_t ld, int dtype,
                       float* inv_norms, void* stream);
@@ -94,9 +95,10 @@ int icr_screen_plane(const float* x, int64_t rows, int64_t dim, int64_t ld,
 int64_t icr_screen_plane_row_elems(int64_t dim); /* = round_up(dim, 64) */
 
 /* Catalog upload helper: fp32 rows as the reference stores them on disk (embeddings.npy,
- * src/inference/serve_recommendations.py:127) -> the HBM-resident form: ICR_F32 or ICR_BF16
- * (round to nearest even), optionally L2-normalised first (x / max(||x||, 1e-12), the reference
- * normalises at encode time, :195-200). x and out are device pointers; dim % 4 == 0. */
+ * src/inference/serve_recommendations.py:127) -> the HBM-resident form: ICR_F32, ICR_BF16 or ICR_F16
+ * (round to nearest even, bit for bit torch's .to(); fp16 overflows to +-inf and keeps subnormals), optionally
+ * L2-normalised first (x / max(||x||, 1e-12) in fp32, the reference normalises at encode time, :195-200). x and out are
+ * device pointers; dim % 4 == 0. */
 int icr_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx,
                      void* out, int64_t ldo, int out_dtype, int normalize, void* stream);
 
@@ -110,10 +112,13 @@ int icr_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx,
  *
  *   queries      [Q, D] dtype, row stride ldq
  *   catalog      [N, D] dtype, row stride ldc          (the shard's rows when sharded)
+ *   dtype        ICR_F32, ICR_BF16 or ICR_F16, shared by queries and catalog; the 16-bit types need D % 8 == 0.
+ *                ICR_F16 scores are fp32 arithmetic on the fp16 values (products of two fp16 numbers are exact in
+ *                fp32): no screening, no re-scoring
  *   cat_planes   optional (may be NULL): the plane of icr_screen_plane(catalog), [N, round_up(D, 64)] fp16;
  *                used by the GEMM path for ICR_F32 catalogs; if NULL it is built in the workspace per call
- *   cat_inv_norms optional (may be NULL): icr_row_inv_norms(catalog); used by the GEMM path (ICR_BF16: epilogue
- *                scaling; ICR_F32: exact re-scoring of the screened rows); if NULL it is computed per call
+ *   cat_inv_norms optional (may be NULL): icr_row_inv_norms(catalog); used by the GEMM path (ICR_BF16, ICR_F16:
+ *                epilogue scaling; ICR_F32: exact re-scoring of the screened rows); if NULL it is computed per call
  *   exclude_mask optional (may be NULL): N bytes, non-zero = row never returned
  *                (exclude_product_ids semantics, serve_recommendations.py:216-221)
  *   row_offset   added to every returned id (global numbering of a row shard)
@@ -172,6 +177,7 @@ int icr_profile_collect(float* total_ms, int* launches, int* kernel_id, int* mma
 /* ---------------------------------------------------------------------------------------
  * Dense cosine similarity  ==  sentence_transformers.util.cos_sim(a, b) -> f32 [Qa, Nb]
  * (hook-compatible path: MNRL similarity_fct, evaluator score_functions).
+ * a and b share dtype: ICR_F32, ICR_BF16 or ICR_F16 (16-bit types: D % 8 == 0).
  * ------------------------------------------------------------------------------------- */
 size_t icr_cos_sim_dense_workspace_bytes(int64_t Qa, int64_t Nb, int64_t D, int dtype);
 int icr_cos_sim_dense(const void* a, int64_t Qa, int64_t lda,
@@ -219,7 +225,7 @@ int icr_peer_exchange_merge(const float* scores, const int64_t* ids, int64_t Q, 
                             const uint64_t* peer_buffers, uint32_t epoch, int64_t n_max,
                             float* out_scores, int64_t* out_ids, void* stream);
 
-/* One rank's call of a search over a ROW-SHARDED catalog: icr_cos_topk over this rank's shard (arguments as there;
+/* One rank's call of a search over a ROW-SHARDED catalog: icr_cos_topk over this rank's shard (arguments and dtypes as there;
  * row_offset = global id of the shard's first row), the exchange of every rank's [Q, k] candidates over NVLink peer memory
  * and the merge - out_scores / out_ids [Q, k] receive the GLOBAL top-k, identical on every rank. Every rank of the group
  * makes the same call (same Q, k, epoch; the shards may differ in size). Request-sized batches (Q <= 7 on the GEMV path,

@@ -87,7 +87,7 @@ int launch_gemm_dense(const void* a, int64_t Qa, int64_t lda, const void* b, int
                       int64_t ldo, void* ws, size_t ws_bytes, cudaStream_t st);
 // the tensor-core dense path pays off once there is a tile's worth of work; below that the CUDA-core kernel wins
 static bool dense_use_gemm(int64_t Qa, int64_t Nb, int64_t D, int dtype) {
-  if (dtype == ICR_BF16 && D % 8 != 0) return false;
+  if (dtype != ICR_F32 && D % 8 != 0) return false;
   return Qa >= 64 && Nb >= 1024;
 }
 
@@ -105,9 +105,9 @@ int launch_ir_metrics(const int64_t* ids, int64_t Q, int K, int64_t ld, const in
 static int elem_size(int dtype) { return dtype == ICR_F32 ? 4 : 2; }
 static int vec_elems(int dtype) { return dtype == ICR_F32 ? 4 : 8; }
 
-static int check_matrix(const char* name, const void* p, int64_t rows, int64_t dim, int64_t ld, int dtype, bool allow_f16 = false) {
-  if (dtype != ICR_F32 && dtype != ICR_BF16 && !(allow_f16 && dtype == ICR_F16)) {
-    set_error("%s: unsupported dtype %d (0 = f32, 1 = bf16%s)", name, dtype, allow_f16 ? ", 2 = f16" : "; f16 is accepted by the MNRL entry points only");
+static int check_matrix(const char* name, const void* p, int64_t rows, int64_t dim, int64_t ld, int dtype) {
+  if (dtype != ICR_F32 && dtype != ICR_BF16 && dtype != ICR_F16) {
+    set_error("%s: unsupported dtype %d (0 = f32, 1 = bf16, 2 = f16)", name, dtype);
     return ICR_ERR_DTYPE;
   }
   if (rows < 0 || dim <= 0 || ld < dim) {
@@ -239,7 +239,8 @@ int icr_screen_plane(const float* x, int64_t rows, int64_t dim, int64_t ld, uint
 
 static int resolve_path(int path, int64_t Q, int64_t N, int64_t D, int dtype, int k, const uint8_t* mask) {
   if (path == ICR_PATH_GEMV || path == ICR_PATH_GEMM) return path;
-  // small batches are HBM-bound GEMVs; larger ones are tensor-core work
+  // small batches are HBM-bound GEMVs; larger ones are tensor-core work. bf16 and fp16 rows have the same bytes and the
+  // same MMA rate, so every threshold below treats them alike
   int gemv_max_q = (dtype == ICR_F32) ? 7 : 3;
   // The tensor-core pipeline costs ~55 us of launches and selects on top of its stream, but streams a large catalog
   // closer to the HBM rate than the multi-query GEMV passes (measured, profiles/r01_notes.md): crossover ~256 MB
@@ -533,8 +534,8 @@ size_t icr_mnrl_workspace_bytes(int64_t B, int64_t D) {
 static int mnrl_common(const void* a, int64_t lda, const void* p, int64_t ldp, int64_t B, int64_t D, int dtype, void* workspace,
                        size_t workspace_bytes) {
   int rc;
-  if ((rc = check_matrix("mnrl.anchors", a, B, D, lda, dtype, true))) return rc;
-  if ((rc = check_matrix("mnrl.positives", p, B, D, ldp, dtype, true))) return rc;
+  if ((rc = check_matrix("mnrl.anchors", a, B, D, lda, dtype))) return rc;
+  if ((rc = check_matrix("mnrl.positives", p, B, D, ldp, dtype))) return rc;
   if (B < 1 || B > (1 << 24)) {
     set_error("mnrl: batch %lld outside [1, 2^24]", (long long)B);
     return ICR_ERR_ARG;
@@ -610,7 +611,7 @@ int icr_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, voi
   g_launches = 0;
   int rc = check_matrix("convert_rows.x", x, rows, dim, ldx, ICR_F32);
   if (rc) return rc;
-  if (out_dtype != ICR_F32 && out_dtype != ICR_BF16) {
+  if (out_dtype != ICR_F32 && out_dtype != ICR_BF16 && out_dtype != ICR_F16) {
     set_error("convert_rows: unsupported output dtype %d", out_dtype);
     return ICR_ERR_DTYPE;
   }
@@ -739,8 +740,8 @@ size_t icr_mnrl_rect_workspace_bytes(int64_t B, int64_t Bc, int64_t D) {
 static int mnrl_rect_common(const void* a, int64_t lda, const void* c, int64_t ldc, int64_t B, int64_t Bc, int64_t label_offset, int64_t D,
                             int dtype, void* workspace, size_t workspace_bytes) {
   int rc;
-  if ((rc = check_matrix("mnrl.anchors", a, B, D, lda, dtype, true))) return rc;
-  if ((rc = check_matrix("mnrl.candidates", c, Bc, D, ldc, dtype, true))) return rc;
+  if ((rc = check_matrix("mnrl.anchors", a, B, D, lda, dtype))) return rc;
+  if ((rc = check_matrix("mnrl.candidates", c, Bc, D, ldc, dtype))) return rc;
   if (B < 1 || Bc < 2 || label_offset < 0 || label_offset + B > Bc || D % 8 != 0 || D > 4096 || B > 65536 || Bc > (1 << 20)) {
     set_error("mnrl (rectangular): need 1 <= B <= 65536, label_offset + B <= Bc <= 2^20, D %% 8 == 0, D <= 4096; got B=%lld Bc=%lld offset=%lld D=%lld",
               (long long)B, (long long)Bc, (long long)label_offset, (long long)D);

@@ -66,6 +66,8 @@ int launch_cos_sim_dense(const void* a, int64_t Qa, int64_t lda, const void* b, 
   dim3 grid(static_cast<unsigned>((Nb + kDT - 1) / kDT), static_cast<unsigned>((Qa + kDT - 1) / kDT));
   if (dtype == ICR_F32)
     cos_sim_dense_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(a), Qa, lda, static_cast<const float*>(b), Nb, ldb, D, inva, invb, out, ldo);
+  else if (dtype == ICR_F16)
+    cos_sim_dense_kernel<__half><<<grid, 256, 0, st>>>(static_cast<const __half*>(a), Qa, lda, static_cast<const __half*>(b), Nb, ldb, D, inva, invb, out, ldo);
   else
     cos_sim_dense_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(static_cast<const __nv_bfloat16*>(a), Qa, lda, static_cast<const __nv_bfloat16*>(b), Nb, ldb, D, inva, invb, out, ldo);
   ICR_LAUNCH_CHECK();

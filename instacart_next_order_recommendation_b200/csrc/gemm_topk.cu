@@ -23,8 +23,8 @@
 //  * fp32 catalogs are swept with ONE MMA term on fp16 screening planes: rows are L2-normalised, scaled by 2^8 and
 //    rounded to fp16 (prep.cu). Screened scores are within a known band of the exact ones (select_args.cuh), so the
 //    thresholds sit that band below the k-th best, and the last select re-scores the rows inside it exactly in fp32
-//    (rescore_rank_kernel). bf16 catalogs take one MMA term on the raw rows and multiply by the two inverse norms in
-//    the epilogue.
+//    (rescore_rank_kernel). bf16 and fp16 catalogs take one MMA term on the raw rows and multiply by the two inverse
+//    norms in the epilogue.
 //  * The dense K2' path (DENSE, icr_cos_sim_dense) keeps fp32 parity for fp32 inputs: rows are split into fp16
 //    hi + lo planes, and hi*hi + hi*lo + lo*hi accumulated in fp32 reproduces the fp32 dot product to ~1e-6 relative
 //    (profiles/r01_split_precision.txt). Each pipeline stage holds the four plane tiles of one 64-wide K block, so no
@@ -70,10 +70,10 @@ struct GemmArgs {
   int tile_begin, tile_end;  // catalog tiles [begin, end) of this phase
   int chunks;                // balanced tile ranges, see chunk_first_tile
   int qblocks;               // blocks of 256 queries
-  float acc_scale;           // 2^-16 for the plane path, 1 for bf16
+  float acc_scale;           // 2^-16 for the plane path, 1 for bf16 / fp16 rows
   const float* tau;          // [Q]
-  const float* qinv;         // [Q]  (bf16 path) or null
-  const float* cinv;         // [N]  (bf16 path) or null
+  const float* qinv;         // [Q]  (bf16 / fp16 rows) or null
+  const float* cinv;         // [N]  (bf16 / fp16 rows) or null
   const uint8_t* mask;       // [N] or null
   uint64_t* cand;            // [Q][chunks * 2][seg_cap]   (segment = query x chunk x column half)
   int* cand_cnt;             // [Q][chunks * 2]
@@ -199,8 +199,8 @@ __device__ __forceinline__ float boot_tau(uint32_t ks, float band) {
 // it gathers them. Scores are in "raw" units - the accumulator itself (plane path) or accumulator * catalog inverse
 // norm (bf16 path); the per-query positive factor (2^-16, or the query's inverse norm) does not change the order
 // within a query and is applied once, to the k final scores, by the select kernel.
-// cmax / cmin: largest / smallest catalog inverse norm of these 32 rows (bf16 path).
-template <bool BF16>
+// cmax / cmin: largest / smallest catalog inverse norm of these 32 rows (SCALED: the bf16 and fp16 row paths).
+template <bool SCALED>
 __device__ __forceinline__ void filter32(const uint32_t (&r)[32], SegState& s, const float* cinv32, float cmax, float cmin, int rbase,
                                          bool fast, int N, const uint8_t* mask) {
   const float tau_f = unorder_bits(s.tau_ob);  // NaN for dead lanes: every comparison below is false
@@ -217,10 +217,10 @@ __device__ __forceinline__ void filter32(const uint32_t (&r)[32], SegState& s, c
     for (int w = 8; w > 0; w >>= 1)
 #pragma unroll
       for (int j = 0; j < w; ++j) m[j] = fmaxf(m[j], m[j + w]);
-    const float bound = BF16 ? fmaxf(m[0] * cmax, m[0] * cmin) : m[0];
+    const float bound = SCALED ? fmaxf(m[0] * cmax, m[0] * cmin) : m[0];
     if (__any_sync(kFull, bound > tau_f)) {
       float sc[32];
-      if (BF16) {
+      if (SCALED) {
 #pragma unroll
         for (int j = 0; j < 32; j += 4) {
           const float4 ci = *reinterpret_cast<const float4*>(cinv32 + j);
@@ -278,7 +278,7 @@ __device__ __forceinline__ void filter32(const uint32_t (&r)[32], SegState& s, c
     for (int j = 0; j < 32; ++j) {
       const int row = rbase + j;
       if (row < N && !(mask && mask[row])) {
-        const float sc = BF16 ? __uint_as_float(r[j]) * cinv32[j] : __uint_as_float(r[j]);
+        const float sc = SCALED ? __uint_as_float(r[j]) * cinv32[j] : __uint_as_float(r[j]);
         append_if(s, sc, tau_f, ~static_cast<uint32_t>(row));
       }
     }
@@ -286,12 +286,12 @@ __device__ __forceinline__ void filter32(const uint32_t (&r)[32], SegState& s, c
 }
 
 // K2' (dense cos_sim): same main loop, the epilogue scales and stores all 32 scores of a batch to this query's row.
-template <bool BF16>
+template <bool SCALED>
 __device__ __forceinline__ void dense_store32(const uint32_t (&r)[32], float* out_row, float qscale, const float* cinv32, int ncols,
                                               bool vec_ok) {
   float v[32];
 #pragma unroll
-  for (int j = 0; j < 32; ++j) v[j] = BF16 ? __uint_as_float(r[j]) * qscale * cinv32[j] : __uint_as_float(r[j]) * qscale;
+  for (int j = 0; j < 32; ++j) v[j] = SCALED ? __uint_as_float(r[j]) * qscale * cinv32[j] : __uint_as_float(r[j]) * qscale;
   if (ncols >= 32 && vec_ok) {
 #pragma unroll
     for (int j = 0; j < 32; j += 4) *reinterpret_cast<float4*>(out_row + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
@@ -329,7 +329,11 @@ __device__ __forceinline__ void k2_grid_barrier(unsigned int* counter, unsigned 
 // MODE = 3: fp16 hi/lo planes, three MMA terms (fp32 parity of every score): instantiated for the dense K2' path only;
 // MODE = 1: raw bf16 rows, one term, inverse norms applied in the epilogue;
 // MODE = 2: one fp16 plane of the normalised fp32 rows, one term: SCREENING scores (select_args.cuh), the survivors
-//           of the whole sweep are re-scored exactly by the last select.
+//           of the whole sweep are re-scored exactly by the last select;
+// MODE = 4: raw fp16 rows, one term, inverse norms applied in the epilogue: MODE 1 with fp16 operands. fp16 x fp16
+//           products are exact in fp32, so the scores are those of fp32 arithmetic on the fp16 values: no band, no
+//           re-scoring.
+// SCALED (MODE 1 and 4): exact scores, multiplied by the catalog's inverse norms in the epilogue.
 // ASTAT (bf16, D <= 384): the work item's 128 query rows stay resident in shared memory for all of its catalog
 // tiles ("A-stationary"), so the ring streams catalog tiles only: 31 instead of 62 B/cycle/SM of L2 traffic,
 // which is the difference between L2-bound and tensor-bound for one-term MMAs (profiles/r01_notes.md).
@@ -340,7 +344,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   constexpr int TERMS = (MODE == 3) ? 3 : 1;
   static_assert(!ASTAT || TERMS == 1, "A-stationary is a one-term variant");
   static_assert(!XB || !DENSE, "dense scores are filtered by the select");
-  constexpr bool BF16 = (MODE == 1);
+  constexpr bool SCALED = (MODE == 1 || MODE == 4);  // exact scores scaled by the catalog's inverse norms in the epilogue
   constexpr int EW = epi_warps(TERMS), EH = EW / 4, ECOLS = BN / EH;  // epilogue warps, column groups, columns per warp
   constexpr int kStageTiles = ASTAT ? 1 : ((TERMS == 3) ? 4 : 2);  // B | A_hi A_lo B_hi B_lo | A B
   constexpr int kStageBytes = kStageTiles * kTileBytes;
@@ -444,7 +448,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     // registers before every tcgen05 instruction. With a single-lane branch that traffic made the issue loop,
     // not the tensor pipe, the limit of the one-term kernels (4 MMAs per stage): profiles/r01_notes.md.
     // instruction descriptor: D=f32, A/B = f16 or bf16, K-major both, N=256, M=256 (two CTAs x 128)
-    const uint32_t fmt = BF16 ? 1u : 0u;
+    const uint32_t fmt = (MODE == 1) ? 1u : 0u;  // bf16 operands; f16 otherwise
     const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (static_cast<uint32_t>(BN >> 3) << 17) | (static_cast<uint32_t>((2 * BM) >> 4) << 24);
     // descriptors differ only in the 16-byte-unit start address (shared memory is < 256 KB: no carry out of the field)
     const uint64_t a_res0 = smem_desc_sw128(smem_u32(a_resident));
@@ -567,7 +571,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
           const int row0 = (t0 + bt) * BN + half * ECOLS;
           stage_words();
           if (bt + 1 < g.boot) load_words(q, live, row0 + BN);
-          if (BF16) {
+          if (SCALED) {
             __syncwarp();
 #pragma unroll
             for (int u = 0; u < ECOLS / 32; ++u) {
@@ -589,13 +593,13 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             float m = -INFINITY;
             if (plain) {
 #pragma unroll
-              for (int j = 0; j < 32; ++j) m = fmaxf(m, BF16 ? __uint_as_float(r[j]) * cinv_s[cb * 32 + j] : __uint_as_float(r[j]));
+              for (int j = 0; j < 32; ++j) m = fmaxf(m, SCALED ? __uint_as_float(r[j]) * cinv_s[cb * 32 + j] : __uint_as_float(r[j]));
             } else {
 #pragma unroll
               for (int j = 0; j < 32; ++j) {
                 const int row = row0 + cb * 32 + j;
                 if (row < g.N && !(g.mask && g.mask[row]))
-                  m = fmaxf(m, BF16 ? __uint_as_float(r[j]) * cinv_s[cb * 32 + j] : __uint_as_float(r[j]));
+                  m = fmaxf(m, SCALED ? __uint_as_float(r[j]) * cinv_s[cb * 32 + j] : __uint_as_float(r[j]));
               }
             }
             m_tile = fmaxf(m_tile, m);
@@ -639,14 +643,14 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
       s.tau_ob = (live && !dense) ? order_bits(__ldcg(g.tau + q)) : 0xFFFFFFFFu;
       float* out_q = dense ? g.dense_out + static_cast<int64_t>(live ? q : 0) * g.dense_ld : nullptr;
       load_words(q, live, t0 * BN + half * ECOLS);
-      const float qscale = dense ? (g.dense_raw ? 1.0f : g.acc_scale * ((BF16 && live) ? g.qinv[q] : 1.0f)) : 0.f;
+      const float qscale = dense ? (g.dense_raw ? 1.0f : g.acc_scale * ((SCALED && live) ? g.qinv[q] : 1.0f)) : 0.f;
       const bool vec_ok = dense && (g.dense_ld % 4 == 0) && ((reinterpret_cast<uintptr_t>(g.dense_out) & 15) == 0);
       for (int tile = t0; tile < t1; ++tile) {
         const int row0 = tile * BN + half * ECOLS;
         stage_words();
         if (tile + 1 < t1) load_words(q, live, row0 + BN);
         float cmax_l = 1.f, cmin_l = 1.f;  // lane u: extremes of the inverse norms of 32-row block u
-        if (BF16) {
+        if (SCALED) {
           // stage this warp's catalog inverse norms once per tile (read back as shared-memory broadcasts), with
           // the extremes of every 32-row block for the screening bound
           static_assert(ECOLS / 32 <= 32, "one lane per 32-row block");
@@ -676,21 +680,21 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
           tmem_ld_wait(ra);
           tmem_ld32(taddr + (cb + 1) * 32, rb);
           if (dense) {
-            if (live) dense_store32<BF16>(ra, out_q + row0 + cb * 32, qscale, cinv_s + cb * 32, g.N - (row0 + cb * 32), vec_ok);
+            if (live) dense_store32<SCALED>(ra, out_q + row0 + cb * 32, qscale, cinv_s + cb * 32, g.N - (row0 + cb * 32), vec_ok);
           } else {
             compact_full_segments(s, scratch, cap, g.k, lane, g.band, g.overflow, q - lane);
             if (XB) exclude32(ra, xs[cb * 32 + lane]);
-            filter32<BF16>(ra, s, cinv_s + cb * 32, __shfl_sync(kFull, cmax_l, cb), __shfl_sync(kFull, cmin_l, cb), row0 + cb * 32, fast,
+            filter32<SCALED>(ra, s, cinv_s + cb * 32, __shfl_sync(kFull, cmax_l, cb), __shfl_sync(kFull, cmin_l, cb), row0 + cb * 32, fast,
                            g.N, g.mask);
           }
           tmem_ld_wait(rb);
           if (cb + 2 < ECOLS / 32) tmem_ld32(taddr + (cb + 2) * 32, ra);
           if (dense) {
-            if (live) dense_store32<BF16>(rb, out_q + row0 + (cb + 1) * 32, qscale, cinv_s + (cb + 1) * 32, g.N - (row0 + (cb + 1) * 32), vec_ok);
+            if (live) dense_store32<SCALED>(rb, out_q + row0 + (cb + 1) * 32, qscale, cinv_s + (cb + 1) * 32, g.N - (row0 + (cb + 1) * 32), vec_ok);
           } else {
             compact_full_segments(s, scratch, cap, g.k, lane, g.band, g.overflow, q - lane);
             if (XB) exclude32(rb, xs[(cb + 1) * 32 + lane]);
-            filter32<BF16>(rb, s, cinv_s + (cb + 1) * 32, __shfl_sync(kFull, cmax_l, cb + 1), __shfl_sync(kFull, cmin_l, cb + 1),
+            filter32<SCALED>(rb, s, cinv_s + (cb + 1) * 32, __shfl_sync(kFull, cmax_l, cb + 1), __shfl_sync(kFull, cmin_l, cb + 1),
                            row0 + (cb + 1) * 32, fast, g.N, g.mask);
           }
         }
@@ -975,7 +979,7 @@ template <int MODE, bool XB = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kSwapThreads, 1)
 gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant__ CUtensorMap tma_c, const GemmArgs g,
                  const __grid_constant__ HistSelectArgs sel) {
-  constexpr bool BF16 = (MODE == 1);
+  constexpr bool SCALED = (MODE == 1 || MODE == 4);  // exact scores scaled by the catalog's inverse norms in the epilogue
   constexpr int kStageBytes = kTileBytes;
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -1053,7 +1057,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
     }
   } else if (warp == 1 && rank == 0) {
     // ================= MMA issuer: whole warp walks the loop, one elected lane issues =================
-    const uint32_t fmt = BF16 ? 1u : 0u;
+    const uint32_t fmt = (MODE == 1) ? 1u : 0u;  // bf16 operands; f16 otherwise
     const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (static_cast<uint32_t>(g.qpad >> 3) << 17) | (static_cast<uint32_t>(BN >> 4) << 24);
     const uint64_t qd0 = smem_desc_sw128(smem_u32(q_res));
     const uint64_t cd0 = smem_desc_sw128(smem_u32(stage_base));
@@ -1123,7 +1127,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
         for (int bt = 0; bt < g.boot; ++bt) {
           const int row = (t0 + bt) * BN + static_cast<int>(rank) * BNH + ew * 32 + lane;
           const bool valid = row < g.N && !(g.mask && g.mask[row]);
-          const float cinv_r = BF16 ? (row < g.N ? __ldg(g.cinv + row) : 0.f) : 1.0f;
+          const float cinv_r = SCALED ? (row < g.N ? __ldg(g.cinv + row) : 0.f) : 1.0f;
           uint32_t xw[8];
           if (XB) load_swap_words(xw, g, (row - lane) >> 5, lane);
           mbar_wait(smem_u32(&tfull_bar[acc]), acc_phase);
@@ -1186,7 +1190,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
       for (int tile = t0; tile < t1; ++tile) {
         const int row = tile * BN + wrow0 + lane;
         const bool valid = row < g.N && !(g.mask && g.mask[row]);
-        const float cinv_r = BF16 ? (row < g.N ? __ldg(g.cinv + row) : 0.f) : 1.0f;
+        const float cinv_r = SCALED ? (row < g.N ? __ldg(g.cinv + row) : 0.f) : 1.0f;
         const uint32_t nrow = ~static_cast<uint32_t>(row);
         if (XB) {
           store_swap_words(xs, xw, g.qpad, lane);
@@ -1308,8 +1312,9 @@ static_assert(kGemmSmemBytes <= 232448, "exceeds the 227 KB of shared memory a C
 constexpr size_t kSwapSmemBytes = static_cast<size_t>(kRingBytes) + 2 * 256 * 4 + 16 + (2 * kSwapMaxStages + 6) * sizeof(uint64_t) + 16 + kSwapBootBytes + 1024;
 static_assert(kSwapSmemBytes <= 232448, "exceeds the 227 KB of shared memory a CTA may use");
 
-// top-k path: MODE 1 on bf16 catalogs, MODE 2 (one-term screening + exact re-scoring of the survivors) on fp32 ones
-static int mode_for(int dtype) { return dtype == ICR_BF16 ? 1 : 2; }
+// top-k path: MODE 2 (one-term screening + exact re-scoring of the survivors) on fp32 catalogs, MODE 1 on bf16 ones,
+// MODE 4 on fp16 ones
+static int mode_for(int dtype) { return dtype == ICR_F32 ? 2 : (dtype == ICR_BF16 ? 1 : 4); }
 // keys carried per query between phases: k exact keys, or k + room for the screening band (select_args.cuh)
 static int carry_cap(int k, int mode) {
   if (mode != 2) return k;
@@ -1394,13 +1399,15 @@ constexpr int kMaxPhases = 16;
 static int dense0_tiles(int64_t Q, int64_t N) { return (Q <= 2 * BM && (N + BN - 1) / BN >= 2048) ? 16 : 4; }
 
 // kernel variants: 1 = bf16 streaming both operands, 2 = bf16 with resident queries, 5 / 6 = fp16 screen plane streaming /
-// resident queries, 4 / 7 = swapped kernel (small batches) on bf16 / the screen plane; DENSE only: 0 = fp16 hi|lo planes,
-// three MMA terms (K2' on fp32 inputs)
+// resident queries, 8 / 9 = fp16 rows streaming / resident queries, 4 / 7 / 3 = swapped kernel (small batches) on bf16 /
+// the screen plane / fp16 rows; DENSE only: 0 = fp16 hi|lo planes, three MMA terms (K2' on fp32 inputs)
 #define ICR_GEMM_VARIANTS(X, DENSE, XB)            \
   X(1, (gemm_topk_kernel<1, false, DENSE, XB>))    \
   X(2, (gemm_topk_kernel<1, true, DENSE, XB>))     \
   X(5, (gemm_topk_kernel<2, false, DENSE, XB>))    \
-  X(6, (gemm_topk_kernel<2, true, DENSE, XB>))
+  X(6, (gemm_topk_kernel<2, true, DENSE, XB>))     \
+  X(8, (gemm_topk_kernel<4, false, DENSE, XB>))    \
+  X(9, (gemm_topk_kernel<4, true, DENSE, XB>))
 
 // Launch helper of the GEMM kernels. The single-launch modes (g.boot > 0) synchronise the whole grid through a counter in
 // global memory, which needs every CTA resident at once: those launches carry the cooperative attribute, so the driver
@@ -1435,7 +1442,7 @@ static void launch_gemm_grid(void (*kernel)(KArgs...), int grid, int threads, si
 // exclusions)
 template <bool DENSE, bool XB = false>
 static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, const CUtensorMap& map_b, const GemmArgs& g, cudaStream_t st) {
-  static thread_local SmemAttrCache cache[8];
+  static thread_local SmemAttrCache cache[10];
   int rc = ICR_OK;
 #define ICR_SET(ID, K) \
   if (which == ID) rc = ensure_dyn_smem(cache[ID], K, kGemmSmemBytes);
@@ -1459,14 +1466,16 @@ static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, co
 template <bool XB = false>
 static int launch_swap_variant(int which, int grid, const CUtensorMap& map_q, const CUtensorMap& map_c, const GemmArgs& g, cudaStream_t st,
                                const HistSelectArgs& sel = HistSelectArgs{}) {
-  static thread_local SmemAttrCache cache[2];
+  static thread_local SmemAttrCache cache[3];
   int rc = ICR_OK;
   if (which == 4) rc = ensure_dyn_smem(cache[0], gemm_swap_kernel<1, XB>, kSwapSmemBytes);
   if (which == 7) rc = ensure_dyn_smem(cache[1], gemm_swap_kernel<2, XB>, kSwapSmemBytes);
+  if (which == 3) rc = ensure_dyn_smem(cache[2], gemm_swap_kernel<4, XB>, kSwapSmemBytes);
   if (rc) return rc;
   profile_begin(kKernelGemm, 1, st);
   if (which == 4) launch_gemm_grid(gemm_swap_kernel<1, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
   if (which == 7) launch_gemm_grid(gemm_swap_kernel<2, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
+  if (which == 3) launch_gemm_grid(gemm_swap_kernel<4, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
   profile_end(st);
   ICR_LAUNCH_CHECK();
   return ICR_OK;
@@ -1608,7 +1617,7 @@ static GemmWs gemm_ws_layout(int64_t Q, int64_t N, int64_t D, int dtype, int k, 
 bool gemm_topk_supported(int64_t Q, int64_t N, int64_t D, int dtype, int k, const uint8_t* mask) {
   (void)mask;
   if (Q < 1 || N < 1 || k > ICR_MAX_K) return false;
-  if (dtype == ICR_BF16 && D % 8 != 0) return false;
+  if (dtype != ICR_F32 && D % 8 != 0) return false;
   if (N > (static_cast<int64_t>(1) << 31) - BN || Q > (static_cast<int64_t>(1) << 30)) return false;
   return true;
 }
@@ -1714,8 +1723,8 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
       if ((rc = launch_row_inv_norms(catalog, N, D, ldc, dtype, built, st))) return rc;
       cinv = built;
     }
-    if ((rc = make_map(&map_a, queries, Q, D, ldq, true))) return rc;
-    if ((rc = make_map(&map_b, catalog, N, D, ldc, true))) return rc;
+    if ((rc = make_map(&map_a, queries, Q, D, ldq, mode == 1))) return rc;
+    if ((rc = make_map(&map_b, catalog, N, D, ldc, mode == 1))) return rc;
     g.kb_per_term = static_cast<int>((D + BK - 1) / BK);
     g.plane_stride = 0;
     g.acc_scale = 1.0f;
@@ -1727,8 +1736,10 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
   const bool swap = swap_applies(Q, N, D);
   const bool astat = g.kb_per_term <= kAStatMaxKB;
   int which;
-  if (swap) which = mode == 1 ? 4 : 7;
-  else which = mode == 1 ? (astat ? 2 : 1) : (astat ? 6 : 5);
+  if (swap) which = mode == 1 ? 4 : (mode == 4 ? 3 : 7);
+  else if (mode == 2) which = astat ? 6 : 5;
+  else if (mode == 1) which = astat ? 2 : 1;
+  else which = astat ? 9 : 8;
   if (swap) {
     g.qpad = static_cast<int>((Q + 31) / 32 * 32);
     if ((rc = make_map(&map_a, q_operand, Q, q_cols, q_ld, mode == 1, g.qpad / 2))) return rc;
@@ -1896,13 +1907,15 @@ int launch_gemm_dense(const void* a, int64_t Qa, int64_t lda, const void* b, int
     float* cinv = reinterpret_cast<float*>(base + align_up(static_cast<size_t>(Qa) * 4, 1024));
     if ((rc = launch_row_inv_norms(a, Qa, D, lda, dtype, qinv, st))) return rc;
     if ((rc = launch_row_inv_norms(b, Nb, D, ldb, dtype, cinv, st))) return rc;
-    if ((rc = make_map(&map_a, a, Qa, D, lda, true))) return rc;
-    if ((rc = make_map(&map_b, b, Nb, D, ldb, true))) return rc;
+    const bool bf16 = dtype == ICR_BF16;
+    if ((rc = make_map(&map_a, a, Qa, D, lda, bf16))) return rc;
+    if ((rc = make_map(&map_b, b, Nb, D, ldb, bf16))) return rc;
     g.kb_per_term = static_cast<int>((D + BK - 1) / BK);
     g.acc_scale = 1.0f;
     g.qinv = qinv;
     g.cinv = cinv;
-    which = g.kb_per_term <= kAStatMaxKB ? 2 : 1;
+    const bool astat = g.kb_per_term <= kAStatMaxKB;
+    which = bf16 ? (astat ? 2 : 1) : (astat ? 9 : 8);
   }
   // work items: (query block, chunk of tiles); enough chunks to fill the pairs a few times over
   const int npairs = kNumSMs / 2;

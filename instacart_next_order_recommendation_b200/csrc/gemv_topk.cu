@@ -969,12 +969,18 @@ static bool g_force_direct = false;  // tuning / test hook, see icr_debug_set
 
 void gemv_force_direct(bool on) { g_force_direct = on; }
 
+template <typename T>
+static int ring_slots_q(int qt, int D) {
+  return qt == 1 ? ring_slots_for<T, 1>(D) : (qt == 3 ? ring_slots_for<T, 3>(D) : ring_slots_for<T, 7>(D));
+}
+
 // contiguous rows, 16-byte aligned slabs and a ring of at least 4 slots -> bulk-copy ring kernel
 static bool ring_ok(int64_t ldc, int D, int dtype, int qt) {
   if (g_force_direct || ldc != D) return false;
   int slots;
-  if (dtype == ICR_F32) slots = qt == 1 ? ring_slots_for<float, 1>(D) : (qt == 3 ? ring_slots_for<float, 3>(D) : ring_slots_for<float, 7>(D));
-  else slots = qt == 1 ? ring_slots_for<__nv_bfloat16, 1>(D) : (qt == 3 ? ring_slots_for<__nv_bfloat16, 3>(D) : ring_slots_for<__nv_bfloat16, 7>(D));
+  if (dtype == ICR_F32) slots = ring_slots_q<float>(qt, D);
+  else if (dtype == ICR_BF16) slots = ring_slots_q<__nv_bfloat16>(qt, D);
+  else slots = ring_slots_q<__half>(qt, D);
   // one slot per warp (no load/compute overlap inside a warp) still wins for 1-3 queries per pass; 4-7 queries
   // (4-row slabs) want two slots per warp
   return qt == 7 ? slots >= 2 * kGemvWarps : slots >= kGemvWarps;
@@ -1049,7 +1055,8 @@ int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, 
     a.rows_per_cta = (N + g - 1) / g;
     int rc;
     if (dtype == ICR_F32) rc = xbits ? launch_gemv_pass<float, true>(a, qt, ring, g, st) : launch_gemv_pass<float, false>(a, qt, ring, g, st);
-    else rc = xbits ? launch_gemv_pass<__nv_bfloat16, true>(a, qt, ring, g, st) : launch_gemv_pass<__nv_bfloat16, false>(a, qt, ring, g, st);
+    else if (dtype == ICR_BF16) rc = xbits ? launch_gemv_pass<__nv_bfloat16, true>(a, qt, ring, g, st) : launch_gemv_pass<__nv_bfloat16, false>(a, qt, ring, g, st);
+    else rc = xbits ? launch_gemv_pass<__half, true>(a, qt, ring, g, st) : launch_gemv_pass<__half, false>(a, qt, ring, g, st);
     if (rc != ICR_OK) return rc;
     q0 += qt;
   }

@@ -131,6 +131,8 @@ int launch_row_inv_norms(const void* x, int64_t rows, int64_t dim, int64_t ld, i
   const int blocks = static_cast<int>(want < 148 * 16 ? want : 148 * 16);
   if (dtype == ICR_F32)
     row_inv_norms_kernel<float><<<blocks, threads, 0, st>>>(static_cast<const float*>(x), rows, dim, ld, inv, tau_init, ovf_init);
+  else if (dtype == ICR_F16)
+    row_inv_norms_kernel<__half><<<blocks, threads, 0, st>>>(static_cast<const __half*>(x), rows, dim, ld, inv, tau_init, ovf_init);
   else
     row_inv_norms_kernel<__nv_bfloat16><<<blocks, threads, 0, st>>>(static_cast<const __nv_bfloat16*>(x), rows, dim, ld, inv, tau_init, ovf_init);
   ICR_LAUNCH_CHECK();
@@ -147,8 +149,23 @@ int launch_split_planes(const float* x, int64_t rows, int64_t dim, int64_t ld, u
   return ICR_OK;
 }
 
-// Catalog upload: fp32 rows as stored on disk -> the resident form (fp32 or bf16), optionally L2-normalised first.
-// One warp per row, 128-bit loads; bf16 rounding is round-to-nearest-even (what torch's .to(bfloat16) does).
+// two fp32 values -> one word of two 16-bit elements, round to nearest even (what torch's .to(bfloat16 / float16) does;
+// fp16 overflows to +-inf and keeps subnormals)
+template <typename OUT>
+__device__ __forceinline__ uint32_t pack_rn(float lo, float hi);
+template <>
+__device__ __forceinline__ uint32_t pack_rn<__nv_bfloat16>(float lo, float hi) {
+  __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<uint32_t*>(&v);
+}
+template <>
+__device__ __forceinline__ uint32_t pack_rn<__half>(float lo, float hi) {
+  __half2 v = __floats2half2_rn(lo, hi);
+  return *reinterpret_cast<uint32_t*>(&v);
+}
+
+// Catalog upload: fp32 rows as stored on disk -> the resident form (fp32, bf16 or fp16), optionally L2-normalised first.
+// One warp per row, 128-bit loads.
 template <typename OUT>
 __global__ void __launch_bounds__(256) convert_rows_kernel(const float* __restrict__ x, int64_t rows, int64_t dim, int64_t ldx,
                                                            OUT* __restrict__ out, int64_t ldo, int normalize) {
@@ -177,13 +194,12 @@ __global__ void __launch_bounds__(256) convert_rows_kernel(const float* __restri
         f.z *= inv;
         f.w *= inv;
       }
-      if (sizeof(OUT) == 4) {
+      if constexpr (sizeof(OUT) == 4) {
         *reinterpret_cast<float4*>(dst + 4 * v) = f;
       } else {
-        __nv_bfloat162 lo = __floats2bfloat162_rn(f.x, f.y), hi = __floats2bfloat162_rn(f.z, f.w);
         uint2 pk;
-        pk.x = *reinterpret_cast<uint32_t*>(&lo);
-        pk.y = *reinterpret_cast<uint32_t*>(&hi);
+        pk.x = pack_rn<OUT>(f.x, f.y);
+        pk.y = pack_rn<OUT>(f.z, f.w);
         *reinterpret_cast<uint2*>(dst + 4 * v) = pk;
       }
     }
@@ -197,6 +213,8 @@ int launch_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, 
   const int blocks = static_cast<int>(want < 148 * 16 ? want : 148 * 16);
   if (out_dtype == ICR_F32)
     convert_rows_kernel<float><<<blocks, 256, 0, st>>>(x, rows, dim, ldx, static_cast<float*>(out), ldo, normalize);
+  else if (out_dtype == ICR_F16)
+    convert_rows_kernel<__half><<<blocks, 256, 0, st>>>(x, rows, dim, ldx, static_cast<__half*>(out), ldo, normalize);
   else
     convert_rows_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(x, rows, dim, ldx, static_cast<__nv_bfloat16*>(out), ldo, normalize);
   ICR_LAUNCH_CHECK();

@@ -14,8 +14,8 @@ over PCIe, valid only while the manifest-validated ``embeddings.npy`` it was mad
 and ``DeviceCatalog.from_index`` streams either one into HBM chunk by chunk through pinned staging
 buffers — for a whole catalog or for one rank's row block of a sharded one (SURVEY §8f row 3).
 
-``DeviceCatalog`` is what the kernels read: the same rows resident in HBM (fp32, or bf16
-on request), plus — for fp32 — the fp16 screening plane and the inverse row norms of the
+``DeviceCatalog`` is what the kernels read: the same rows resident in HBM (fp32, or bf16 or fp16
+on request), plus the inverse row norms and — for fp32 — the fp16 screening plane of the
 tensor-core path, built once at load instead of re-normalising the catalog on every request as
 ``sentence_transformers.util.cos_sim`` does (serve_recommendations.py:214).
 """
@@ -156,25 +156,48 @@ class EmbeddingIndex:
         logger.info("Saved embedding index to %s (%d products)", self._dir, len(product_ids))
 
 
+def _is_f16(x) -> bool:
+    return getattr(x, "dtype", None) in (torch.float16, np.float16)
+
+
+def _f16_matrix(x, device: torch.device) -> torch.Tensor:
+    """A float16 tensor or array as a [rows, dim] tensor on `device`, values untouched (no round trip through fp32)."""
+    t = x if isinstance(x, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(x))
+    if t.dim() == 1:
+        t = t.unsqueeze(0)
+    if t.dim() != 2:
+        raise ValueError(f"expected a vector or a [rows, dim] matrix, got shape {tuple(t.shape)}")
+    return t.to(device, non_blocking=True)
+
+
 class DeviceCatalog:
     """Catalog rows resident in HBM, with whatever the kernels want precomputed.
 
     dtype float32 keeps the reference's numerics (scores within 1e-5 of the fp32 oracle);
-    dtype bfloat16 halves the bytes a batch-1 request streams (scores within 2e-3).
+    dtype bfloat16 halves the bytes a batch-1 request streams (scores within 2e-3);
+    dtype float16 streams as many bytes as bfloat16 with 8x finer rounding: scores are fp32 arithmetic on the fp16
+    values (within 1e-5 of fp64 on them), and queries are L2-normalised in fp32 before they are rounded to fp16.
+    float16 rows must be finite: un-normalised rows beyond fp16's range raise (normalise them first).
     """
 
     def __init__(self, embeddings, *, device: torch.device | None = None, dtype: torch.dtype = torch.float32,
                  row_offset: int = 0, build_planes: bool | None = None):
-        if dtype not in (torch.float32, torch.bfloat16):
-            raise TypeError("catalog dtype must be float32 or bfloat16")
+        if dtype not in (torch.float32, torch.bfloat16, torch.float16):
+            raise TypeError("catalog dtype must be float32, bfloat16 or float16")
         dev = device if device is not None else (embeddings.device if isinstance(embeddings, torch.Tensor) and embeddings.is_cuda else default_device())
-        rows = to_device_matrix(embeddings, device=dev)  # uploaded in the dtype it has (float64 / float16 become float32)
+        if dtype == torch.float16 and _is_f16(embeddings):
+            rows = _f16_matrix(embeddings, dev)  # taken bit for bit
+        else:
+            rows = to_device_matrix(embeddings, device=dev)  # uploaded in the dtype it has (float64 / float16 become float32)
         if rows.dtype != dtype:
             if rows.dtype == torch.float32 and rows.dim() == 2 and rows.shape[1] % 4 == 0 and rows.shape[0] > 0:
                 rows = ops._rows(rows)
-                rows = ops.convert_rows(rows, torch.empty(rows.shape, dtype=dtype, device=dev))  # fp32 -> bf16 on the device (RNE)
+                rows = ops.convert_rows(rows, torch.empty(rows.shape, dtype=dtype, device=dev))  # fp32 -> bf16 / fp16 on the device (RNE)
             else:
                 rows = rows.to(dtype)
+        if dtype == torch.float16 and rows.numel() and not bool(torch.isfinite(rows).all()):
+            raise ValueError("catalog rows exceed float16's range (inf or NaN after conversion): L2-normalise them first "
+                             "(convert with normalize=True, e.g. DeviceCatalog.from_index(..., normalize=True))")
         self.input_dim = int(rows.shape[1]) if rows.dim() == 2 else 0  # before the 16-byte padding of _rows()
         self.rows = ops._rows(rows)
         self.row_offset = int(row_offset)
@@ -199,8 +222,8 @@ class DeviceCatalog:
 
         None if the index is missing or stale (the caller re-encodes, as the reference does,
         serve_recommendations.py:183-204). With dtype bfloat16 a valid ``embeddings.bf16.bin`` sidecar is uploaded
-        as is (half the bytes); otherwise the fp32 rows go up chunk by chunk and ``icr_convert_rows`` writes the
-        resident form. ``row_offset`` defaults to lo, so a row-sharded catalog returns global ids.
+        as is (half the bytes); otherwise (and always for float16) the fp32 rows go up chunk by chunk and
+        ``icr_convert_rows`` writes the resident form. ``row_offset`` defaults to lo, so a row-sharded catalog returns global ids.
         """
         emb = index.open(product_ids)
         if emb is None:
@@ -233,24 +256,37 @@ class DeviceCatalog:
     def dim(self) -> int:
         return self.rows.shape[1]
 
+    def _device_queries(self, queries) -> torch.Tensor:
+        """Queries on the catalog's device in the form its kernels take: its dtype; for float16 catalogs float16 queries
+        as given and any other dtype through ``ops.normalized_f16``."""
+        if self.dtype != torch.float16:
+            return to_device_matrix(queries, device=self.device, dtype=self.dtype)
+        if _is_f16(queries):
+            return _f16_matrix(queries, self.device)
+        return ops.normalized_f16(to_device_matrix(queries, device=self.device))
+
     @property
     def nbytes(self) -> int:
         extra = sum(t.numel() * t.element_size() for t in (self.planes, self.inv_norms) if t is not None)
         return self.rows.numel() * self.rows.element_size() + extra
 
     # ---- request-sized calls: one CUDA graph per (Q, k) -------------------------------------------------
-    def _graph_for(self, Q: int, k: int, path: int):
+    def _graph_for(self, Q: int, k: int, path: int, convert: bool = False):
         """Capture prep + scoring + select of a fixed-shape request once; replays cost one graph launch.
 
         The serve path is launch-latency-bound (a batch-1 request streams 76 MB in ~12 µs of HBM time), so the
         Python/ctypes work and the gaps between the 2-3 kernels of a call matter more than the kernels.
+        ``convert`` (float16 catalogs, queries of another dtype): the graph takes fp32 queries and its first kernel
+        normalises and rounds them (``ops.normalized_f16``).
         """
         if not hasattr(self, "_graphs"):
             self._graphs = {}
-        key = (Q, k, path)
+        key = (Q, k, path, convert)
         entry = self._graphs.get(key)
         if entry is None:
-            static_q = torch.zeros(Q, self.rows.shape[1], dtype=self.dtype, device=self.device)
+            static_q = torch.zeros(Q, self.rows.shape[1], dtype=torch.float32 if convert else self.dtype, device=self.device)
+            static_q16 = torch.empty(Q, self.rows.shape[1], dtype=torch.float16, device=self.device) if convert else None
+
             # the graph owns its workspace: zero-filled once here, then only this graph's kernels touch it, so the per-call
             # memset of the merge counter drops out of the captured sequence (ICR_PATH_WS_RESIDENT)
             lib = ops._lib.load()
@@ -258,16 +294,21 @@ class DeviceCatalog:
                                                     int(self.planes is not None))
             resident = torch.zeros(max(int(need), 256), dtype=torch.uint8, device=self.device)
             kw = dict(cat_planes=self.planes, cat_inv_norms=self.inv_norms, row_offset=self.row_offset, path=path, workspace=resident)
+
+            def call():
+                q = ops.convert_rows(static_q, static_q16, normalize=True) if convert else static_q
+                return ops.cos_topk(q, self.rows, k, **kw)
+
             side = torch.cuda.Stream(self.device)
             side.wait_stream(torch.cuda.current_stream(self.device))
             with torch.cuda.stream(side):  # warm-up outside capture: one-time attribute setting, lazy module load
-                ops.cos_topk(static_q, self.rows, k, **kw)
+                call()
             torch.cuda.current_stream(self.device).wait_stream(side)
             torch.cuda.synchronize(self.device)
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                vals, ids = ops.cos_topk(static_q, self.rows, k, **kw)
-            entry = (graph, static_q, vals, ids, resident)
+                vals, ids = call()
+            entry = (graph, static_q, vals, ids, resident, static_q16)
             self._graphs[key] = entry
         return entry
 
@@ -297,7 +338,8 @@ class DeviceCatalog:
                 vals, ids = self._prepared_call(q, k, path)
                 return (vals.clone(), ids.clone()) if copy else (vals, ids)
         with self.request_lock:
-            graph, static_q, vals, ids, _ = self._graph_for(q.shape[0], k, path)
+            convert = self.dtype == torch.float16 and q.dtype != torch.float16
+            graph, static_q, vals, ids = self._graph_for(q.shape[0], k, path, convert)[:4]
             D = q.shape[1]  # columns beyond the catalog's own dim are the zero padding of _rows(); they stay zero
             static_q[:, :D].copy_(q, non_blocking=True)  # H2D (or D2D) + dtype conversion in one op
             graph.replay()
@@ -444,8 +486,7 @@ class DeviceCatalog:
         for (lo, hi), (qd, ev) in zip(bounds, staged):
             rank.wait_event(ev)
             with torch.cuda.stream(rank):
-                if qd.dtype != self.dtype:
-                    qd = qd.to(self.dtype)
+                qd = ops._like_catalog(qd, self.dtype)
                 v, i = ops.cos_topk(qd, self.rows, k, cat_planes=self.planes, cat_inv_norms=self.inv_norms,
                                     row_offset=self.row_offset, path=path)
                 v.record_stream(down)
@@ -487,7 +528,7 @@ class DeviceCatalog:
             # request-sized device query in the catalog's layout: the prepared argument list of the request path, fresh outputs
             with self.request_lock:
                 return self._prepared_call(q, int(k), path, fresh_out=True)
-        q = to_device_matrix(queries, device=self.device, dtype=self.dtype)
+        q = self._device_queries(queries)
         if peer is not None and int(k) > len(self):
             raise ValueError("a sharded call needs k <= the shard's rows (pad the shard's own lists and use peer_exchange_merge instead)")
         k = min(int(k), len(self))
@@ -500,7 +541,7 @@ class DeviceCatalog:
     def _topk_excluding(self, queries, k: int, exclude_rows, exclude_mask, path: int, peer):
         if peer is not None:
             raise ValueError("exclude_rows is not supported on a sharded call")
-        q = to_device_matrix(queries, device=self.device, dtype=self.dtype)
+        q = self._device_queries(queries)
         if q.dim() == 1:
             q = q.unsqueeze(0)
         Q = q.shape[0]

@@ -13,14 +13,14 @@ import torch
 from . import _lib
 from ._lib import ICR_BF16, ICR_F16, ICR_F32, MAX_K, PATH_AUTO, PATH_GEMM, PATH_GEMV, PATH_WS_RESIDENT  # noqa: F401
 
-_DTYPES = {torch.float32: ICR_F32, torch.bfloat16: ICR_BF16, torch.float16: ICR_F16}  # float16: MNRL entry points only
+_DTYPES = {torch.float32: ICR_F32, torch.bfloat16: ICR_BF16, torch.float16: ICR_F16}
 
 
 def _dtype_code(t: torch.Tensor) -> int:
     try:
         return _DTYPES[t.dtype]
     except KeyError:
-        raise TypeError(f"libicr_b200 supports float32 and bfloat16 embeddings (float16 for the MNRL loss only), got {t.dtype}") from None
+        raise TypeError(f"libicr_b200 supports float32, bfloat16 and float16 embeddings, got {t.dtype}") from None
 
 
 def _require_cuda(name: str, t: torch.Tensor) -> None:
@@ -143,7 +143,8 @@ def screen_plane(x: torch.Tensor, *, with_inv_norms: bool = True):
 
 
 def convert_rows(x: torch.Tensor, out: torch.Tensor, *, normalize: bool = False) -> torch.Tensor:
-    """fp32 device rows -> `out` (float32 or bfloat16 device rows of the same shape), optionally L2-normalised first."""
+    """fp32 device rows -> `out` (float32, bfloat16 or float16 device rows of the same shape), optionally L2-normalised
+    first. The rounding is round-to-nearest-even, bit for bit torch's ``.to(out.dtype)``."""
     _require_cuda("x", x)
     _require_cuda("out", out)
     if x.dtype != torch.float32 or x.dim() != 2 or out.shape != x.shape or x.stride(1) != 1 or out.stride(1) != 1:
@@ -153,6 +154,28 @@ def convert_rows(x: torch.Tensor, out: torch.Tensor, *, normalize: bool = False)
         _lib.check(lib.icr_convert_rows(x.data_ptr(), x.shape[0], x.shape[1], _ld(x), out.data_ptr(), _ld(out), _dtype_code(out), int(normalize),
                                         _stream(x.device)))
     return out
+
+
+def normalized_f16(x: torch.Tensor) -> torch.Tensor:
+    """Device rows -> float16 [rows, round_up(dim, 8)]: L2-normalised in fp32, then rounded (one ``icr_convert_rows``).
+
+    The form queries take against a float16 catalog. Cosine does not depend on a row's scale, while a plain
+    ``.to(float16)`` of un-normalised fp32 rows overflows to inf or flushes to zero. The padding columns are zero."""
+    _require_cuda("x", x)
+    if x.dim() != 2:
+        raise ValueError(f"expected a [rows, dim] matrix, got shape {tuple(x.shape)}")
+    x = x.float()
+    if x.shape[1] % 8:
+        x = torch.nn.functional.pad(x, (0, 8 - x.shape[1] % 8))
+    x = _rows(x)
+    return convert_rows(x, torch.empty(x.shape, dtype=torch.float16, device=x.device), normalize=True)
+
+
+def _like_catalog(q: torch.Tensor, catalog_dtype: torch.dtype) -> torch.Tensor:
+    """Queries in the catalog's dtype: float16 catalogs take normalised-then-rounded queries (``normalized_f16``)."""
+    if q.dtype == catalog_dtype:
+        return q
+    return normalized_f16(q) if catalog_dtype == torch.float16 else q.to(catalog_dtype)
 
 
 def exclusion_words(n_rows: int) -> int:
@@ -214,7 +237,8 @@ def cos_topk(
 ):
     """(values f32 [Q,k] descending, ids int64 [Q,k]) == torch.topk(cos_sim(q, c), k, dim=1).
 
-    ``exclude_mask`` (uint8/bool [N]) drops rows for every query; ``exclude_bits`` (``query_exclusion_bits``, uint32
+    The catalog is float32, bfloat16 or float16; queries of another dtype are converted to the catalog's (for float16:
+    ``normalized_f16``). ``exclude_mask`` (uint8/bool [N]) drops rows for every query; ``exclude_bits`` (``query_exclusion_bits``, uint32
     [ceil(N/32), Q]) drops rows per query. A row is dropped when either says so; queries with fewer than k eligible rows
     get a (-inf, -1) tail.
 
@@ -223,9 +247,7 @@ def cos_topk(
     (``icr_cos_topk_sharded``): the outputs are the GLOBAL top-k, identical on every rank. Collective: every rank calls."""
     _require_cuda("queries", queries)
     _require_cuda("catalog", catalog)
-    if queries.dtype != catalog.dtype:
-        queries = queries.to(catalog.dtype)
-    queries, catalog = _rows(queries), _rows(catalog)
+    queries, catalog = _rows(_like_catalog(queries, catalog.dtype)), _rows(catalog)
     if queries.shape[1] != catalog.shape[1]:
         raise ValueError(f"embedding dims differ: {queries.shape[1]} vs {catalog.shape[1]}")
     Q, D = queries.shape
@@ -317,12 +339,10 @@ def lib_call(name: str):
 
 
 def cos_sim_dense(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
-    """f32 [Qa, Nb] cosine similarity matrix."""
+    """f32 [Qa, Nb] cosine similarity matrix. `a` is converted to b's dtype as ``cos_topk`` converts queries."""
     _require_cuda("a", a)
     _require_cuda("b", b)
-    if a.dtype != b.dtype:
-        a = a.to(b.dtype)
-    a, b = _rows(a), _rows(b)
+    a, b = _rows(_like_catalog(a, b.dtype)), _rows(b)
     if a.shape[1] != b.shape[1]:
         raise ValueError(f"embedding dims differ: {a.shape[1]} vs {b.shape[1]}")
     lib = _lib.load()

@@ -66,7 +66,8 @@ class Recommender:
         # host copy kept because callers read `.product_embeddings` (routes, tests/conftest.py:34-49)
         self.product_embeddings = self._load_or_build_embeddings(batch_size, use_index)
         if catalog_dtype is None:
-            catalog_dtype = torch.bfloat16 if os.getenv("ICR_CATALOG_DTYPE", "fp32").lower() in ("bf16", "bfloat16") else torch.float32
+            env = os.getenv("ICR_CATALOG_DTYPE", "fp32").lower()
+            catalog_dtype = {"bf16": torch.bfloat16, "bfloat16": torch.bfloat16, "fp16": torch.float16, "float16": torch.float16}.get(env, torch.float32)
         dev = torch.device(device) if device is not None else None
         self.catalog = DeviceCatalog(self.product_embeddings, device=dev, dtype=catalog_dtype)
         # SURVEY §8f row 1: ask the encoder for a device tensor so that the query never visits the host between the

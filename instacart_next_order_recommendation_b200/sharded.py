@@ -16,7 +16,7 @@ import torch
 import torch.distributed as dist
 
 from . import _lib, ops
-from .index import DeviceCatalog, to_device_matrix
+from .index import DeviceCatalog
 
 
 def shard_bounds(n_rows: int, world_size: int, rank: int) -> tuple[int, int]:
@@ -216,7 +216,7 @@ class ShardedCatalog:
         if self.exchange == "peer" and self.world_size > 1 and self._local_topk is None and 1 <= k <= self.n_local:
             # one library call: the shard's search with the exchange and the merge behind it - a single launch for request-sized
             # batches (icr_cos_topk_sharded). Ranks whose shard is shorter than k take the route below; the protocols mix.
-            q = to_device_matrix(queries, device=self.device, dtype=self.local.dtype)
+            q = self.local._device_queries(queries)
             return self.local.topk(q, k, peer=self._peer_for(q.shape[0] * k).next_call())
         vals, ids = self.local_topk(queries, k)
         return self.exchange_merge(vals, ids, k)
