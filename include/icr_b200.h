@@ -46,8 +46,10 @@ typedef enum {
 typedef enum {
   ICR_F32 = 0,
   ICR_BF16 = 1,
-  ICR_F16 = 2 /* embeddings as the reference's fp16-autocast training produces them (train_sbert.py:210,232); the MNRL entry
-                points, and catalogs of icr_cos_topk / icr_cos_sim_dense: 2 bytes per element like bf16, 8x finer rounding */
+  ICR_F16 = 2, /* embeddings as the reference's fp16-autocast training produces them (train_sbert.py:210,232); the MNRL entry
+                 points, and catalogs of icr_cos_topk / icr_cos_sim_dense: 2 bytes per element like bf16, 8x finer rounding */
+  ICR_I8 = 3   /* catalogs of the fused top-k only (icr_cos_topk, icr_cos_topk_excl, icr_cos_topk_sharded): per-row int8 codes
+                  with one fp32 factor per row, icr_quantize_rows. Every other entry point returns ICR_ERR_DTYPE */
 } icr_dtype;
 
 /* which kernel family serves a cos_topk call */
@@ -102,6 +104,15 @@ int64_t icr_screen_plane_row_elems(int64_t dim); /* = round_up(dim, 64) */
 int icr_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx,
                      void* out, int64_t ldo, int out_dtype, int normalize, void* stream);
 
+/* fp32 rows -> int8 codes + one factor per row (per-row symmetric scalar quantisation, the format of ICR_I8 catalogs):
+ *   m = max |x_i|;  c_i = clamp(rint(127 * (x_i / m)), -127, 127);  factors[r] = (m / 127) / max(||x_r||, 1e-12)
+ * in fp32 with round-to-nearest at every step (an all-zero row has zero codes and factor 0). The factor carries the row's
+ * inverse norm: cosine needs no separate normalisation. codes [rows, ldc] int8, ldc >= round_up(dim, 16) and a multiple of
+ * 16, 16-byte aligned; the columns past dim are written as zero. dim % 4 == 0. One launch. icr_cos_topk quantises its fp32
+ * queries with the same code, so a query and a catalog row quantise to the same bits. */
+int icr_quantize_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, int8_t* codes, int64_t ldc, float* factors,
+                      void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Fused cosine top-k  ==  torch.topk(cos_sim(queries, catalog), k, dim=1, sorted=True)
  * with ties broken by the lower catalog row.
@@ -118,7 +129,13 @@ int icr_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx,
  *   cat_planes   optional (may be NULL): the plane of icr_screen_plane(catalog), [N, round_up(D, 64)] fp16;
  *                used by the GEMM path for ICR_F32 catalogs; if NULL it is built in the workspace per call
  *   cat_inv_norms optional (may be NULL): icr_row_inv_norms(catalog); used by the GEMM path (ICR_BF16, ICR_F16:
- *                epilogue scaling; ICR_F32: exact re-scoring of the screened rows); if NULL it is computed per call
+ *                epilogue scaling; ICR_F32: exact re-scoring of the screened rows); if NULL it is computed per call.
+ *                ICR_I8: REQUIRED (NULL is ICR_ERR_ARG), 16-byte aligned: the catalog's factors from icr_quantize_rows
+ *   ICR_I8       catalog = int8 codes [N, D], D % 16 == 0, ldc in bytes, 16-byte rows; queries = FP32 [Q, D] (ldq in fp32
+ *                elements), quantised by the call itself as icr_quantize_rows does; cat_planes is ignored. With S the exact
+ *                int32 dot product of the codes, rows are ranked by key = fp32(S) * f_row (ties: lower row) and the
+ *                returned score is key * f_query (fp32, round to nearest), the same bits on the GEMV and the tensor-core
+ *                path (tcgen05 kind::i8, s32 accumulators). The plan treats the call as an ICR_F16 call of the same shape
  *   exclude_mask optional (may be NULL): N bytes, non-zero = row never returned
  *                (exclude_product_ids semantics, serve_recommendations.py:216-221)
  *   row_offset   added to every returned id (global numbering of a row shard)

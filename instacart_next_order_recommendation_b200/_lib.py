@@ -17,7 +17,7 @@ import os
 # `python -m ...build --trace`); the default is the library build() produces
 LIB_PATH = Path(os.environ.get("ICR_B200_LIB") or Path(__file__).resolve().parent / "lib" / "libicr_b200.so")
 
-ICR_F32, ICR_BF16, ICR_F16 = 0, 1, 2
+ICR_F32, ICR_BF16, ICR_F16, ICR_I8 = 0, 1, 2, 3  # ICR_I8: top-k catalogs only (codes + factors of icr_quantize_rows)
 PATH_AUTO, PATH_GEMV, PATH_GEMM = 0, 1, 2
 PATH_WS_RESIDENT = 0x100  # OR-ed into a path: resident workspace, see include/icr_b200.h
 MAX_K = 256
@@ -47,6 +47,7 @@ SIGNATURES = {
     "icr_screen_plane": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p]),
     "icr_screen_plane_row_elems": (c_int64, [c_int64]),
     "icr_convert_rows": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_int, c_int, c_void_p]),
+    "icr_quantize_rows": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p]),
     "icr_cos_topk_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int, c_int, c_int, c_int]),
     "icr_cos_topk": (
         c_int,

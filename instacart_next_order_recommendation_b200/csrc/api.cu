@@ -57,6 +57,8 @@ int launch_screen_plane(const float* x, int64_t rows, int64_t dim, int64_t ld, u
                         unsigned int* ovf_init = nullptr);
 int launch_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, void* out, int64_t ldo, int out_dtype, int normalize,
                         cudaStream_t st);
+int launch_quantize_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, int8_t* codes, int64_t ldc, float* factors, cudaStream_t st,
+                         float* tau_init = nullptr, unsigned int* ovf_init = nullptr);
 int launch_peer_exchange_merge(const float* scores, const int64_t* ids, int64_t Q, int k, const PeerTail& peer, float* os, int64_t* oi,
                                cudaStream_t st);
 bool gemv_peer_tail_fits(int Q, int k, int world);
@@ -107,7 +109,7 @@ static int vec_elems(int dtype) { return dtype == ICR_F32 ? 4 : 8; }
 
 static int check_matrix(const char* name, const void* p, int64_t rows, int64_t dim, int64_t ld, int dtype) {
   if (dtype != ICR_F32 && dtype != ICR_BF16 && dtype != ICR_F16) {
-    set_error("%s: unsupported dtype %d (0 = f32, 1 = bf16, 2 = f16)", name, dtype);
+    set_error("%s: unsupported dtype %d (0 = f32, 1 = bf16, 2 = f16; int8 rows are top-k catalogs only)", name, dtype);
     return ICR_ERR_DTYPE;
   }
   if (rows < 0 || dim <= 0 || ld < dim) {
@@ -124,6 +126,23 @@ static int check_matrix(const char* name, const void* p, int64_t rows, int64_t d
   }
   if ((reinterpret_cast<uintptr_t>(p) & 15) != 0 || (ld * elem_size(dtype)) % 16 != 0) {
     set_error("%s: base pointer and row stride must be 16-byte aligned", name);
+    return ICR_ERR_ALIGN;
+  }
+  return ICR_OK;
+}
+
+// int8 codes (ICR_I8) of a top-k catalog: 16 codes per 16-byte vector, rows 16-byte aligned
+static int check_codes(const char* name, const void* p, int64_t rows, int64_t dim, int64_t ld) {
+  if (rows < 0 || dim <= 0 || ld < dim) {
+    set_error("%s: bad shape rows=%lld dim=%lld ld=%lld", name, (long long)rows, (long long)dim, (long long)ld);
+    return ICR_ERR_ARG;
+  }
+  if (rows > 0 && p == nullptr) {
+    set_error("%s: null pointer", name);
+    return ICR_ERR_ARG;
+  }
+  if (dim % 16 != 0 || ld % 16 != 0 || (reinterpret_cast<uintptr_t>(p) & 15) != 0) {
+    set_error("%s: int8 rows need dim %% 16 == 0 (got %lld) and a 16-byte aligned base and row stride", name, (long long)dim);
     return ICR_ERR_ALIGN;
   }
   return ICR_OK;
@@ -240,20 +259,22 @@ int icr_screen_plane(const float* x, int64_t rows, int64_t dim, int64_t ld, uint
 static int resolve_path(int path, int64_t Q, int64_t N, int64_t D, int dtype, int k, const uint8_t* mask) {
   if (path == ICR_PATH_GEMV || path == ICR_PATH_GEMM) return path;
   // small batches are HBM-bound GEMVs; larger ones are tensor-core work. bf16 and fp16 rows have the same bytes and the
-  // same MMA rate, so every threshold below treats them alike
-  int gemv_max_q = (dtype == ICR_F32) ? 7 : 3;
+  // same MMA rate, so every threshold below treats them alike. int8 rows are planned as fp16 rows of the same shape (the
+  // crossover has not been re-tuned for their half bytes and double MMA rate)
+  const int plan = dtype == ICR_I8 ? ICR_F16 : dtype;
+  int gemv_max_q = (plan == ICR_F32) ? 7 : 3;
   // The tensor-core pipeline costs ~55 us of launches and selects on top of its stream, but streams a large catalog
   // closer to the HBM rate than the multi-query GEMV passes (measured, profiles/r01_notes.md): crossover ~256 MB
   // for 4-7 queries, ~640 MB for 2-3.
-  const double cat_bytes = static_cast<double>(N) * static_cast<double>(D) * (dtype == ICR_F32 ? 4.0 : 2.0);
+  const double cat_bytes = static_cast<double>(N) * static_cast<double>(D) * (plan == ICR_F32 ? 4.0 : 2.0);
   if (cat_bytes >= 256e6 && gemv_max_q > 3) gemv_max_q = 3;
   // 2 GB catalogs, whole call: fp32 rows, 2-3 queries: one GEMV pass 0.36 ms against 0.40 ms on the tensor path (the pass
   // re-uses each row for all its queries and fp32 needs no unpacking); bf16 rows: 0.43 ms against 0.39 ms
-  if (cat_bytes >= 640e6) gemv_max_q = (dtype == ICR_F32) ? 3 : 1;
+  if (cat_bytes >= 640e6) gemv_max_q = (plan == ICR_F32) ? 3 : 1;
   // rows shorter than 512 bytes leave the GEMV kernel instruction-bound even for one query (per-row reduction and
   // threshold test against 256 bytes of FMAs: 20 % of the HBM rate measured at D=128 bf16); the swapped tensor-core
   // kernel streams such a catalog at 74 % with the query padded to N=32
-  if (cat_bytes >= 640e6 && D * (dtype == ICR_F32 ? 4 : 2) < 512) gemv_max_q = 0;
+  if (cat_bytes >= 640e6 && D * (plan == ICR_F32 ? 4 : 2) < 512) gemv_max_q = 0;
   if (Q > gemv_max_q && gemm_topk_supported(Q, N, D, dtype, k, mask)) return ICR_PATH_GEMM;
   return ICR_PATH_GEMV;
 }
@@ -279,8 +300,21 @@ static int cos_topk_impl(const void* queries, int64_t Q, int64_t ldq, const void
                          int64_t row_offset, int path, float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes,
                          void* stream, const PeerTail* peer, float* stage_scores, int64_t* stage_ids) {
   int rc;
-  if ((rc = check_matrix("cos_topk.queries", queries, Q, D, ldq, dtype))) return rc;
-  if ((rc = check_matrix("cos_topk.catalog", catalog, N, D, ldc, dtype))) return rc;
+  if (dtype == ICR_I8) {  // fp32 queries, quantised by the call; the catalog's codes come with their factors
+    if ((rc = check_matrix("cos_topk.queries", queries, Q, D, ldq, ICR_F32))) return rc;
+    if ((rc = check_codes("cos_topk.catalog", catalog, N, D, ldc))) return rc;
+    if (N > 0 && !cat_inv_norms) {
+      set_error("cos_topk: an int8 catalog needs its factors in cat_inv_norms (icr_quantize_rows)");
+      return ICR_ERR_ARG;
+    }
+    if ((reinterpret_cast<uintptr_t>(cat_inv_norms) & 15) != 0) {
+      set_error("cos_topk: the factors of an int8 catalog must be 16-byte aligned");
+      return ICR_ERR_ALIGN;
+    }
+  } else {
+    if ((rc = check_matrix("cos_topk.queries", queries, Q, D, ldq, dtype))) return rc;
+    if ((rc = check_matrix("cos_topk.catalog", catalog, N, D, ldc, dtype))) return rc;
+  }
   if (k < 1 || k > ICR_MAX_K) {
     set_error("cos_topk: k=%d outside [1, %d]", k, ICR_MAX_K);
     return ICR_ERR_K;
@@ -338,7 +372,7 @@ static int cos_topk_impl(const void* queries, int64_t Q, int64_t ldq, const void
   w += align_up(static_cast<size_t>(qc) * grid * sizeof(int), 256);
   w += align_up(select_scratch_bytes(qc, grid, k, k), 256);
   unsigned int* done_counter = reinterpret_cast<unsigned int*>(w);
-  const size_t esz = elem_size(dtype);
+  const size_t esz = dtype == ICR_I8 ? sizeof(float) : elem_size(dtype);  // of a query element
   // the last CTA of every GEMV launch merges the per-CTA lists itself (no select launch on the latency path)
   if (!ws_resident) ICR_CUDA_CHECK(cudaMemsetAsync(done_counter, 0, 2 * sizeof(unsigned int), st));  // ticket + slab-chunk counter
   if (peer)  // the merging CTA of the one GEMV launch also exchanges and merges (gemv_topk.cu peer_tail_merge)
@@ -604,6 +638,18 @@ int icr_mnrl_bwd(const void* a, int64_t lda, const void* p, int64_t ldp, int64_t
   g.ldgp = ldgp;
   if (mnrl_use_tc(B, D, dtype)) return launch_mnrl_tc(g, dtype, 1, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
   return launch_mnrl_dispatch(g, dtype, true, static_cast<cudaStream_t>(stream));
+}
+
+int icr_quantize_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, int8_t* codes, int64_t ldc, float* factors, void* stream) {
+  g_launches = 0;
+  int rc = check_matrix("quantize_rows.x", x, rows, dim, ldx, ICR_F32);
+  if (rc) return rc;
+  if (rows > 0 && (!codes || !factors || ldc < (dim + 15) / 16 * 16 || ldc % 16 != 0 || (reinterpret_cast<uintptr_t>(codes) & 15))) {
+    set_error("quantize_rows: codes and factors must be non-null, codes 16-byte aligned with a row stride >= round_up(dim, 16) and a multiple of 16");
+    return ICR_ERR_ALIGN;
+  }
+  if ((rc = check_device())) return rc;
+  return launch_quantize_rows(x, rows, dim, ldx, codes, ldc, factors, static_cast<cudaStream_t>(stream));
 }
 
 int icr_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, void* out, int64_t ldo, int out_dtype, int normalize,

@@ -119,6 +119,56 @@ struct Exclusions {
   }
 };
 
+// ---- int8 rows (ICR_I8) -----------------------------------------------------------------------
+// Per-row symmetric scalar quantisation. For an fp32 row x of D elements (D % 4 == 0, 16-byte aligned):
+//   m  = max |x_i|,  n2 = sum x_i^2 (lane l accumulates, with fmaf in increasing i, the elements of its float4 vectors
+//        l, l + 32, ...; then an xor-shuffle tree 16, 8, 4, 2, 1)
+//   m == 0: every code and the factor are 0; otherwise
+//   c_i = clamp(rint(127 * (x_i / m)), -127, 127),   f = (m / 127) / max(sqrt(n2), 1e-12)
+// with every operation an explicit round-to-nearest intrinsic, so that compiler flags cannot change a bit. The factor
+// carries the row's 1 / |x|: the key of row r for query q is fp32(S) * f_r with S the exact int32 dot product of the
+// codes, and the score is key * f_q. The quantise kernel, the GEMV prologue and every other site call this one function,
+// so codes and factors are bit-identical wherever a row is quantised.
+struct I8Rows {
+  // Warp-level (all 32 lanes): quantises x[0, D) and returns the factor on every lane. `store(w, word)` receives the
+  // packed codes - word w holds codes 4w .. 4w+3, lowest byte first - for w in [0, nwords); words past D / 4 are zero.
+  template <typename Store>
+  __device__ static __forceinline__ float quantize(const float* x, int D, int nwords, int lane, Store store) {
+    const int nvec = D / 4;
+    const float4* xv = reinterpret_cast<const float4*>(x);
+    float m = 0.f, n2 = 0.f;
+    for (int v = lane; v < nvec; v += 32) {
+      const float4 f = __ldg(xv + v);
+      m = fmaxf(m, fmaxf(fmaxf(fabsf(f.x), fabsf(f.y)), fmaxf(fabsf(f.z), fabsf(f.w))));
+      n2 = __fmaf_rn(f.x, f.x, n2);
+      n2 = __fmaf_rn(f.y, f.y, n2);
+      n2 = __fmaf_rn(f.z, f.z, n2);
+      n2 = __fmaf_rn(f.w, f.w, n2);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      m = fmaxf(m, __shfl_xor_sync(kFull, m, o));
+      n2 = __fadd_rn(n2, __shfl_xor_sync(kFull, n2, o));
+    }
+    for (int w = lane; w < nwords; w += 32) {
+      uint32_t word = 0u;
+      if (w < nvec && m > 0.f) {
+        const float4 f = __ldg(xv + w);
+        const float e[4] = {f.x, f.y, f.z, f.w};
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const int c = min(127, max(-127, __float2int_rn(__fmul_rn(127.f, __fdiv_rn(e[i], m)))));
+          word |= (static_cast<uint32_t>(c) & 0xffu) << (8 * i);
+        }
+      }
+      store(w, word);
+    }
+    return m > 0.f ? __fdiv_rn(__fdiv_rn(m, 127.f), fmaxf(__fsqrt_rn(n2), kNormEps)) : 0.f;
+  }
+  // ranking key of a row with exact code dot product S and factor f (the returned score is key * f_query)
+  __device__ static __forceinline__ float key(int S, float f) { return __fmul_rn(__int2float_rn(S), f); }
+};
+
 // ---- vector loads -------------------------------------------------------------------------
 // streaming 128-bit load: read-only path, do not allocate in L1 (catalog rows are used once)
 __device__ __forceinline__ uint4 ldg_stream(const void* p) {
@@ -180,6 +230,12 @@ struct Elem<__half> {
   __device__ static __forceinline__ __half from_f32(float x) { return __float2half_rn(x); }
 };
 
+// int8 codes (ICR_I8): 16 per 16-byte load, consumed as packed words by __dp4a (gemv_topk.cu), never unpacked
+template <>
+struct Elem<int8_t> {
+  static constexpr int VEC = 16;
+};
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(kFull, v, o);
@@ -193,9 +249,9 @@ __device__ __forceinline__ float warp_max(float v) {
 
 // Transposing warp reduction: every lane holds V partial sums acc[0..V); on return lane l
 // holds in acc[0] the full 32-lane sum of value index (l >> (5 - log2 V)). V shuffles in
-// total instead of 5*V.
-template <int V>
-__device__ __forceinline__ void warp_transpose_reduce(float (&acc)[V], int lane) {
+// total instead of 5*V. Integer partial sums (int8 rows) reduce exactly, in any order.
+template <int V, typename A = float>
+__device__ __forceinline__ void warp_transpose_reduce(A (&acc)[V], int lane) {
   static_assert(V == 1 || V == 2 || V == 4 || V == 8 || V == 16 || V == 32, "V must be a power of two <= 32");
   int off = 16;
 #pragma unroll
@@ -203,8 +259,8 @@ __device__ __forceinline__ void warp_transpose_reduce(float (&acc)[V], int lane)
     const bool upper = (lane & off) != 0;
 #pragma unroll
     for (int i = 0; i < n / 2; ++i) {
-      const float send = upper ? acc[i] : acc[i + n / 2];
-      const float keep = upper ? acc[i + n / 2] : acc[i];
+      const A send = upper ? acc[i] : acc[i + n / 2];
+      const A keep = upper ? acc[i + n / 2] : acc[i];
       acc[i] = keep + __shfl_xor_sync(kFull, send, off);
     }
   }

@@ -175,6 +175,28 @@ __device__ __forceinline__ void append_if(SegState& s, float sc, float tau_f, ui
   s.cnt += static_cast<int>(inc);
 }
 
+// MODE 5 (int8 rows): the accumulators are exact s32 dot products; converted once after each TMEM load (__int2float_rn, the
+// rounding K1 applies too), every consumer below reads fp32 bits as for the other modes
+template <int MODE>
+__device__ __forceinline__ void acc_to_f32(uint32_t (&r)[32]) {
+  if constexpr (MODE == 5) {
+#pragma unroll
+    for (int j = 0; j < 32; ++j) r[j] = __float_as_uint(__int2float_rn(static_cast<int>(r[j])));
+  }
+}
+// the one-term MMA of a mode: kind::i8 for int8 rows, kind::f16 (f16 / bf16 operands) otherwise
+template <int MODE>
+__device__ __forceinline__ void umma_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  if constexpr (MODE == 5) umma_i8_pair(d_tmem, adesc, bdesc, idesc, accumulate);
+  else umma_f16_pair(d_tmem, adesc, bdesc, idesc, accumulate);
+}
+// instruction descriptor bits 4-12: D format (1 = F32, 2 = S32) and the A / B formats (kind::f16: 0 = F16, 1 = BF16;
+// kind::i8: 1 = signed 8-bit)
+template <int MODE>
+__host__ __device__ constexpr uint32_t idesc_formats() {
+  return MODE == 5 ? ((2u << 4) | (1u << 7) | (1u << 10)) : ((1u << 4) | ((MODE == 1 ? 1u : 0u) << 7) | ((MODE == 1 ? 1u : 0u) << 10));
+}
+
 // Per-query exclusions (XB kernels): the accumulators of the rows that this thread's bitmap word `w` excludes become -inf
 // before any filter, maximum or bound sees them. Every filter is a strict ">", which never admits -inf (not even against
 // the first phase's tau = -inf), so the fast paths stay as they are; a warp whose 32 words are all zero skips the selects.
@@ -188,10 +210,13 @@ __device__ __forceinline__ void exclude32(uint32_t (&r)[32], uint32_t w) {
 // Bootstrap threshold from the k-th largest group maximum `ks` (order bits): one ulp below it, minus the screening band.
 // XB kernels: a query with fewer than k eligible groups (rows excluded) has a k-th maximum of -inf, and its threshold
 // is -inf rather than the NaN one ulp below -inf would give (which no score passes).
+// A k-th maximum of exactly 0 (a zero query: every key is 0) steps over the image of -0.0, which no score maps to and which
+// no zero score would pass, to the largest negative float.
 template <bool XB>
 __device__ __forceinline__ float boot_tau(uint32_t ks, float band) {
   if (XB && ks <= order_bits(-INFINITY)) return -INFINITY;
-  return unorder_bits(ks > 1u ? ks - 1u : ks) - band;
+  const uint32_t below = ks == 0x80000000u ? 0x7ffffffeu : ks - 1u;
+  return unorder_bits(ks > 1u ? below : ks) - band;
 }
 
 // Filter 32 accumulator columns (catalog rows rbase .. rbase+31) of this thread's query.
@@ -333,7 +358,10 @@ __device__ __forceinline__ void k2_grid_barrier(unsigned int* counter, unsigned 
 // MODE = 4: raw fp16 rows, one term, inverse norms applied in the epilogue: MODE 1 with fp16 operands. fp16 x fp16
 //           products are exact in fp32, so the scores are those of fp32 arithmetic on the fp16 values: no band, no
 //           re-scoring.
-// SCALED (MODE 1 and 4): exact scores, multiplied by the catalog's inverse norms in the epilogue.
+// MODE = 5: int8 rows (ICR_I8), one kind::i8 term (K = 32 codes = 32 bytes, the bytes of one f16 MMA step, so the tiles,
+//           swizzle and descriptor advance are those of a 16-bit matrix of D / 2 columns); the s32 accumulators become
+//           fp32 once (acc_to_f32) and are scaled by the catalog's factors: keys fp32(S) * f_row, exactly K1's.
+// SCALED (MODE 1, 4 and 5): exact scores, multiplied by the catalog's inverse norms (int8: factors) in the epilogue.
 // ASTAT (bf16, D <= 384): the work item's 128 query rows stay resident in shared memory for all of its catalog
 // tiles ("A-stationary"), so the ring streams catalog tiles only: 31 instead of 62 B/cycle/SM of L2 traffic,
 // which is the difference between L2-bound and tensor-bound for one-term MMAs (profiles/r01_notes.md).
@@ -344,7 +372,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   constexpr int TERMS = (MODE == 3) ? 3 : 1;
   static_assert(!ASTAT || TERMS == 1, "A-stationary is a one-term variant");
   static_assert(!XB || !DENSE, "dense scores are filtered by the select");
-  constexpr bool SCALED = (MODE == 1 || MODE == 4);  // exact scores scaled by the catalog's inverse norms in the epilogue
+  constexpr bool SCALED = (MODE == 1 || MODE == 4 || MODE == 5);  // exact scores scaled by the catalog's inverse norms in the epilogue
   constexpr int EW = epi_warps(TERMS), EH = EW / 4, ECOLS = BN / EH;  // epilogue warps, column groups, columns per warp
   constexpr int kStageTiles = ASTAT ? 1 : ((TERMS == 3) ? 4 : 2);  // B | A_hi A_lo B_hi B_lo | A B
   constexpr int kStageBytes = kStageTiles * kTileBytes;
@@ -448,8 +476,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     // registers before every tcgen05 instruction. With a single-lane branch that traffic made the issue loop,
     // not the tensor pipe, the limit of the one-term kernels (4 MMAs per stage): profiles/r01_notes.md.
     // instruction descriptor: D=f32, A/B = f16 or bf16, K-major both, N=256, M=256 (two CTAs x 128)
-    const uint32_t fmt = (MODE == 1) ? 1u : 0u;  // bf16 operands; f16 otherwise
-    const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (static_cast<uint32_t>(BN >> 3) << 17) | (static_cast<uint32_t>((2 * BM) >> 4) << 24);
+    const uint32_t idesc = idesc_formats<MODE>() | (static_cast<uint32_t>(BN >> 3) << 17) | (static_cast<uint32_t>((2 * BM) >> 4) << 24);
     // descriptors differ only in the 16-byte-unit start address (shared memory is < 256 KB: no carry out of the field)
     const uint64_t a_res0 = smem_desc_sw128(smem_u32(a_resident));
     const uint64_t st0 = smem_desc_sw128(smem_u32(stage_base));
@@ -482,7 +509,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
               for (int k4 = 0; k4 < BK / 16; ++k4) {
                 // advancing 16 elements (32 bytes) along K inside the swizzle atom = +2 in the 16-byte address field
                 const uint64_t o = static_cast<uint64_t>(k4 * 2);
-                umma_f16_pair(d_tmem, adesc + o, bdesc + o, idesc, (kb | k4) != 0 ? 1u : 0u);
+                umma_pair<MODE>(d_tmem, adesc + o, bdesc + o, idesc, (kb | k4) != 0 ? 1u : 0u);
               }
             } else if (TERMS == 3) {
               const uint64_t a_hi = sd, a_lo = sd + kTileUnits, b_hi = sd + 2 * kTileUnits, b_lo = sd + 3 * kTileUnits;
@@ -498,7 +525,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 #pragma unroll
               for (int k4 = 0; k4 < BK / 16; ++k4) {
                 const uint64_t o = static_cast<uint64_t>(k4 * 2);
-                umma_f16_pair(d_tmem, adesc + o, bdesc + o, idesc, (kb | k4) != 0 ? 1u : 0u);
+                umma_pair<MODE>(d_tmem, adesc + o, bdesc + o, idesc, (kb | k4) != 0 ? 1u : 0u);
               }
             }
             umma_commit_pair(smem_u32(&empty_bar[stage]));  // frees the stage in both CTAs when these MMAs have read it
@@ -589,6 +616,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
             uint32_t r[32];
             tmem_ld32(taddr + cb * 32, r);
             tmem_ld_wait(r);
+            acc_to_f32<MODE>(r);
             if (XB) exclude32(r, xs[cb * 32 + lane]);  // an excluded row must not be a block's maximum: the k-th maximum stays a lower bound
             float m = -INFINITY;
             if (plain) {
@@ -678,6 +706,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         for (int cb = 0; cb < ECOLS / 32; cb += 2) {
           // the next 32 columns are in flight while the current 32 are filtered
           tmem_ld_wait(ra);
+          acc_to_f32<MODE>(ra);
           tmem_ld32(taddr + (cb + 1) * 32, rb);
           if (dense) {
             if (live) dense_store32<SCALED>(ra, out_q + row0 + cb * 32, qscale, cinv_s + cb * 32, g.N - (row0 + cb * 32), vec_ok);
@@ -688,6 +717,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
                            g.N, g.mask);
           }
           tmem_ld_wait(rb);
+          acc_to_f32<MODE>(rb);
           if (cb + 2 < ECOLS / 32) tmem_ld32(taddr + (cb + 2) * 32, ra);
           if (dense) {
             if (live) dense_store32<SCALED>(rb, out_q + row0 + (cb + 1) * 32, qscale, cinv_s + (cb + 1) * 32, g.N - (row0 + (cb + 1) * 32), vec_ok);
@@ -979,7 +1009,7 @@ template <int MODE, bool XB = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kSwapThreads, 1)
 gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant__ CUtensorMap tma_c, const GemmArgs g,
                  const __grid_constant__ HistSelectArgs sel) {
-  constexpr bool SCALED = (MODE == 1 || MODE == 4);  // exact scores scaled by the catalog's inverse norms in the epilogue
+  constexpr bool SCALED = (MODE == 1 || MODE == 4 || MODE == 5);  // exact scores scaled by the catalog's inverse norms in the epilogue
   constexpr int kStageBytes = kTileBytes;
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   unsigned char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -1057,8 +1087,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
     }
   } else if (warp == 1 && rank == 0) {
     // ================= MMA issuer: whole warp walks the loop, one elected lane issues =================
-    const uint32_t fmt = (MODE == 1) ? 1u : 0u;  // bf16 operands; f16 otherwise
-    const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | (static_cast<uint32_t>(g.qpad >> 3) << 17) | (static_cast<uint32_t>(BN >> 4) << 24);
+    const uint32_t idesc = idesc_formats<MODE>() | (static_cast<uint32_t>(g.qpad >> 3) << 17) | (static_cast<uint32_t>(BN >> 4) << 24);
     const uint64_t qd0 = smem_desc_sw128(smem_u32(q_res));
     const uint64_t cd0 = smem_desc_sw128(smem_u32(stage_base));
     constexpr uint64_t kStageUnits = kStageBytes >> 4;
@@ -1084,7 +1113,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
 #pragma unroll
             for (int k4 = 0; k4 < BK / 16; ++k4) {
               const uint64_t o = static_cast<uint64_t>(k4 * 2);
-              umma_f16_pair(d_tmem, cdesc + o, qdesc + o, idesc, (kb | k4) != 0 ? 1u : 0u);
+              umma_pair<MODE>(d_tmem, cdesc + o, qdesc + o, idesc, (kb | k4) != 0 ? 1u : 0u);
             }
             umma_commit_pair(smem_u32(&empty_bar[stage]));
             if (kb == KB - 1) umma_commit_pair(smem_u32(&tfull_bar[acc]));
@@ -1140,6 +1169,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
               uint32_t r[32];
               tmem_ld32(taddr + b * 32, r);
               tmem_ld_wait(r);
+              acc_to_f32<MODE>(r);
               float sc[32];
               const uint32_t xm = XB ? swap_excluded32(xs, b * 32, lane) : 0u;  // excluded (row, query) pairs do not bound anything
 #pragma unroll
@@ -1203,6 +1233,7 @@ gemm_swap_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constan
           uint32_t r[32];
           tmem_ld32(taddr + jb, r);
           tmem_ld_wait(r);
+          acc_to_f32<MODE>(r);
           float sc[32];
           unsigned m = 0;
 #pragma unroll
@@ -1301,6 +1332,8 @@ int launch_row_inv_norms(const void* x, int64_t rows, int64_t dim, int64_t ld, i
 int launch_split_planes(const float* x, int64_t rows, int64_t dim, int64_t ld, uint16_t* planes, cudaStream_t st);
 int launch_screen_plane(const float* x, int64_t rows, int64_t dim, int64_t ld, uint16_t* plane, float* inv, cudaStream_t st, float* tau_init = nullptr,
                         unsigned int* ovf_init = nullptr);
+int launch_quantize_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, int8_t* codes, int64_t ldc, float* factors, cudaStream_t st,
+                         float* tau_init = nullptr, unsigned int* ovf_init = nullptr);
 
 constexpr size_t kGemmSmemBytes = static_cast<size_t>(kRingBytes) + 4 * BN * sizeof(float) +  // EW * ECOLS = 4 * BN inverse norms
                                  
@@ -1313,8 +1346,11 @@ constexpr size_t kSwapSmemBytes = static_cast<size_t>(kRingBytes) + 2 * 256 * 4 
 static_assert(kSwapSmemBytes <= 232448, "exceeds the 227 KB of shared memory a CTA may use");
 
 // top-k path: MODE 2 (one-term screening + exact re-scoring of the survivors) on fp32 catalogs, MODE 1 on bf16 ones,
-// MODE 4 on fp16 ones
-static int mode_for(int dtype) { return dtype == ICR_F32 ? 2 : (dtype == ICR_BF16 ? 1 : 4); }
+// MODE 4 on fp16 ones, MODE 5 on int8 ones
+static int mode_for(int dtype) { return dtype == ICR_F32 ? 2 : (dtype == ICR_BF16 ? 1 : (dtype == ICR_I8 ? 5 : 4)); }
+// The tile geometry sees an int8 row of D codes as a 16-bit row of D / 2 elements (the same bytes): swap_applies, the
+// bootstrap plans, the K-block count ceil(D / 128) and the A-stationary limit (D <= 768) all follow from the true bytes.
+static int64_t geometry_dim(int64_t D, int dtype) { return dtype == ICR_I8 ? D / 2 : D; }
 // keys carried per query between phases: k exact keys, or k + room for the screening band (select_args.cuh)
 static int carry_cap(int k, int mode) {
   if (mode != 2) return k;
@@ -1399,15 +1435,18 @@ constexpr int kMaxPhases = 16;
 static int dense0_tiles(int64_t Q, int64_t N) { return (Q <= 2 * BM && (N + BN - 1) / BN >= 2048) ? 16 : 4; }
 
 // kernel variants: 1 = bf16 streaming both operands, 2 = bf16 with resident queries, 5 / 6 = fp16 screen plane streaming /
-// resident queries, 8 / 9 = fp16 rows streaming / resident queries, 4 / 7 / 3 = swapped kernel (small batches) on bf16 /
-// the screen plane / fp16 rows; DENSE only: 0 = fp16 hi|lo planes, three MMA terms (K2' on fp32 inputs)
+// resident queries, 8 / 9 = fp16 rows streaming / resident queries, 10 / 11 = int8 rows streaming / resident queries,
+// 4 / 7 / 3 / 12 = swapped kernel (small batches) on bf16 / the screen plane / fp16 rows / int8 rows; DENSE only: 0 = fp16
+// hi|lo planes, three MMA terms (K2' on fp32 inputs)
 #define ICR_GEMM_VARIANTS(X, DENSE, XB)            \
   X(1, (gemm_topk_kernel<1, false, DENSE, XB>))    \
   X(2, (gemm_topk_kernel<1, true, DENSE, XB>))     \
   X(5, (gemm_topk_kernel<2, false, DENSE, XB>))    \
   X(6, (gemm_topk_kernel<2, true, DENSE, XB>))     \
   X(8, (gemm_topk_kernel<4, false, DENSE, XB>))    \
-  X(9, (gemm_topk_kernel<4, true, DENSE, XB>))
+  X(9, (gemm_topk_kernel<4, true, DENSE, XB>))     \
+  X(10, (gemm_topk_kernel<5, false, DENSE, XB>))   \
+  X(11, (gemm_topk_kernel<5, true, DENSE, XB>))
 
 // Launch helper of the GEMM kernels. The single-launch modes (g.boot > 0) synchronise the whole grid through a counter in
 // global memory, which needs every CTA resident at once: those launches carry the cooperative attribute, so the driver
@@ -1442,7 +1481,7 @@ static void launch_gemm_grid(void (*kernel)(KArgs...), int grid, int threads, si
 // exclusions)
 template <bool DENSE, bool XB = false>
 static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, const CUtensorMap& map_b, const GemmArgs& g, cudaStream_t st) {
-  static thread_local SmemAttrCache cache[10];
+  static thread_local SmemAttrCache cache[12];
   int rc = ICR_OK;
 #define ICR_SET(ID, K) \
   if (which == ID) rc = ensure_dyn_smem(cache[ID], K, kGemmSmemBytes);
@@ -1466,16 +1505,18 @@ static int launch_gemm_variant(int which, int grid, const CUtensorMap& map_a, co
 template <bool XB = false>
 static int launch_swap_variant(int which, int grid, const CUtensorMap& map_q, const CUtensorMap& map_c, const GemmArgs& g, cudaStream_t st,
                                const HistSelectArgs& sel = HistSelectArgs{}) {
-  static thread_local SmemAttrCache cache[3];
+  static thread_local SmemAttrCache cache[4];
   int rc = ICR_OK;
   if (which == 4) rc = ensure_dyn_smem(cache[0], gemm_swap_kernel<1, XB>, kSwapSmemBytes);
   if (which == 7) rc = ensure_dyn_smem(cache[1], gemm_swap_kernel<2, XB>, kSwapSmemBytes);
   if (which == 3) rc = ensure_dyn_smem(cache[2], gemm_swap_kernel<4, XB>, kSwapSmemBytes);
+  if (which == 12) rc = ensure_dyn_smem(cache[3], gemm_swap_kernel<5, XB>, kSwapSmemBytes);
   if (rc) return rc;
   profile_begin(kKernelGemm, 1, st);
   if (which == 4) launch_gemm_grid(gemm_swap_kernel<1, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
   if (which == 7) launch_gemm_grid(gemm_swap_kernel<2, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
   if (which == 3) launch_gemm_grid(gemm_swap_kernel<4, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
+  if (which == 12) launch_gemm_grid(gemm_swap_kernel<5, XB>, grid, kSwapThreads, kSwapSmemBytes, st, g.boot > 0, map_q, map_c, g, sel);
   profile_end(st);
   ICR_LAUNCH_CHECK();
   return ICR_OK;
@@ -1568,6 +1609,7 @@ static int boot_pairs_for(int64_t Q, int64_t N, int64_t D, int k, int* boot_tile
 static GemmWs gemm_ws_layout(int64_t Q, int64_t N, int64_t D, int dtype, int k, int have_planes, int have_cinv) {
   GemmWs w{};
   const int mode = mode_for(dtype);
+  D = geometry_dim(D, dtype);
   const int qblocks = static_cast<int>((Q + 2 * BM - 1) / (2 * BM));
   Phase ph[kMaxPhases];
   const bool swap = swap_applies(Q, N, D);
@@ -1590,7 +1632,7 @@ static GemmWs gemm_ws_layout(int64_t Q, int64_t N, int64_t D, int dtype, int k, 
     off += align_up(bytes, 1024);
     return o;
   };
-  w.q_planes = take(mode == 2 ? static_cast<size_t>(Q) * dp * 2 : 0);
+  w.q_planes = take(mode == 2 ? static_cast<size_t>(Q) * dp * 2 : (mode == 5 ? static_cast<size_t>(Q) * D * 2 : 0));  // int8: query codes
   w.c_planes = take((mode == 2 && !have_planes) ? static_cast<size_t>(N) * dp * 2 : 0);
   w.qinv = take(static_cast<size_t>(Q) * 4);
   w.cinv = take(!have_cinv ? static_cast<size_t>(N) * 4 : 0);
@@ -1714,6 +1756,22 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
     sa.rs_qinv = qinv;
     sa.rs_cinv = cinv;
     sa.mask = mask;  // the exact ranking of an overflowed query walks the catalog itself
+  } else if (mode == 5) {
+    // int8 rows: the fp32 queries are quantised into the workspace (I8Rows, as K1 and icr_quantize_rows do), their factors
+    // are the query scale of the select; the catalog's factors are required (icr_cos_topk checked them)
+    int8_t* qc = reinterpret_cast<int8_t*>(base + L.q_planes);
+    float* qinv = reinterpret_cast<float*>(base + L.qinv);
+    if ((rc = launch_quantize_rows(static_cast<const float*>(queries), Q, D, ldq, qc, D, qinv, st, const_cast<float*>(g.tau), g.overflow))) return rc;
+    const int64_t d2 = D / 2;  // D % 16 == 0: the codes as a 16-bit matrix of D / 2 columns
+    if ((rc = make_map(&map_a, qc, Q, d2, d2, false))) return rc;
+    if ((rc = make_map(&map_b, catalog, N, d2, ldc / 2, false))) return rc;
+    g.kb_per_term = static_cast<int>((d2 + BK - 1) / BK);
+    g.plane_stride = 0;
+    g.acc_scale = 1.0f;
+    g.qinv = qinv;
+    g.cinv = cat_inv_norms;
+    q_operand = qc;
+    q_cols = q_ld = d2;
   } else {
     float* qinv = reinterpret_cast<float*>(base + L.qinv);
     if ((rc = launch_row_inv_norms(queries, Q, D, ldq, dtype, qinv, st, const_cast<float*>(g.tau), g.overflow))) return rc;
@@ -1733,12 +1791,13 @@ int launch_gemm_topk(const void* queries, int64_t Q, int64_t ldq, const void* ca
   }
   sa.out_scale = g.acc_scale;
   sa.out_qscale = g.qinv;
-  const bool swap = swap_applies(Q, N, D);
+  const bool swap = swap_applies(Q, N, geometry_dim(D, dtype));
   const bool astat = g.kb_per_term <= kAStatMaxKB;
   int which;
-  if (swap) which = mode == 1 ? 4 : (mode == 4 ? 3 : 7);
+  if (swap) which = mode == 1 ? 4 : (mode == 4 ? 3 : (mode == 5 ? 12 : 7));
   else if (mode == 2) which = astat ? 6 : 5;
   else if (mode == 1) which = astat ? 2 : 1;
+  else if (mode == 5) which = astat ? 11 : 10;
   else which = astat ? 9 : 8;
   if (swap) {
     g.qpad = static_cast<int>((Q + 31) / 32 * 32);

@@ -20,6 +20,7 @@
 // Replaces, for one request: torch.tensor(catalog) + F.normalize x2 + torch.mm + argsort
 // (reference src/inference/serve_recommendations.py:213-215 via sentence_transformers.util.cos_sim).
 #include <cstdlib>
+#include <type_traits>
 
 #include "common.cuh"
 #include "peer.cuh"
@@ -64,7 +65,7 @@ struct GemvArgs {
   int64_t N;
   int64_t ldc;
   int D;
-  const void* q;  // [Q][D] same dtype as the catalog
+  const void* q;  // [Q][D] same dtype as the catalog (int8 catalogs: fp32 queries, quantised by every CTA)
   int64_t ldq;
   int Q;
   const uint8_t* mask;  // optional exclusion mask
@@ -131,6 +132,11 @@ struct GemvSmem {
     return static_cast<size_t>(QT) * (CAND * 8 + kMergeSel * 8 + kHsBins * 4 + 8) + static_cast<size_t>(QT) * D * 4 + 512 * 4 + 16;
   }
 };
+
+// floats of the query area per query (GemvSmem::qs): the fp32 row for the float kernels; the int8 kernels stage D / 4 packed
+// words and keep the query factors in the last 8 floats of the area (i8_query_factors), so each query gets 8 floats more
+template <typename T>
+__host__ __device__ constexpr int query_area(int D) { return std::is_same_v<T, int8_t> ? D / 4 + 8 : D; }
 
 // ---- stage the L2-normalised queries in shared memory (fp32) ----------------------------------------
 // One warp per query; the row is fetched with 16-byte loads issued back to back (one memory round trip: this
@@ -230,6 +236,87 @@ __device__ __forceinline__ void reduce_and_append(float (&acc)[RB * (QT + (NORMS
   }
 }
 
+// ---- int8 rows (ICR_I8) ----------------------------------------------------------------------------------
+// Each CTA quantises its queries from the fp32 rows (I8Rows) in the prologue, so a request stays one launch. The codes are
+// staged as packed words [QT][D / 4] at the start of the query area (query_area<int8_t>: QT * (D / 4 + 8) floats); the query
+// factors sit in its last 8 floats, behind the codes, where the merging CTA reads them back to scale the k final keys.
+template <int QT>
+__device__ __forceinline__ float* i8_query_factors(GemvSmem<QT>& sm) { return reinterpret_cast<float*>(sm.ncand) - 8; }
+
+template <int QT>
+__device__ __forceinline__ void stage_queries_i8(const GemvArgs& a, GemvSmem<QT>& sm, int D, int nq, int warp, int lane) {
+  const int nwords = D / 4;
+  const float* qg = static_cast<const float*>(a.q);
+  for (int t = warp; t < QT; t += kGemvWarps) {
+    uint32_t* dst = reinterpret_cast<uint32_t*>(sm.qs) + t * nwords;
+    float f = 0.f;
+    if (t < nq) {
+      f = I8Rows::quantize(qg + static_cast<int64_t>(a.q0 + t) * a.ldq, D, nwords, lane, [dst](int w, uint32_t word) { dst[w] = word; });
+    } else {
+      for (int w = lane; w < nwords; w += 32) dst[w] = 0u;
+    }
+    if (lane == 0) i8_query_factors(sm)[t] = f;
+  }
+}
+
+// int8 counterpart of fma_vector: exact int32 dot products, four codes per __dp4a. The accumulators are laid out as
+// [VT][RB] like the float kernels'; slots t >= QT (the norm slot the int8 kernels keep for QT > 1, so that V stays a power
+// of two) stay zero.
+template <int RB, int QT, int VT>
+__device__ __forceinline__ void dp4a_vector(const uint4 (&c)[RB], const float* qs, int dpad, int v, int (&acc)[RB * VT]) {
+  const uint32_t* qw = reinterpret_cast<const uint32_t*>(qs);
+  uint4 qv[QT];
+#pragma unroll
+  for (int t = 0; t < QT; ++t) qv[t] = *reinterpret_cast<const uint4*>(qw + t * (dpad / 4) + v * 4);
+#pragma unroll
+  for (int r = 0; r < RB; ++r) {
+#pragma unroll
+    for (int t = 0; t < QT; ++t) {
+      int s = acc[t * RB + r];
+      s = __dp4a(static_cast<int>(c[r].x), static_cast<int>(qv[t].x), s);
+      s = __dp4a(static_cast<int>(c[r].y), static_cast<int>(qv[t].y), s);
+      s = __dp4a(static_cast<int>(c[r].z), static_cast<int>(qv[t].z), s);
+      acc[t * RB + r] = __dp4a(static_cast<int>(c[r].w), static_cast<int>(qv[t].w), s);
+    }
+  }
+}
+
+// one 16-byte vector of RB rows, whichever the element type (float kernels: fma_vector; int8: dp4a_vector)
+template <typename T, int RB, int QT, bool NORMS, int VT, typename A>
+__device__ __forceinline__ void accumulate_vector(const uint4 (&c)[RB], const float* qs, int dpad, int v, A (&acc)[RB * VT]) {
+  if constexpr (std::is_same_v<T, int8_t>) dp4a_vector<RB, QT, VT>(c, qs, dpad, v, acc);
+  else fma_vector<T, RB, QT, NORMS>(c, qs, dpad, v, acc);
+}
+
+// int8 counterpart of reduce_and_append: integer reduction, then key = fp32(S) * f_row (I8Rows::key). Lane r (< RB) brings
+// the factor of row r0 + r in `f_lane`.
+template <int RB, int QT, int VT, bool XB>
+__device__ __forceinline__ void reduce_and_append_i8(int (&acc)[RB * VT], const GemvArgs& a, GemvSmem<QT>& sm, int nq, int64_t r0,
+                                                     int64_t row_limit, int lane, float f_lane) {
+  constexpr int V = RB * VT;
+  constexpr int SH = (V == 32) ? 0 : (V == 16 ? 1 : (V == 8 ? 2 : 3));
+  warp_transpose_reduce<V>(acc, lane);
+  const int idx = lane >> SH;
+  const int t = idx / RB, r = idx % RB;
+  const float f = __shfl_sync(kFull, f_lane, r);
+  const int64_t row = r0 + r;
+  if (t < nq && (lane & ((1 << SH) - 1)) == 0 && row < row_limit) {
+    const bool excluded = a.mask && a.mask[row];
+    const float key = I8Rows::key(acc[0], f);
+    if (!excluded && key > sm.tau[t] && !(XB && Exclusions{nullptr, a.xbits, a.xld}.bit(a.q0 + t, row))) {
+      const int pos = atomicAdd(&sm.ncand[t], 1);
+      if (pos < GemvSmem<QT>::CAND) sm.cand[t * GemvSmem<QT>::CAND + pos] = make_key(key, static_cast<uint32_t>(row));
+    }
+  }
+}
+
+// the score the merge writes for a key of query t: the key itself, or for int8 rows key * f_query
+template <bool I8, int QT>
+__device__ __forceinline__ float out_score(uint64_t key, GemvSmem<QT>& sm, int t) {
+  if constexpr (I8) return __fmul_rn(key_score(key), i8_query_factors(sm)[t]);
+  else return key_score(key);
+}
+
 // If a list could overflow during the next block of rows (or at the end), keep its k best and raise tau.
 // One warp per query (QT <= 7 < 8 warps), histogram selection instead of a sort: no CTA-wide barrier inside, and
 // every query of the pass is handled at the same time. The final lists are sorted (k keys only) for the merge.
@@ -306,7 +393,7 @@ __device__ __forceinline__ void refresh_single(const GemvArgs& a, GemvSmem<1>& s
 }
 
 // Merge of the G per-CTA lists of query t by a group of GT threads (gtid = index in the group); LISTS * GT >= G.
-template <int QT, int GT, int LISTS, typename Sync>
+template <int QT, int GT, int LISTS, bool I8, typename Sync>
 __device__ __forceinline__ void merge_query(const GemvArgs& a, GemvSmem<QT>& sm, int t, int gtid, Sync sync) {
   constexpr int kGemvCand = GemvSmem<QT>::CAND;
   const int k = a.k, G = gridDim.x, lane = gtid & 31;
@@ -385,7 +472,7 @@ __device__ __forceinline__ void merge_query(const GemvArgs& a, GemvSmem<QT>& sm,
 #pragma unroll 8
       for (int j = 0; j < n; ++j) rank += (buf[j] > key) ? 1 : 0;
       if (rank < k) {
-        a.out_scores[qo + rank] = key_score(key);
+        a.out_scores[qo + rank] = out_score<I8>(key, sm, t);
         a.out_ids[qo + rank] = static_cast<int64_t>(key_row(key)) + a.id_offset;
       }
     }
@@ -424,7 +511,7 @@ __device__ __forceinline__ void merge_query(const GemvArgs& a, GemvSmem<QT>& sm,
     warp_bitonic_sort_desc(sel, P, lane);
     for (int i = lane; i < k; i += 32) {
       const bool ok = i < kept;
-      a.out_scores[qo + i] = ok ? key_score(sel[i]) : -INFINITY;
+      a.out_scores[qo + i] = ok ? out_score<I8>(sel[i], sm, t) : -INFINITY;
       a.out_ids[qo + i] = ok ? static_cast<int64_t>(key_row(sel[i])) + a.id_offset : -1;
     }
     __syncwarp();
@@ -446,7 +533,7 @@ __device__ __forceinline__ bool flat_tail(const GemvArgs& a, int nq) {
 }
 
 // returns false when more keys than the buffer holds reach the floor (the caller then takes the general merge)
-template <int QT, typename Sync>
+template <int QT, bool I8, typename Sync>
 __device__ __forceinline__ bool merge_query_flat(const GemvArgs& a, GemvSmem<QT>& sm, int tid, Sync sync) {
   const int k = a.k, G = gridDim.x, tot = G * k, lane = tid & 31, warp = tid >> 5;
   uint64_t* surv = sm.cand;  // [kFlatSurv]
@@ -493,7 +580,7 @@ __device__ __forceinline__ bool merge_query_flat(const GemvArgs& a, GemvSmem<QT>
     const uint64_t mine = surv[tid];
     const int rank = cta_key_rank(surv, n, mine);
     if (rank < k) {
-      a.out_scores[qo + rank] = key_score(mine);
+      a.out_scores[qo + rank] = out_score<I8>(mine, sm, 0);
       a.out_ids[qo + rank] = static_cast<int64_t>(key_row(mine)) + a.id_offset;
     }
   }
@@ -578,7 +665,7 @@ __device__ __forceinline__ void peer_tail_merge(const GemvArgs& a, GemvSmem<QT>&
 // `pending`: the caller has not run the final threshold refresh (ring kernel): it happens here, and on a flat tail the whole
 // CTA ranks the (<= 256) candidates by counting and stores the k best straight into the global list - one warp ordering
 // ~50 keys alone took 1.4-1.9 us per CTA, on the critical path of the slowest one.
-template <int QT, bool NAMED>
+template <int QT, bool NAMED, bool I8 = false>
 __device__ __forceinline__ void emit_and_merge(const GemvArgs& a, GemvSmem<QT>& sm, int nq, bool has_rows, int tid, bool pending = false) {
   const int lane = tid & 31, warp = tid >> 5;
   const int k = a.k, G = gridDim.x;
@@ -633,13 +720,13 @@ __device__ __forceinline__ void emit_and_merge(const GemvArgs& a, GemvSmem<QT>& 
   // which also yields the sorted output positions directly. One query: the whole CTA works on it. Several
   // queries: one warp each, side by side.
   if (nq == 1) {
-    if (!flat || !merge_query_flat<QT>(a, sm, tid, [] { compute_sync<NAMED>(); }))
-      merge_query<QT, kGemvThreads, 2>(a, sm, 0, tid, [] { compute_sync<NAMED>(); });
+    if (!flat || !merge_query_flat<QT, I8>(a, sm, tid, [] { compute_sync<NAMED>(); }))
+      merge_query<QT, kGemvThreads, 2, I8>(a, sm, 0, tid, [] { compute_sync<NAMED>(); });
   } else if (nq <= 4) {  // two warps per query, each pair on its own named barrier
     const int t = warp >> 1;
-    if (t < nq) merge_query<QT, 64, 5>(a, sm, t, tid & 63, [t] { ptx::named_sync(2 + t, 64); });
+    if (t < nq) merge_query<QT, 64, 5, I8>(a, sm, t, tid & 63, [t] { ptx::named_sync(2 + t, 64); });
   } else if (warp < nq) {
-    merge_query<QT, 32, 10>(a, sm, warp, lane, [] { __syncwarp(); });
+    merge_query<QT, 32, 10, I8>(a, sm, warp, lane, [] { __syncwarp(); });
   }
   compute_sync<NAMED>();
   ICR_MSTAMP(4);
@@ -655,17 +742,20 @@ __device__ __forceinline__ void emit_and_merge(const GemvArgs& a, GemvSmem<QT>& 
 // =====================================================================================================
 template <typename T, int RB, int QT, bool XB = false>
 __global__ void __launch_bounds__(kGemvThreads) gemv_topk_kernel(GemvArgs a) {
+  constexpr bool I8 = std::is_same_v<T, int8_t>;  // int8 rows: fp32 queries quantised here, factors in a.cat_inv
+  using Acc = std::conditional_t<I8, int, float>;
   constexpr int VEC = Elem<T>::VEC;
   constexpr int V = RB * (QT + 1);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int nvec = a.D / VEC;
   const int dpad = nvec * VEC;
-  GemvSmem<QT> sm(smem_raw, dpad);
+  GemvSmem<QT> sm(smem_raw, query_area<T>(dpad));
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const T* cat = static_cast<const T*>(a.cat);
   const int nq = min(QT, a.Q - a.q0);
 
-  stage_queries<T, QT>(a, sm.qs, dpad, nq, warp, lane);
+  if constexpr (I8) stage_queries_i8<QT>(a, sm, dpad, nq, warp, lane);
+  else stage_queries<T, QT>(a, sm.qs, dpad, nq, warp, lane);
   if (tid < QT) {
     sm.ncand[tid] = 0;
     sm.tau[tid] = -INFINITY;
@@ -679,9 +769,9 @@ __global__ void __launch_bounds__(kGemvThreads) gemv_topk_kernel(GemvArgs a) {
   for (int64_t blk = row_begin; blk < row_end; blk += kBlockRows) {
     const int64_t blk_end = min(row_end, blk + kBlockRows);
     for (int64_t r0 = blk + warp * RB; r0 < blk_end; r0 += kGemvWarps * RB) {
-      float acc[V];
+      Acc acc[V];
 #pragma unroll
-      for (int i = 0; i < V; ++i) acc[i] = 0.f;
+      for (int i = 0; i < V; ++i) acc[i] = 0;
       for (int vb = 0; vb < nvec; vb += 32 * kGemvUnroll) {
         uint4 c[kGemvUnroll][RB];
 #pragma unroll
@@ -696,15 +786,20 @@ __global__ void __launch_bounds__(kGemvThreads) gemv_topk_kernel(GemvArgs a) {
 #pragma unroll
         for (int u = 0; u < kGemvUnroll; ++u) {
           const int v = vb + u * 32 + lane;
-          if (v < nvec) fma_vector<T, RB, QT>(c[u], sm.qs, dpad, v, acc);
+          if (v < nvec) accumulate_vector<T, RB, QT, false, QT + 1>(c[u], sm.qs, dpad, v, acc);
         }
       }
-      reduce_and_append<RB, QT, false, XB>(acc, a, sm, nq, r0, blk_end, lane);
+      if constexpr (I8) {
+        const float f_lane = (lane < RB && r0 + lane < blk_end) ? __ldg(a.cat_inv + r0 + lane) : 0.f;
+        reduce_and_append_i8<RB, QT, QT + 1, XB>(acc, a, sm, nq, r0, blk_end, lane, f_lane);
+      } else {
+        reduce_and_append<RB, QT, false, XB>(acc, a, sm, nq, r0, blk_end, lane);
+      }
     }
     __syncthreads();
     refresh_thresholds<QT, false>(a, sm, nq, blk + kBlockRows >= row_end, kBlockRows, tid);
   }
-  emit_and_merge<QT, false>(a, sm, nq, row_begin < row_end, tid);
+  emit_and_merge<QT, false, I8>(a, sm, nq, row_begin < row_end, tid);
 }
 
 // =====================================================================================================
@@ -712,11 +807,17 @@ __global__ void __launch_bounds__(kGemvThreads) gemv_topk_kernel(GemvArgs a) {
 // =====================================================================================================
 template <typename T, int QT, bool NORMS = false, bool XB = false>
 __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) {
-  static_assert(!NORMS || QT == 1, "precomputed norms: single-query kernel only (V must stay a power of two)");
+  // int8 rows: fp32 queries quantised here; the row factors always come precomputed (NORMS), and for QT > 1 the unused norm
+  // slot of the accumulators is kept so that V stays a power of two
+  constexpr bool I8 = std::is_same_v<T, int8_t>;
+  using Acc = std::conditional_t<I8, int, float>;
+  static_assert(!NORMS || QT == 1 || I8, "precomputed norms: single-query kernel only (V must stay a power of two)");
+  static_assert(!I8 || NORMS, "int8 rows come with their factors");
   constexpr int VEC = Elem<T>::VEC;
   constexpr int RB = (QT == 7) ? 4 : 8;  // rows reduced together (V = RB * (QT + 1) <= 32) = rows per ring slot
   constexpr int kSlabRows = RB;
-  constexpr int V = RB * (QT + (NORMS ? 0 : 1));
+  constexpr int VT = (NORMS && QT == 1) ? 1 : QT + 1;  // accumulator slots per row: the queries (+ the norm)
+  constexpr int V = RB * VT;
   extern __shared__ __align__(128) unsigned char ring_smem_raw[];
   const int nvec = a.D / VEC;
   const int dpad = nvec * VEC;
@@ -730,7 +831,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) 
   // precomputed inverse norms of the slab's rows, copied next to it (NORMS): a global load per slab from the consumer waited
   // behind the whole ring's worth of queued catalog reads - 3.7 us of an 18 us stream on a cold 76 MB catalog
   float* slot_inv = reinterpret_cast<float*>(slot_row + kMaxSlots);  // [kMaxSlots][8]
-  GemvSmem<QT> sm(reinterpret_cast<unsigned char*>(slot_inv + kMaxSlots * 8), dpad);
+  GemvSmem<QT> sm(reinterpret_cast<unsigned char*>(slot_inv + kMaxSlots * 8), query_area<T>(dpad));
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int nq = min(QT, a.Q - a.q0);
   constexpr int kProducers = 4;
@@ -811,7 +912,8 @@ __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) 
   }
 
   // ================= consumers =================
-  stage_queries<T, QT>(a, sm.qs, dpad, nq, warp, lane);
+  if constexpr (I8) stage_queries_i8<QT>(a, sm, dpad, nq, warp, lane);
+  else stage_queries<T, QT>(a, sm.qs, dpad, nq, warp, lane);
   if (tid < QT) {
     sm.ncand[tid] = 0;
     sm.tau[tid] = -INFINITY;
@@ -834,9 +936,9 @@ __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) 
 #endif
       const unsigned char* slab = ring + static_cast<size_t>(slot) * slot_bytes;
       constexpr int g = 0;
-      float acc[V];
+      Acc acc[V];
 #pragma unroll
-      for (int i = 0; i < V; ++i) acc[i] = 0.f;
+      for (int i = 0; i < V; ++i) acc[i] = 0;
       float inv_lane = 0.f;
       if (NORMS && lane < RB && r0 + lane < a.N) inv_lane = (r0 + RB <= a.N) ? slot_inv[slot * 8 + lane] : __ldg(a.cat_inv + r0 + lane);
       const int nfull = nvec & ~31;  // vectors covered by iterations in which every lane has one
@@ -847,29 +949,28 @@ __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) 
           // rows past the end of the catalog were not copied: stale ring bytes, masked by row_limit below
           c[r] = *reinterpret_cast<const uint4*>(slab + static_cast<size_t>(g * RB + r) * row_bytes + static_cast<size_t>(v) * 16);
         }
-        fma_vector<T, RB, QT, NORMS>(c, sm.qs, dpad, v, acc);
+        accumulate_vector<T, RB, QT, NORMS, VT>(c, sm.qs, dpad, v, acc);
       }
       if (nvec - nfull == 16) {
         // Half-filled last iteration (768-byte and 256-byte bf16 rows, ...): instead of idling 16 lanes, the two
         // half-warps split the ROWS of the tail — lanes 0-15 take rows 0,2,4,.., lanes 16-31 rows 1,3,5,.. — and
         // the partial sums are folded into the full-width accumulators with predicated adds (static indices).
         constexpr int HB = RB / 2;
-        constexpr int VT = QT + (NORMS ? 0 : 1);
         const int h = lane >> 4, v = nfull + (lane & 15);
         uint4 c[HB];
 #pragma unroll
         for (int i = 0; i < HB; ++i)
           c[i] = *reinterpret_cast<const uint4*>(slab + static_cast<size_t>(g * RB + 2 * i + h) * row_bytes + static_cast<size_t>(v) * 16);
-        float tacc[HB * VT];
+        Acc tacc[HB * VT];
 #pragma unroll
-        for (int i = 0; i < HB * VT; ++i) tacc[i] = 0.f;
-        fma_vector<T, HB, QT, NORMS>(c, sm.qs, dpad, v, tacc);
+        for (int i = 0; i < HB * VT; ++i) tacc[i] = 0;
+        accumulate_vector<T, HB, QT, NORMS, VT>(c, sm.qs, dpad, v, tacc);
 #pragma unroll
         for (int t = 0; t < VT; ++t)
 #pragma unroll
           for (int i = 0; i < HB; ++i) {
-            acc[t * RB + 2 * i] += h == 0 ? tacc[t * HB + i] : 0.f;
-            acc[t * RB + 2 * i + 1] += h == 1 ? tacc[t * HB + i] : 0.f;
+            acc[t * RB + 2 * i] += h == 0 ? tacc[t * HB + i] : Acc(0);
+            acc[t * RB + 2 * i + 1] += h == 1 ? tacc[t * HB + i] : Acc(0);
           }
       } else if (lane < nvec - nfull) {
         const int v = nfull + lane;
@@ -877,9 +978,10 @@ __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) 
 #pragma unroll
         for (int r = 0; r < RB; ++r)
           c[r] = *reinterpret_cast<const uint4*>(slab + static_cast<size_t>(g * RB + r) * row_bytes + static_cast<size_t>(v) * 16);
-        fma_vector<T, RB, QT, NORMS>(c, sm.qs, dpad, v, acc);
+        accumulate_vector<T, RB, QT, NORMS, VT>(c, sm.qs, dpad, v, acc);
       }
-      reduce_and_append<RB, QT, NORMS, XB>(acc, a, sm, nq, r0 + g * RB, a.N, lane, inv_lane);
+      if constexpr (I8) reduce_and_append_i8<RB, QT, VT, XB>(acc, a, sm, nq, r0 + g * RB, a.N, lane, inv_lane);
+      else reduce_and_append<RB, QT, NORMS, XB>(acc, a, sm, nq, r0 + g * RB, a.N, lane, inv_lane);
     }
     __syncwarp();
     if (lane == 0) ptx::mbar_arrive(ptx::smem_u32(&empty_bar[slot]));
@@ -899,7 +1001,7 @@ __global__ void __launch_bounds__(kRingThreads, 1) gemv_ring_kernel(GemvArgs a) 
   }
   compute_sync<true>();
   ICR_STAMP(4);
-  emit_and_merge<QT, true>(a, sm, nq, true, tid, true);
+  emit_and_merge<QT, true, I8>(a, sm, nq, true, tid, true);
   ICR_STAMP(7);
 }
 
@@ -908,7 +1010,7 @@ constexpr size_t kSmemBudget = 227 * 1024 - 1024;
 
 template <typename T, int RB, int QT, bool XB>
 static int launch_direct(const GemvArgs& a, int grid, cudaStream_t st) {
-  const size_t smem = GemvSmem<QT>::bytes(a.D);
+  const size_t smem = GemvSmem<QT>::bytes(query_area<T>(a.D));
   static thread_local SmemSizeCache configured;  // per device (ADVICE r1): a thread may serve several GPUs
   if (smem > 48 * 1024) {
     const int rc = ensure_dyn_smem_size(configured, gemv_topk_kernel<T, RB, QT, XB>, smem);
@@ -923,7 +1025,7 @@ static int launch_direct(const GemvArgs& a, int grid, cudaStream_t st) {
 
 template <typename T, int QT>
 static int ring_slots_for(int D) {
-  const size_t fixed = GemvSmem<QT>::bytes(D) + 3 * kMaxSlots * sizeof(uint64_t) + kMaxSlots * 8 * sizeof(float) + 128;
+  const size_t fixed = GemvSmem<QT>::bytes(query_area<T>(D)) + 3 * kMaxSlots * sizeof(uint64_t) + kMaxSlots * 8 * sizeof(float) + 128;
   const size_t slot = static_cast<size_t>(QT == 7 ? 4 : 8) * D * sizeof(T);
   if (fixed + kGemvWarps * slot > kSmemBudget) return 0;
   const size_t n = (kSmemBudget - fixed) / slot;
@@ -952,7 +1054,7 @@ static int launch_ring(GemvArgs a, int grid, cudaStream_t st) {
     if (a.dbg & 2) a.static_slabs = static_cast<int>((total_slabs + grid - 1) / grid + 3) / 4 * 4;
 #endif
   }
-  const size_t smem = static_cast<size_t>(a.ring_slots) * (QT == 7 ? 4 : 8) * a.D * sizeof(T) + 3 * kMaxSlots * sizeof(uint64_t) + kMaxSlots * 8 * sizeof(float) + GemvSmem<QT>::bytes(a.D) + 128;
+  const size_t smem = static_cast<size_t>(a.ring_slots) * (QT == 7 ? 4 : 8) * a.D * sizeof(T) + 3 * kMaxSlots * sizeof(uint64_t) + kMaxSlots * 8 * sizeof(float) + GemvSmem<QT>::bytes(query_area<T>(a.D)) + 128;
   static thread_local SmemSizeCache configured;  // per device
   {
     const int rc = ensure_dyn_smem_size(configured, gemv_ring_kernel<T, QT, NORMS, XB>, smem);
@@ -980,6 +1082,7 @@ static bool ring_ok(int64_t ldc, int D, int dtype, int qt) {
   int slots;
   if (dtype == ICR_F32) slots = ring_slots_q<float>(qt, D);
   else if (dtype == ICR_BF16) slots = ring_slots_q<__nv_bfloat16>(qt, D);
+  else if (dtype == ICR_I8) slots = ring_slots_q<int8_t>(qt, D);
   else slots = ring_slots_q<__half>(qt, D);
   // one slot per warp (no load/compute overlap inside a warp) still wins for 1-3 queries per pass; 4-7 queries
   // (4-row slabs) want two slots per warp
@@ -1012,6 +1115,14 @@ static int launch_gemv_pass(const GemvArgs& a, int qt, bool ring, int g, cudaStr
   return ring ? launch_ring<T, 7, false, XB>(a, g, st) : launch_direct<T, 4, 7, XB>(a, g, st);
 }
 
+// int8 rows: the ring kernels always take the precomputed factors
+template <bool XB>
+static int launch_gemv_pass_i8(const GemvArgs& a, int qt, bool ring, int g, cudaStream_t st) {
+  if (qt == 1) return ring ? launch_ring<int8_t, 1, true, XB>(a, g, st) : launch_direct<int8_t, 8, 1, XB>(a, g, st);
+  if (qt == 3) return ring ? launch_ring<int8_t, 3, true, XB>(a, g, st) : launch_direct<int8_t, 8, 3, XB>(a, g, st);
+  return ring ? launch_ring<int8_t, 7, true, XB>(a, g, st) : launch_direct<int8_t, 4, 7, XB>(a, g, st);
+}
+
 // Runs ceil(Q/7) passes (one for Q <= 7). part_keys/part_cnt sized [Q][grid][k] / [Q][grid].
 // xbits: per-query exclusions of these Q queries (Exclusions::bits with ld xld), or null.
 int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, const void* q, int64_t ldq, int Q,
@@ -1026,7 +1137,8 @@ int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, 
     a.fin_ids = fin_ids;
   }
   // the ring kernel copies the inverse norms with 16-byte bulk copies; an unaligned array falls back to norms from the rows
-  a.cat_inv = (reinterpret_cast<uintptr_t>(cat_inv) & 15) == 0 ? cat_inv : nullptr;
+  // (int8 factors cannot be recovered from the codes: icr_cos_topk requires them 16-byte aligned)
+  a.cat_inv = (dtype == ICR_I8 || (reinterpret_cast<uintptr_t>(cat_inv) & 15) == 0) ? cat_inv : nullptr;
   a.cat = cat;
   a.N = N;
   a.ldc = ldc;
@@ -1056,6 +1168,7 @@ int launch_gemv_topk(const void* cat, int64_t N, int64_t ldc, int D, int dtype, 
     int rc;
     if (dtype == ICR_F32) rc = xbits ? launch_gemv_pass<float, true>(a, qt, ring, g, st) : launch_gemv_pass<float, false>(a, qt, ring, g, st);
     else if (dtype == ICR_BF16) rc = xbits ? launch_gemv_pass<__nv_bfloat16, true>(a, qt, ring, g, st) : launch_gemv_pass<__nv_bfloat16, false>(a, qt, ring, g, st);
+    else if (dtype == ICR_I8) rc = xbits ? launch_gemv_pass_i8<true>(a, qt, ring, g, st) : launch_gemv_pass_i8<false>(a, qt, ring, g, st);
     else rc = xbits ? launch_gemv_pass<__half, true>(a, qt, ring, g, st) : launch_gemv_pass<__half, false>(a, qt, ring, g, st);
     if (rc != ICR_OK) return rc;
     q0 += qt;

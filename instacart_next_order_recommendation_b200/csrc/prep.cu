@@ -221,6 +221,36 @@ int launch_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, 
   return ICR_OK;
 }
 
+// ---- int8 rows (icr_quantize_rows): one warp per row, the format of I8Rows -------------------------------------
+__global__ void __launch_bounds__(256) quantize_rows_kernel(const float* __restrict__ x, int64_t rows, int dim, int64_t ldx,
+                                                            int8_t* __restrict__ codes, int64_t ldc, float* __restrict__ factors,
+                                                            float* __restrict__ tau_init, unsigned int* __restrict__ ovf_init) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+  const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * blockDim.x) >> 5;
+  const int nwords = static_cast<int>(ldc / 4);  // the padding up to the row stride is written as zero codes
+  for (int64_t r = warp; r < rows; r += nwarps) {
+    uint32_t* dst = reinterpret_cast<uint32_t*>(codes + r * ldc);
+    const float f = I8Rows::quantize(x + r * ldx, dim, nwords, lane, [dst](int w, uint32_t word) { dst[w] = word; });
+    if (lane == 0) {
+      factors[r] = f;
+      if (tau_init) tau_init[r] = -INFINITY;  // query side of a tensor-core top-k call, as row_inv_norms_kernel
+      if (ovf_init) ovf_init[r] = 0u;
+    }
+    if (ovf_init && r == 0 && lane < 8) ovf_init[rows + lane] = 0u;  // the grid-barrier counters kept behind the flags
+  }
+}
+
+int launch_quantize_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, int8_t* codes, int64_t ldc, float* factors, cudaStream_t st,
+                         float* tau_init, unsigned int* ovf_init) {
+  if (rows == 0) return ICR_OK;
+  const int64_t want = (rows + 7) / 8;
+  const int blocks = static_cast<int>(want < 148 * 16 ? want : 148 * 16);
+  quantize_rows_kernel<<<blocks, 256, 0, st>>>(x, rows, static_cast<int>(dim), ldx, codes, ldc, factors, tau_init, ovf_init);
+  ICR_LAUNCH_CHECK();
+  return ICR_OK;
+}
+
 // ---- per-query exclusion bitmap (icr_query_exclusion_bits) ------------------------------------------------
 // One warp per query scatters its CSR list into bits[row / 32][q]; rows outside [0, N) are ignored, duplicates are harmless.
 __global__ void __launch_bounds__(256) query_exclusion_bits_kernel(const int64_t* __restrict__ offsets, const int64_t* __restrict__ rows,

@@ -87,6 +87,16 @@ __device__ __forceinline__ void umma_f16_pair(uint32_t d_tmem, uint64_t adesc, u
       "}\n" ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// int8 operands (signed 8-bit A and B, s32 accumulate): K = 32 elements per instruction, the 32 bytes of one f16 step
+__device__ __forceinline__ void umma_i8_pair(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n"
+      ".reg .pred p;\n"
+      "setp.ne.b32 p, %4, 0;\n"
+      "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n"
+      "}\n" ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // arrives (once all MMAs issued so far have completed) on the barrier at this offset in BOTH CTAs
 __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),

@@ -178,13 +178,29 @@ class DeviceCatalog:
     dtype float16 streams as many bytes as bfloat16 with 8x finer rounding: scores are fp32 arithmetic on the fp16
     values (within 1e-5 of fp64 on them), and queries are L2-normalised in fp32 before they are rounded to fp16.
     float16 rows must be finite: un-normalised rows beyond fp16's range raise (normalise them first).
+    dtype int8 quarters the bytes of fp32: each row is stored as int8 codes with one fp32 factor (``ops.quantize_rows``,
+    per-row scalar quantisation) and queries stay float32, quantised by the kernel the same way. Results are exact on the
+    quantised values (ids and score bits are those of integer dot products scaled by the two factors), not within a
+    tolerance of fp32: expect recall@10 around 0.98 against fp32 exact. Rows must be finite.
     """
 
     def __init__(self, embeddings, *, device: torch.device | None = None, dtype: torch.dtype = torch.float32,
                  row_offset: int = 0, build_planes: bool | None = None):
-        if dtype not in (torch.float32, torch.bfloat16, torch.float16):
-            raise TypeError("catalog dtype must be float32, bfloat16 or float16")
+        if dtype not in (torch.float32, torch.bfloat16, torch.float16, torch.int8):
+            raise TypeError("catalog dtype must be float32, bfloat16, float16 or int8")
         dev = device if device is not None else (embeddings.device if isinstance(embeddings, torch.Tensor) and embeddings.is_cuda else default_device())
+        if dtype == torch.int8:
+            if isinstance(embeddings, tuple):  # (codes, factors) of from_index, quantised while streaming
+                codes, factors, input_dim = embeddings
+            else:
+                x = to_device_matrix(embeddings, device=dev).float()
+                if x.numel() and not bool(torch.isfinite(x).all()):
+                    raise ValueError("int8 catalog rows must be finite")
+                input_dim = int(x.shape[1])
+                codes, factors = ops.quantize_rows(x) if x.shape[0] > 0 else (
+                    torch.empty(0, (input_dim + 15) // 16 * 16, dtype=torch.int8, device=dev), torch.empty(0, device=dev))
+            self._init_i8(codes, factors, input_dim, row_offset)
+            return
         if dtype == torch.float16 and _is_f16(embeddings):
             rows = _f16_matrix(embeddings, dev)  # taken bit for bit
         else:
@@ -214,6 +230,17 @@ class DeviceCatalog:
         elif self.rows.shape[0] > 0:
             self.inv_norms = ops.row_inv_norms(self.rows)
 
+    def _init_i8(self, codes: torch.Tensor, factors: torch.Tensor | None, input_dim: int, row_offset: int) -> None:
+        self.input_dim = input_dim
+        self.rows = codes
+        self.row_offset = int(row_offset)
+        self.request_lock = threading.RLock()
+        self._plans: dict = {}
+        self.planes = None
+        # int8 catalogs: the per-row factors of ops.quantize_rows, passed where the ABI takes inverse norms (the factor
+        # carries the row's 1 / |x|, times its quantisation step)
+        self.inv_norms = factors
+
     @classmethod
     def from_index(cls, index: "EmbeddingIndex", product_ids: list[str], *, dtype: torch.dtype = torch.float32,
                    device: torch.device | None = None, rows: tuple[int, int] | None = None, normalize: bool = False,
@@ -224,13 +251,23 @@ class DeviceCatalog:
         serve_recommendations.py:183-204). With dtype bfloat16 a valid ``embeddings.bf16.bin`` sidecar is uploaded
         as is (half the bytes); otherwise (and always for float16) the fp32 rows go up chunk by chunk and
         ``icr_convert_rows`` writes the resident form. ``row_offset`` defaults to lo, so a row-sharded catalog returns global ids.
+        dtype int8 streams the fp32 rows through ``icr_quantize_rows`` (never the sidecar); ``normalize=True`` is rejected,
+        since the factors already normalise.
         """
+        if dtype == torch.int8 and normalize:
+            raise ValueError("normalize=True does not apply to an int8 catalog: its factors carry each row's inverse norm")
         emb = index.open(product_ids)
         if emb is None:
             return None
         dev = device if device is not None else default_device()
         lo, hi = (0, emb.shape[0]) if rows is None else (max(0, int(rows[0])), min(emb.shape[0], int(rows[1])))
         hi = max(lo, hi)
+        if dtype == torch.int8:
+            if emb.shape[1] % 4:  # icr_quantize_rows reads 16-byte vectors: such a catalog goes up as fp32 and is padded
+                resident = upload_rows(emb, lo, hi, device=dev, dtype=torch.float32, chunk_rows=chunk_rows)
+                return cls(resident, device=dev, dtype=dtype, row_offset=lo if row_offset is None else row_offset)
+            codes, factors = upload_quantized(emb, lo, hi, device=dev, chunk_rows=chunk_rows)
+            return cls((codes, factors, int(emb.shape[1])), device=dev, dtype=dtype, row_offset=lo if row_offset is None else row_offset)
         side = index.open_bf16_sidecar(product_ids, _emb=emb) if (use_sidecar and dtype == torch.bfloat16 and not normalize) else None
         # icr_convert_rows works on 16-byte vectors: an embedding dim that is not a multiple of 4 goes up as fp32 and is
         # converted (and padded) by the DeviceCatalog constructor instead
@@ -256,9 +293,16 @@ class DeviceCatalog:
     def dim(self) -> int:
         return self.rows.shape[1]
 
+    @property
+    def query_dtype(self) -> torch.dtype:
+        """The dtype of the queries the kernels read: the catalog's, except float32 for an int8 catalog."""
+        return torch.float32 if self.dtype == torch.int8 else self.dtype
+
     def _device_queries(self, queries) -> torch.Tensor:
-        """Queries on the catalog's device in the form its kernels take: its dtype; for float16 catalogs float16 queries
-        as given and any other dtype through ``ops.normalized_f16``."""
+        """Queries on the catalog's device in the form its kernels take: ``query_dtype``; for float16 catalogs float16
+        queries as given and any other dtype through ``ops.normalized_f16``."""
+        if self.dtype == torch.int8:
+            return to_device_matrix(queries, device=self.device, dtype=torch.float32)
         if self.dtype != torch.float16:
             return to_device_matrix(queries, device=self.device, dtype=self.dtype)
         if _is_f16(queries):
@@ -284,7 +328,7 @@ class DeviceCatalog:
         key = (Q, k, path, convert)
         entry = self._graphs.get(key)
         if entry is None:
-            static_q = torch.zeros(Q, self.rows.shape[1], dtype=torch.float32 if convert else self.dtype, device=self.device)
+            static_q = torch.zeros(Q, self.rows.shape[1], dtype=torch.float32 if convert else self.query_dtype, device=self.device)
             static_q16 = torch.empty(Q, self.rows.shape[1], dtype=torch.float16, device=self.device) if convert else None
 
             # the graph owns its workspace: zero-filled once here, then only this graph's kernels touch it, so the per-call
@@ -330,7 +374,7 @@ class DeviceCatalog:
             return self.topk(q, max(k, 1))
         if D != self.input_dim:
             raise ValueError(f"embedding dims differ: query {D} vs catalog {self.input_dim}")
-        if Q <= 7 and q.is_cuda and q.dtype == rows.dtype and q.device == rows.device and D == rows.shape[1] and q.is_contiguous() \
+        if Q <= 7 and q.is_cuda and q.dtype == self.query_dtype and q.device == rows.device and D == rows.shape[1] and q.is_contiguous() \
                 and q.data_ptr() % 16 == 0:
             # a device-resident query in the catalog's own layout (what encode(convert_to_tensor=True) hands over): the kernel
             # reads it where it lies - no copy into a graph's input buffer, one kernel launch through a prepared argument list
@@ -359,7 +403,7 @@ class DeviceCatalog:
         k = min(int(k), rows.shape[0])
         Q, D = q.shape
         with self.request_lock:
-            if not (1 <= Q <= 7 and k >= 1 and q.is_cuda and q.dtype == rows.dtype and q.device == rows.device and D == rows.shape[1]
+            if not (1 <= Q <= 7 and k >= 1 and q.is_cuda and q.dtype == self.query_dtype and q.device == rows.device and D == rows.shape[1]
                     and D == self.input_dim and q.is_contiguous() and q.data_ptr() % 16 == 0):
                 vals, ids = self.topk_small(q, k, path=path, copy=False)
                 return vals.tolist(), ids.tolist()
@@ -523,7 +567,7 @@ class DeviceCatalog:
         q = queries
         rows = self.rows
         if (exclude_mask is None and peer is None and isinstance(q, torch.Tensor) and q.dim() == 2 and 1 <= q.shape[0] <= 7 and q.is_cuda
-                and q.dtype == rows.dtype and q.device == rows.device and q.shape[1] == rows.shape[1] == self.input_dim and q.is_contiguous()
+                and q.dtype == self.query_dtype and q.device == rows.device and q.shape[1] == rows.shape[1] == self.input_dim and q.is_contiguous()
                 and q.data_ptr() % 16 == 0 and 1 <= int(k) <= rows.shape[0]):
             # request-sized device query in the catalog's layout: the prepared argument list of the request path, fresh outputs
             with self.request_lock:
@@ -670,3 +714,44 @@ def upload_rows(src: np.ndarray, lo: int, hi: int, *, device: torch.device, dtyp
         t.record_stream(side)  # allocated on the current stream, last used on the side stream
     side.synchronize()  # the staging buffers are reused by the next load
     return out
+
+
+def upload_quantized(src: np.ndarray, lo: int, hi: int, *, device: torch.device,
+                     chunk_rows: int = 1 << 15) -> tuple[torch.Tensor, torch.Tensor]:
+    """Rows [lo, hi) of a host fp32 matrix (D % 4 == 0) -> (int8 codes [hi-lo, round_up(D, 16)], factors [hi-lo]) on the
+    device, chunk by chunk through the pinned staging of ``upload_rows``: ``icr_quantize_rows`` writes each chunk's codes
+    and factors where they belong. Raises ValueError if a row is not finite (checked on the device, one sync at the end)."""
+    n, D = hi - lo, int(src.shape[1])
+    codes = torch.empty(n, (D + 15) // 16 * 16, dtype=torch.int8, device=device)
+    factors = torch.empty(n, dtype=torch.float32, device=device)
+    if n == 0:
+        return codes, factors
+    lib = ops._lib.load()
+    chunk_rows = min(max(1, int(chunk_rows)), n)
+    pinned = [_pinned_stage(b, chunk_rows, D, torch.float32) for b in range(2)]
+    staged = [torch.empty(chunk_rows, D, dtype=torch.float32, device=device) for _ in range(2)]
+    bad = torch.zeros((), dtype=torch.int64, device=device)
+    free = [torch.cuda.Event(), torch.cuda.Event()]
+    side = torch.cuda.Stream(device)
+    side.wait_stream(torch.cuda.current_stream(device))
+    for i, (s0, s1) in enumerate(chunk_spans(lo, hi, chunk_rows)):
+        b, m = i & 1, s1 - s0
+        if i >= 2:
+            free[b].synchronize()
+        host = pinned[b][:m]
+        _host_copy(host.numpy(), src[s0:s1])
+        with torch.cuda.stream(side):
+            x = staged[b][:m]
+            x.copy_(host, non_blocking=True)
+            bad += (~torch.isfinite(x)).sum()
+            with ops._on(device):
+                ops._lib.check(lib.icr_quantize_rows(x.data_ptr(), m, D, D, codes[s0 - lo].data_ptr(), codes.shape[1],
+                                                     factors[s0 - lo :].data_ptr(), side.cuda_stream))
+            free[b].record(side)
+    torch.cuda.current_stream(device).wait_stream(side)
+    for t in (*staged, bad):
+        t.record_stream(side)
+    side.synchronize()
+    if int(bad):
+        raise ValueError("int8 catalog rows must be finite")
+    return codes, factors

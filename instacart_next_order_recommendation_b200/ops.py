@@ -11,16 +11,16 @@ import contextlib
 import torch
 
 from . import _lib
-from ._lib import ICR_BF16, ICR_F16, ICR_F32, MAX_K, PATH_AUTO, PATH_GEMM, PATH_GEMV, PATH_WS_RESIDENT  # noqa: F401
+from ._lib import ICR_BF16, ICR_F16, ICR_F32, ICR_I8, MAX_K, PATH_AUTO, PATH_GEMM, PATH_GEMV, PATH_WS_RESIDENT  # noqa: F401
 
-_DTYPES = {torch.float32: ICR_F32, torch.bfloat16: ICR_BF16, torch.float16: ICR_F16}
+_DTYPES = {torch.float32: ICR_F32, torch.bfloat16: ICR_BF16, torch.float16: ICR_F16, torch.int8: ICR_I8}
 
 
 def _dtype_code(t: torch.Tensor) -> int:
     try:
         return _DTYPES[t.dtype]
     except KeyError:
-        raise TypeError(f"libicr_b200 supports float32, bfloat16 and float16 embeddings, got {t.dtype}") from None
+        raise TypeError(f"libicr_b200 supports float32, bfloat16 and float16 embeddings and int8 top-k catalogs, got {t.dtype}") from None
 
 
 def _require_cuda(name: str, t: torch.Tensor) -> None:
@@ -171,8 +171,32 @@ def normalized_f16(x: torch.Tensor) -> torch.Tensor:
     return convert_rows(x, torch.empty(x.shape, dtype=torch.float16, device=x.device), normalize=True)
 
 
+def quantize_rows(x: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:
+    """Device rows -> (int8 codes [rows, round_up(dim, 16)], float32 factors [rows]): the int8 catalog format.
+
+    Per row, m = max |x_i|, code_i = clamp(rint(127 * (x_i / m)), -127, 127) and factor = (m / 127) / max(|x|, 1e-12), in
+    fp32 with round-to-nearest at every step (one ``icr_quantize_rows`` launch); an all-zero row has zero codes and
+    factor 0. The factor carries the row's inverse norm, so the rows need no normalisation. Other dtypes are up-cast to
+    float32 first; the padding columns are zero codes. The rows must be finite."""
+    _require_cuda("x", x)
+    if x.dim() != 2:
+        raise ValueError(f"expected a [rows, dim] matrix, got shape {tuple(x.shape)}")
+    x = _rows(x.float())
+    rows, dim = x.shape
+    codes = torch.empty(rows, (dim + 15) // 16 * 16, dtype=torch.int8, device=x.device)
+    factors = torch.empty(rows, dtype=torch.float32, device=x.device)
+    lib = _lib.load()
+    with _on(x.device):
+        _lib.check(lib.icr_quantize_rows(x.data_ptr(), rows, dim, _ld(x), codes.data_ptr(), codes.shape[1], factors.data_ptr(),
+                                         _stream(x.device)))
+    return codes, factors
+
+
 def _like_catalog(q: torch.Tensor, catalog_dtype: torch.dtype) -> torch.Tensor:
-    """Queries in the catalog's dtype: float16 catalogs take normalised-then-rounded queries (``normalized_f16``)."""
+    """Queries in the form a catalog takes: its dtype; float16 catalogs take normalised-then-rounded queries
+    (``normalized_f16``); int8 catalogs take float32 queries (the call quantises them)."""
+    if catalog_dtype == torch.int8:
+        return q.float()
     if q.dtype == catalog_dtype:
         return q
     return normalized_f16(q) if catalog_dtype == torch.float16 else q.to(catalog_dtype)
@@ -238,7 +262,9 @@ def cos_topk(
     """(values f32 [Q,k] descending, ids int64 [Q,k]) == torch.topk(cos_sim(q, c), k, dim=1).
 
     The catalog is float32, bfloat16 or float16; queries of another dtype are converted to the catalog's (for float16:
-    ``normalized_f16``). ``exclude_mask`` (uint8/bool [N]) drops rows for every query; ``exclude_bits`` (``query_exclusion_bits``, uint32
+    ``normalized_f16``). An int8 catalog (the codes of ``quantize_rows``) needs its factors as ``cat_inv_norms`` and takes
+    float32 queries (others are up-cast), which the call quantises the same way: rows are ranked by fp32(S) * factor, S the
+    exact integer dot product of the codes, and the scores are that times the query's factor. ``exclude_mask`` (uint8/bool [N]) drops rows for every query; ``exclude_bits`` (``query_exclusion_bits``, uint32
     [ceil(N/32), Q]) drops rows per query. A row is dropped when either says so; queries with fewer than k eligible rows
     get a (-inf, -1) tail.
 
@@ -248,6 +274,11 @@ def cos_topk(
     _require_cuda("queries", queries)
     _require_cuda("catalog", catalog)
     queries, catalog = _rows(_like_catalog(queries, catalog.dtype)), _rows(catalog)
+    if catalog.dtype == torch.int8:
+        if cat_inv_norms is None:
+            raise ValueError("an int8 catalog needs its factors (quantize_rows) as cat_inv_norms")
+        if queries.shape[1] < catalog.shape[1]:  # the catalog's padding columns are zero codes: pad the queries alike
+            queries = _rows(torch.nn.functional.pad(queries, (0, catalog.shape[1] - queries.shape[1])))
     if queries.shape[1] != catalog.shape[1]:
         raise ValueError(f"embedding dims differ: {queries.shape[1]} vs {catalog.shape[1]}")
     Q, D = queries.shape
@@ -274,7 +305,7 @@ def cos_topk(
             raise ValueError("cat_planes must be the contiguous plane returned by screen_plane(catalog)")
     if cat_inv_norms is not None:
         if cat_inv_norms.dtype != torch.float32 or cat_inv_norms.shape != (N,) or not cat_inv_norms.is_contiguous():
-            raise ValueError("cat_inv_norms must be the output of row_inv_norms(catalog)")
+            raise ValueError("cat_inv_norms must be the output of row_inv_norms(catalog) (int8: the factors of quantize_rows)")
     if out is None:
         vals = torch.empty(Q, k, dtype=torch.float32, device=dev)
         ids = torch.empty(Q, k, dtype=torch.int64, device=dev)

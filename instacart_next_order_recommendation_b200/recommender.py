@@ -67,7 +67,8 @@ class Recommender:
         self.product_embeddings = self._load_or_build_embeddings(batch_size, use_index)
         if catalog_dtype is None:
             env = os.getenv("ICR_CATALOG_DTYPE", "fp32").lower()
-            catalog_dtype = {"bf16": torch.bfloat16, "bfloat16": torch.bfloat16, "fp16": torch.float16, "float16": torch.float16}.get(env, torch.float32)
+            catalog_dtype = {"bf16": torch.bfloat16, "bfloat16": torch.bfloat16, "fp16": torch.float16, "float16": torch.float16,
+                             "int8": torch.int8, "i8": torch.int8}.get(env, torch.float32)
         dev = torch.device(device) if device is not None else None
         self.catalog = DeviceCatalog(self.product_embeddings, device=dev, dtype=catalog_dtype)
         # SURVEY §8f row 1: ask the encoder for a device tensor so that the query never visits the host between the
