@@ -113,6 +113,23 @@ int icr_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx,
 int icr_quantize_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, int8_t* codes, int64_t ldc, float* factors,
                       void* stream);
 
+/* In-place catalog update: source row i of the fp32 rows x [M, dim] (row stride ldx) replaces catalog row dst_rows[i], in
+ * the catalog's resident form and with that row's derived data, bit for bit what the bulk entries write for the same row:
+ *   ICR_F32   rows[r] = x_i, or x_i / max(||x_i||, 1e-12) with `normalize`, as icr_convert_rows; with `plane` (non-NULL) the
+ *             plane row [round_up(dim, 64)] and inv_norms[r] as icr_screen_plane over the row written, otherwise inv_norms[r]
+ *             as icr_row_inv_norms. The two fp32 inverse norms can differ in the last bit: pass the plane exactly when the
+ *             catalog's inverse norms came from icr_screen_plane
+ *   ICR_BF16 / ICR_F16  rows[r] converted as icr_convert_rows (RNE, optional normalisation); inv_norms[r] as
+ *             icr_row_inv_norms over the CONVERTED row; dim % 8 == 0 (x padded with zero columns to the row width)
+ *   ICR_I8    codes rows[r] (ld_rows bytes, >= round_up(dim, 16), the padding written as zero codes) and factor inv_norms[r]
+ *             as icr_quantize_rows; `normalize` is ICR_ERR_ARG, `plane` must be NULL
+ * dim is the row width of x and of the catalog's rows (dim % 4 == 0); inv_norms is required. dst_rows [M] int64 is device
+ * memory; entries outside [0, N) are ignored, as icr_query_exclusion_bits ignores them; duplicate destinations are
+ * undefined. One launch, one warp per row, on `stream`: the caller orders it after the calls that read the rows. Pointers
+ * and N stay valid, so a prepared call or a captured graph over the catalog returns the new rows' results afterwards. */
+int icr_update_rows(const float* x, int64_t M, int64_t dim, int64_t ldx, const int64_t* dst_rows, int64_t N,
+                    int dtype, void* rows, int64_t ld_rows, uint16_t* plane, float* inv_norms, int normalize, void* stream);
+
 /* ---------------------------------------------------------------------------------------
  * Fused cosine top-k  ==  torch.topk(cos_sim(queries, catalog), k, dim=1, sorted=True)
  * with ties broken by the lower catalog row.

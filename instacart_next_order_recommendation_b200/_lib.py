@@ -48,6 +48,10 @@ SIGNATURES = {
     "icr_screen_plane_row_elems": (c_int64, [c_int64]),
     "icr_convert_rows": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_int, c_int, c_void_p]),
     "icr_quantize_rows": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_void_p, c_void_p]),
+    "icr_update_rows": (
+        c_int,
+        [c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_int, c_void_p],
+    ),
     "icr_cos_topk_workspace_bytes": (c_size_t, [c_int64, c_int64, c_int64, c_int, c_int, c_int, c_int]),
     "icr_cos_topk": (
         c_int,

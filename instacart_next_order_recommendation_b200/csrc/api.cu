@@ -59,6 +59,8 @@ int launch_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, 
                         cudaStream_t st);
 int launch_quantize_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, int8_t* codes, int64_t ldc, float* factors, cudaStream_t st,
                          float* tau_init = nullptr, unsigned int* ovf_init = nullptr);
+int launch_update_rows(const float* x, int64_t M, int64_t dim, int64_t ldx, const int64_t* dst_rows, int64_t N, int dtype, void* rows,
+                       int64_t ld_rows, uint16_t* plane, float* inv_norms, int normalize, cudaStream_t st);
 int launch_peer_exchange_merge(const float* scores, const int64_t* ids, int64_t Q, int k, const PeerTail& peer, float* os, int64_t* oi,
                                cudaStream_t st);
 bool gemv_peer_tail_fits(int Q, int k, int world);
@@ -668,6 +670,48 @@ int icr_convert_rows(const float* x, int64_t rows, int64_t dim, int64_t ldx, voi
   }
   if ((rc = check_device())) return rc;
   return launch_convert_rows(x, rows, dim, ldx, out, ldo, out_dtype, normalize ? 1 : 0, static_cast<cudaStream_t>(stream));
+}
+
+int icr_update_rows(const float* x, int64_t M, int64_t dim, int64_t ldx, const int64_t* dst_rows, int64_t N, int dtype, void* rows,
+                    int64_t ld_rows, uint16_t* plane, float* inv_norms, int normalize, void* stream) {
+  g_launches = 0;
+  if (dtype != ICR_F32 && dtype != ICR_BF16 && dtype != ICR_F16 && dtype != ICR_I8) {
+    set_error("update_rows: unsupported catalog dtype %d", dtype);
+    return ICR_ERR_DTYPE;
+  }
+  if (M < 0 || N < 0 || N >= 0xffffffffll) {
+    set_error("update_rows: bad arguments M=%lld N=%lld", (long long)M, (long long)N);
+    return ICR_ERR_ARG;
+  }
+  if (dtype == ICR_I8 && normalize) {
+    set_error("update_rows: normalize does not apply to an int8 catalog (its factors carry each row's inverse norm)");
+    return ICR_ERR_ARG;
+  }
+  if (plane && dtype != ICR_F32) {
+    set_error("update_rows: only fp32 catalogs have a screening plane");
+    return ICR_ERR_ARG;
+  }
+  int rc = check_matrix("update_rows.x", x, M, dim, ldx, ICR_F32);
+  if (rc) return rc;
+  if (M > 0 && (!dst_rows || !rows || !inv_norms)) {
+    set_error("update_rows: dst_rows, rows and inv_norms must be non-null");
+    return ICR_ERR_ARG;
+  }
+  if (dtype == ICR_I8) {
+    if (ld_rows < (dim + 15) / 16 * 16 || ld_rows % 16 != 0 || (reinterpret_cast<uintptr_t>(rows) & 15)) {
+      set_error("update_rows: int8 codes need a 16-byte aligned base and a row stride >= round_up(dim, 16), a multiple of 16");
+      return ICR_ERR_ALIGN;
+    }
+  } else if ((rc = check_matrix("update_rows.rows", M > 0 ? rows : nullptr, M > 0 ? 1 : 0, dim, ld_rows, dtype))) {
+    return rc;
+  }
+  if (plane && (reinterpret_cast<uintptr_t>(plane) & 127)) {
+    set_error("update_rows: plane must be 128-byte aligned");
+    return ICR_ERR_ALIGN;
+  }
+  if ((rc = check_device())) return rc;
+  return launch_update_rows(x, M, dim, ldx, dst_rows, N, dtype, rows, ld_rows, plane, inv_norms, normalize ? 1 : 0,
+                            static_cast<cudaStream_t>(stream));
 }
 
 size_t icr_peer_buffer_bytes(int64_t n_max, int world) {

@@ -182,7 +182,20 @@ class DeviceCatalog:
     per-row scalar quantisation) and queries stay float32, quantised by the kernel the same way. Results are exact on the
     quantised values (ids and score bits are those of integer dot products scaled by the two factors), not within a
     tolerance of fp32: expect recall@10 around 0.98 against fp32 exact. Rows must be finite.
+
+    ``update_rows``, ``append_rows`` and ``remove_rows`` change the catalog in place. The result equals a catalog freshly built
+    from the updated fp32 matrix in the same row order through the same constructor path: rows, planes and inverse norms
+    bit for bit, and so every top-k result. Updated rows are normalised when ``from_index(normalize=True)`` normalised the
+    catalog (``normalized``). A bfloat16 catalog loaded from the sidecar converts updated fp32 rows with round-to-nearest-even,
+    as ``from_index(use_sidecar=False)`` would. A catalog built from a float32 device tensor shares that tensor's memory until
+    its first change, which copies it. Each change holds ``request_lock``, waits for the work already enqueued on the device
+    and synchronises before it returns; ``topk`` batches that other threads run during a change must be ordered by the caller.
     """
+
+    # the kernels keep row ids in 32 bits, with 2^32 - 1 reserved
+    MAX_ROWS = 0xFFFFFFFF - 1
+    # first growth of an appended catalog: rows, plane and inverse norms are reallocated together with this much headroom
+    GROWTH = 1.5
 
     def __init__(self, embeddings, *, device: torch.device | None = None, dtype: torch.dtype = torch.float32,
                  row_offset: int = 0, build_planes: bool | None = None):
@@ -222,6 +235,12 @@ class DeviceCatalog:
         self.planes: torch.Tensor | None = None
         if build_planes is None:
             build_planes = dtype == torch.float32
+        self.normalized = False  # set by from_index(normalize=True): updated rows are normalised alike
+        self._with_planes = bool(build_planes) and dtype == torch.float32
+        # the rows may be the caller's tensor (an fp32 device matrix is taken as is): the first change copies them
+        self._shared_rows = isinstance(embeddings, torch.Tensor) and embeddings.is_cuda and \
+            embeddings.untyped_storage().data_ptr() == self.rows.untyped_storage().data_ptr()
+        self._reserve: tuple | None = None  # (rows, planes, inv_norms) storage once the catalog has changed
         self.inv_norms: torch.Tensor | None = None
         if build_planes and dtype == torch.float32 and self.rows.shape[0] > 0:
             # fp32 catalogs: the fp32 rows serve the GEMV path and the exact re-scoring; the tensor-core sweep reads a
@@ -237,6 +256,7 @@ class DeviceCatalog:
         self.request_lock = threading.RLock()
         self._plans: dict = {}
         self.planes = None
+        self.normalized, self._with_planes, self._shared_rows, self._reserve = False, False, False, None
         # int8 catalogs: the per-row factors of ops.quantize_rows, passed where the ABI takes inverse norms (the factor
         # carries the row's 1 / |x|, times its quantisation step)
         self.inv_norms = factors
@@ -276,7 +296,10 @@ class DeviceCatalog:
             raise ValueError("normalize=True needs an embedding dim that is a multiple of 4")
         resident = upload_rows(side if side is not None else emb, lo, hi, device=dev, dtype=torch.float32 if odd else dtype,
                                normalize=normalize, chunk_rows=chunk_rows, source_is_bf16_bits=side is not None)
-        return cls(resident, device=dev, dtype=dtype, row_offset=lo if row_offset is None else row_offset)
+        cat = cls(resident, device=dev, dtype=dtype, row_offset=lo if row_offset is None else row_offset)
+        cat.normalized = bool(normalize)
+        cat._shared_rows = False  # the loader's tensor: nobody else holds it
+        return cat
 
     @property
     def device(self) -> torch.device:
@@ -313,6 +336,139 @@ class DeviceCatalog:
     def nbytes(self) -> int:
         extra = sum(t.numel() * t.element_size() for t in (self.planes, self.inv_norms) if t is not None)
         return self.rows.numel() * self.rows.element_size() + extra
+
+    # ---- in-place changes ----------------------------------------------------------------------------------
+    def update_rows(self, rows, embeddings) -> None:
+        """Replace the local rows `rows` (before ``row_offset``) with `embeddings` [len(rows), input_dim] of any float
+        dtype (up-cast to float32; float16 rows land bit for bit in a float16 catalog), in place: one ``icr_update_rows``
+        launch writes each row in the resident form with its inverse norm (int8: codes and factor) and, for float32, its
+        screening-plane row. Pointers and length do not change, so cached CUDA graphs, prepared calls and resident
+        workspaces stay valid and return the new rows' results. Raises ValueError, leaving the catalog unchanged, on
+        duplicate or out-of-range rows, a dim mismatch, non-finite input or float16 overflow."""
+        with self.request_lock:
+            idx = self._row_index(rows, len(self))
+            x = self._update_source(embeddings)
+            if x.shape[0] != idx.size:
+                raise ValueError(f"{idx.size} rows but {x.shape[0]} embeddings")
+            if idx.size == 0:
+                return
+            torch.cuda.synchronize(self.device)  # work enqueued on any stream of the device reads the old rows first
+            if self._shared_rows:
+                self._reallocate(len(self), len(self))
+            self._write(idx, x)
+            torch.cuda.current_stream(self.device).synchronize()
+
+    def append_rows(self, embeddings) -> range:
+        """Append `embeddings` [M, input_dim] as new rows; returns their local row range. The first append reserves
+        ``GROWTH`` times the rows (rows, plane and inverse norms reallocated together); later appends write into the reserve
+        until it is full. ``rows`` stays a [len, ld] tensor (a view of the reserve). Prepared calls, CUDA graphs and resident
+        workspaces are sized for the old length and are dropped. Validation as ``update_rows``; more than ``MAX_ROWS`` rows
+        raise."""
+        with self.request_lock:
+            x = self._update_source(embeddings)
+            n, m = len(self), x.shape[0]
+            if m == 0:
+                return range(n, n)
+            if n + m > self.MAX_ROWS:
+                raise ValueError(f"a catalog holds at most {self.MAX_ROWS} rows ({n} + {m} requested)")
+            torch.cuda.synchronize(self.device)
+            cap = self._reserve[0].shape[0] if self._reserve is not None and not self._shared_rows else 0
+            if n + m > cap:
+                self._reallocate(n, max(n + m, int(n * self.GROWTH)))
+            self._set_length(n + m)
+            self._write(np.arange(n, n + m, dtype=np.int64), x)
+            torch.cuda.current_stream(self.device).synchronize()
+            return range(n, n + m)
+
+    # rows moved per step of remove_rows: its extra memory is one such chunk of rows, planes and norms
+    REMOVE_CHUNK_ROWS = 1 << 16
+
+    def remove_rows(self, rows) -> np.ndarray:
+        """Remove the local rows `rows` and compact the rest in place, stably: the remaining rows keep their order (ties
+        still go to the lower row, as in a fresh build). Returns the old indices of the kept rows, ascending. The memory
+        freed stays reserved for appends; the extra memory of the call is one chunk of ``REMOVE_CHUNK_ROWS`` rows. Drops the
+        cached request state as ``append_rows`` does. Duplicate or out-of-range rows raise ValueError and change nothing."""
+        with self.request_lock:
+            n = len(self)
+            idx = self._row_index(rows, n)
+            keep = np.ones(n, dtype=bool)
+            keep[idx] = False
+            kept = np.flatnonzero(keep)
+            if idx.size == 0:
+                return kept
+            torch.cuda.synchronize(self.device)
+            if self._shared_rows:
+                self._reallocate(n, n)
+            self._reserve = self._storage()
+            bufs = [t for t in self._reserve if t is not None]
+            first = int(idx.min())  # rows below the first removed one stay where they are
+            for a in range(first, kept.size, self.REMOVE_CHUNK_ROWS):
+                b = min(kept.size, a + self.REMOVE_CHUNK_ROWS)
+                src = torch.from_numpy(kept[a:b]).to(self.device)
+                for t in bufs:  # kept[j] >= j: a chunk reads only rows at or beyond the ones it writes
+                    t[a:b] = t.index_select(0, src)
+            self._set_length(kept.size)
+            torch.cuda.current_stream(self.device).synchronize()
+            return kept
+
+    def _row_index(self, rows, n: int) -> np.ndarray:
+        t = rows.detach().cpu().numpy() if isinstance(rows, torch.Tensor) else np.asarray(list(rows) if not isinstance(rows, np.ndarray) else rows)
+        if t.size and not np.issubdtype(t.dtype, np.integer):
+            raise ValueError(f"row indices must be integers, got {t.dtype}")
+        idx = t.astype(np.int64).reshape(-1)
+        if idx.size and (idx.min() < 0 or idx.max() >= n):
+            raise ValueError(f"row indices must lie in [0, {n})")
+        if np.unique(idx).size != idx.size:
+            raise ValueError("duplicate row indices")
+        return idx
+
+    def _update_source(self, embeddings) -> torch.Tensor:
+        """`embeddings` as validated float32 device rows [M, rows.shape[1]] (the padding columns zero)."""
+        x = embeddings if isinstance(embeddings, torch.Tensor) else torch.as_tensor(np.asarray(embeddings))
+        if x.dim() == 1:
+            x = x.unsqueeze(0)
+        if x.dim() != 2 or not x.is_floating_point():
+            raise ValueError(f"expected floating-point [rows, dim] embeddings, got {x.dtype} {tuple(x.shape)}")
+        if x.shape[1] != self.input_dim:
+            raise ValueError(f"embedding dims differ: {x.shape[1]} vs catalog {self.input_dim}")
+        x = x.to(device=self.device, dtype=torch.float32)
+        if x.numel() and not bool(torch.isfinite(x).all()):
+            raise ValueError("catalog rows must be finite")
+        if self.dtype == torch.float16 and not self.normalized and x.numel() and not bool(torch.isfinite(x.half()).all()):
+            raise ValueError("catalog rows exceed float16's range (inf after conversion): L2-normalise them first")
+        if x.shape[1] != self.rows.shape[1]:
+            x = torch.nn.functional.pad(x, (0, self.rows.shape[1] - x.shape[1]))
+        return x.contiguous()
+
+    def _write(self, idx: np.ndarray, x: torch.Tensor) -> None:
+        ops.update_rows(x, torch.from_numpy(idx).to(self.device), self.rows, self.inv_norms, planes=self.planes, normalize=self.normalized)
+
+    def _storage(self) -> tuple:
+        return self._reserve if self._reserve is not None else (self.rows, self.planes, self.inv_norms)
+
+    def _reallocate(self, n: int, cap: int) -> None:
+        """New storage for `cap` rows holding the first `n` rows of the current one."""
+        dev, width = self.device, self.rows.shape[1]
+        rows = torch.empty(cap, width, dtype=self.rows.dtype, device=dev)
+        rows[:n] = self.rows[:n]
+        planes = None
+        if self.planes is not None or (n == 0 and self._with_planes):
+            planes = torch.empty(cap, ops._lib.load().icr_screen_plane_row_elems(width), dtype=torch.float16, device=dev)
+            if n:
+                planes[:n] = self.planes[:n]
+        inv = torch.empty(cap, dtype=torch.float32, device=dev)
+        if n:
+            inv[:n] = self.inv_norms[:n]
+        self._reserve, self._shared_rows = (rows, planes, inv), False
+        self._set_length(n)
+
+    def _set_length(self, n: int) -> None:
+        """Views of the first n rows of the storage; the request state bound to the old length or pointers is dropped."""
+        rows, planes, inv = self._storage()
+        self.rows, self.planes, self.inv_norms = rows[:n], None if planes is None else planes[:n], inv[:n]
+        self._plans = {}
+        self.__dict__.pop("_graphs", None)
+        self.__dict__.pop("_resident", None)
 
     # ---- request-sized calls: one CUDA graph per (Q, k) -------------------------------------------------
     def _graph_for(self, Q: int, k: int, path: int, convert: bool = False):

@@ -192,6 +192,28 @@ def quantize_rows(x: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:
     return codes, factors
 
 
+def update_rows(x: torch.Tensor, dst_rows: torch.Tensor, rows: torch.Tensor, inv_norms: torch.Tensor, *,
+                planes: torch.Tensor | None = None, normalize: bool = False) -> None:
+    """Catalog rows ``rows[dst_rows[i]] <- x[i]`` in place, in the catalog's resident form, with their derived data
+    (``icr_update_rows``, one launch): ``inv_norms`` (int8: the factors) and, for float32 catalogs with a screening plane,
+    ``planes``. Each row is bit for bit what the bulk path writes for it (``convert_rows`` / ``screen_plane`` /
+    ``row_inv_norms`` / ``quantize_rows``). `x` is float32 [M, rows.shape[1]] (pad the catalog's zero columns with zeros),
+    `dst_rows` int64 [M] on the device; entries outside [0, len(rows)) are ignored and duplicates are undefined.
+    ``normalize`` L2-normalises the rows first, as ``convert_rows(normalize=True)``; not for int8."""
+    for name, t in (("x", x), ("dst_rows", dst_rows), ("rows", rows), ("inv_norms", inv_norms)):
+        _require_cuda(name, t)
+    if x.dtype != torch.float32 or x.dim() != 2 or x.shape[1] != rows.shape[1] or x.stride(1) != 1:
+        raise ValueError(f"update_rows expects float32 [M, {rows.shape[1]}] rows contiguous in dim, got {x.dtype} {tuple(x.shape)}")
+    if dst_rows.dtype != torch.int64 or dst_rows.shape != (x.shape[0],) or not dst_rows.is_contiguous():
+        raise ValueError("dst_rows must be a contiguous int64 vector with one entry per source row")
+    if inv_norms.dtype != torch.float32 or inv_norms.shape != (rows.shape[0],) or not inv_norms.is_contiguous():
+        raise ValueError("inv_norms must be the catalog's float32 inverse norms (int8: factors), one per row")
+    lib = _lib.load()
+    with _on(rows.device):
+        _lib.check(lib.icr_update_rows(x.data_ptr(), x.shape[0], x.shape[1], _ld(x), dst_rows.data_ptr(), rows.shape[0], _dtype_code(rows),
+                                       rows.data_ptr(), _ld(rows), _ptr(planes), inv_norms.data_ptr(), int(normalize), _stream(rows.device)))
+
+
 def _like_catalog(q: torch.Tensor, catalog_dtype: torch.dtype) -> torch.Tensor:
     """Queries in the form a catalog takes: its dtype; float16 catalogs take normalised-then-rounded queries
     (``normalized_f16``); int8 catalogs take float32 queries (the call quantises them)."""

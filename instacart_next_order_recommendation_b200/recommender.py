@@ -11,9 +11,11 @@ serves many requests in one encode and one fused top-k, each request with its ow
 
 from __future__ import annotations
 
+import contextlib
 import json
 import logging
 import os
+import threading
 import time
 from dataclasses import dataclass
 from pathlib import Path
@@ -42,8 +44,53 @@ class RecommendationMetrics:
     timestamp: float
 
 
+class _ReadWriteLock:
+    """Many readers or one writer; a waiting writer keeps new readers out until it is done."""
+
+    def __init__(self):
+        self._cond = threading.Condition()
+        self._readers = 0
+        self._writing = False
+        self._writers_waiting = 0
+
+    @contextlib.contextmanager
+    def read(self):
+        with self._cond:
+            while self._writing or self._writers_waiting:
+                self._cond.wait()
+            self._readers += 1
+        try:
+            yield
+        finally:
+            with self._cond:
+                self._readers -= 1
+                if self._readers == 0:
+                    self._cond.notify_all()
+
+    @contextlib.contextmanager
+    def write(self):
+        with self._cond:
+            self._writers_waiting += 1
+            while self._writing or self._readers:
+                self._cond.wait()
+            self._writers_waiting -= 1
+            self._writing = True
+        try:
+            yield
+        finally:
+            with self._cond:
+                self._writing = False
+                self._cond.notify_all()
+
+
 class Recommender:
-    """Two-tower recommender: encode the user context, return top-k products by cosine similarity."""
+    """Two-tower recommender: encode the user context, return top-k products by cosine similarity.
+
+    ``update_products``, ``remove_products`` and ``update_corpus`` change the catalog under a running server: the texts that
+    are new or changed are encoded, and the resident catalog is changed in place (``DeviceCatalog.update_rows`` /
+    ``append_rows`` / ``remove_rows``) instead of being rebuilt. Requests run concurrently with each other; a change waits
+    for the running ones and holds new ones back until it is done, so a request sees the catalog wholly before or wholly
+    after it."""
 
     def __init__(
         self,
@@ -58,6 +105,9 @@ class Recommender:
     ):
         p = Path(model_dir)
         self.model_dir = p.resolve() if p.exists() else model_dir
+        self._batch_size = batch_size
+        self._rw = _ReadWriteLock()  # requests read, catalog changes write
+        self._update_lock = threading.RLock()  # one change at a time, encoding included
         self.corpus_path = Path(corpus_path).resolve()
         self.product_ids, self.product_texts = self._load_corpus()
         self.pid_to_text = dict(zip(self.product_ids, self.product_texts))
@@ -123,6 +173,10 @@ class Recommender:
 
     def _rank(self, query_emb, top_k: int, exclude_product_ids: set[str] | None) -> list[tuple[str, float]]:
         """Equals: sort all rows by score, drop excluded ids, keep the first top_k."""
+        with self._rw.read():
+            return self._rank_locked(query_emb, top_k, exclude_product_ids)
+
+    def _rank_locked(self, query_emb, top_k: int, exclude_product_ids: set[str] | None) -> list[tuple[str, float]]:
         n = len(self.product_ids)
         if top_k <= 0 or n == 0:
             return []
@@ -195,16 +249,96 @@ class Recommender:
             raise ValueError(f"exclude_product_ids has {len(exclude_product_ids)} entries for {len(queries)} queries")
         if not queries:
             return []
-        n = len(self.product_ids)
-        if top_k <= 0 or n == 0:
+        if top_k <= 0 or not self.product_ids:
             return [[] for _ in queries]
         if top_k > ops.MAX_K:
             raise ValueError(f"top_k={top_k} exceeds the fused kernel limit {ops.MAX_K} (the reference API caps top_k at 100)")
-        excluded = [[self._pid_to_row[p] for p in (ex or ()) if p in self._pid_to_row] for ex in (exclude_product_ids or [None] * len(queries))]
         embs = self._encode_queries(queries)
-        k = min(top_k, n)
-        vals, ids = self.catalog.topk(embs, k, exclude_rows=excluded if any(excluded) else None)
-        return [[(self.product_ids[r], float(s)) for s, r in zip(vr, ir) if r >= 0] for vr, ir in zip(vals.tolist(), ids.tolist())]
+        with self._rw.read():
+            n = len(self.product_ids)  # the catalog may have changed while the queries were encoded
+            if n == 0:
+                return [[] for _ in queries]
+            excluded = [[self._pid_to_row[p] for p in (ex or ()) if p in self._pid_to_row]
+                        for ex in (exclude_product_ids or [None] * len(queries))]
+            k = min(top_k, n)
+            vals, ids = self.catalog.topk(embs, k, exclude_rows=excluded if any(excluded) else None)
+            return [[(self.product_ids[r], float(s)) for s, r in zip(vr, ir) if r >= 0] for vr, ir in zip(vals.tolist(), ids.tolist())]
+
+    # ---- catalog changes ---------------------------------------------------------------------------------
+    def update_products(self, products: dict[str, str]) -> None:
+        """Add or change products ({product id: text}). Only texts that are new or differ from the current ones are encoded,
+        in one ``encode`` call; changed products are replaced in place and new ones appended, in the dict's order.
+        ``product_ids``, ``product_texts``, ``pid_to_text`` and ``product_embeddings`` follow."""
+        self._change({}, products)
+
+    def remove_products(self, ids) -> None:
+        """Remove products by id; unknown ids are ignored. The remaining products keep their order."""
+        with self._update_lock:
+            gone = [pid for pid in dict.fromkeys(ids) if pid in self._pid_to_row]
+            with self._rw.write():
+                self._remove_locked(gone)
+
+    def update_corpus(self, corpus: dict[str, str]) -> None:
+        """The corpus becomes `corpus`: products not in it are removed, changed ones replaced and new ones appended.
+        Afterwards ``product_ids`` holds the surviving ids in their old order, then the new ids in corpus order, and
+        ``recommend`` / ``recommend_batch`` answer as a fresh ``Recommender`` over ``{pid: corpus[pid] for pid in
+        product_ids}`` with the same encoder. Writing the corpus file or the ``EmbeddingIndex`` is left to the caller
+        (``EmbeddingIndex.save(product_ids, product_embeddings)``)."""
+        with self._update_lock:
+            self._change(corpus, corpus, remove_missing=True)
+
+    def _plan_change(self, corpus: dict[str, str], products: dict[str, str], remove_missing: bool):
+        """(removed ids, changed ids, new ids) of a change; reads the current state only."""
+        gone = [pid for pid in self.product_ids if pid not in corpus] if remove_missing else []
+        changed = [pid for pid, text in products.items() if pid in self._pid_to_row and self.pid_to_text[pid] != text]
+        new = [pid for pid in products if pid not in self._pid_to_row]
+        return gone, changed, new
+
+    def _change(self, corpus: dict[str, str], products: dict[str, str], remove_missing: bool = False) -> None:
+        with self._update_lock:
+            products = {str(pid): text for pid, text in products.items()}
+            gone, changed, new = self._plan_change(corpus, products, remove_missing)
+            emb = None
+            if changed or new:  # encoded before requests are held back
+                emb = np.asarray(self.model.encode([products[p] for p in changed + new], batch_size=self._batch_size,
+                                                   show_progress_bar=False, normalize_embeddings=True), dtype=np.float32)
+                if emb.ndim != 2 or emb.shape[0] != len(changed) + len(new) or emb.shape[1] != self.catalog.input_dim:
+                    raise ValueError(f"the encoder returned {emb.shape} for {len(changed) + len(new)} texts of dim {self.catalog.input_dim}")
+                if not np.isfinite(emb).all():
+                    raise ValueError("the encoder returned non-finite embeddings")
+            if not (gone or changed or new):
+                return
+            with self._rw.write():
+                self._remove_locked(gone)
+                nc = len(changed)
+                if changed:
+                    rows = [self._pid_to_row[p] for p in changed]
+                    self.catalog.update_rows(rows, emb[:nc])
+                    if not self.product_embeddings.flags.writeable:
+                        self.product_embeddings = np.array(self.product_embeddings)
+                    self.product_embeddings[rows] = emb[:nc]
+                    for p, r in zip(changed, rows):
+                        self.product_texts[r] = products[p]
+                        self.pid_to_text[p] = products[p]
+                if new:
+                    first = self.catalog.append_rows(emb[nc:]).start
+                    self.product_embeddings = np.concatenate([np.asarray(self.product_embeddings), emb[nc:].astype(self.product_embeddings.dtype)])
+                    for j, p in enumerate(new):
+                        self.product_ids.append(p)
+                        self.product_texts.append(products[p])
+                        self.pid_to_text[p] = products[p]
+                        self._pid_to_row[p] = first + j
+
+    def _remove_locked(self, gone: list[str]) -> None:
+        if not gone:
+            return
+        kept = self.catalog.remove_rows([self._pid_to_row[p] for p in gone])
+        for p in gone:
+            del self.pid_to_text[p]
+        self.product_ids = [self.product_ids[i] for i in kept]
+        self.product_texts = [self.product_texts[i] for i in kept]
+        self.product_embeddings = np.asarray(self.product_embeddings)[kept]
+        self._pid_to_row = {pid: i for i, pid in enumerate(self.product_ids)}
 
 
 class MonitoredRecommender(Recommender):

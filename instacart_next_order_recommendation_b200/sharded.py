@@ -12,6 +12,7 @@ from __future__ import annotations
 
 from typing import Callable
 
+import numpy as np
 import torch
 import torch.distributed as dist
 
@@ -220,6 +221,24 @@ class ShardedCatalog:
             return self.local.topk(q, k, peer=self._peer_for(q.shape[0] * k).next_call())
         vals, ids = self.local_topk(queries, k)
         return self.exchange_merge(vals, ids, k)
+
+    def update_rows(self, global_rows, embeddings) -> None:
+        """Replace catalog rows by GLOBAL id in place (``DeviceCatalog.update_rows``). Every rank makes the same call and
+        applies the rows that fall in its block; no collective is needed. Appending and removing rows would move the shard
+        boundaries, and with them the global ids, so a sharded catalog does not offer them."""
+        g = np.asarray(global_rows.detach().cpu() if isinstance(global_rows, torch.Tensor) else global_rows, dtype=np.int64).reshape(-1)
+        if g.size and (g.min() < 0 or g.max() >= self.total_rows):
+            raise ValueError(f"global row ids must lie in [0, {self.total_rows})")
+        if np.unique(g).size != g.size:
+            raise ValueError("duplicate row ids")
+        if len(embeddings) != g.size:
+            raise ValueError(f"{g.size} rows but {len(embeddings)} embeddings")
+        pick = np.flatnonzero((g >= self.row_offset) & (g < self.row_offset + self.n_local))
+        if isinstance(embeddings, torch.Tensor):
+            mine = embeddings[torch.from_numpy(pick).to(embeddings.device)]
+        else:
+            mine = np.asarray(embeddings)[pick]
+        self.local.update_rows(g[pick] - self.row_offset, mine)
 
     def _peer_for(self, n: int) -> "PeerExchange":
         if self._peer is None or self._peer.n_max < n:
