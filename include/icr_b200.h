@@ -198,6 +198,31 @@ int icr_cos_topk_excl(const void* queries, int64_t Q, int64_t ldq,
                       float* out_scores, int64_t* out_ids,
                       void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------------------------------
+ * Cosine top-k over per-query candidate lists: query q ranks only the catalog rows rows[offsets[q] .. offsets[q+1])
+ * (CSR: offsets [Q + 1] int64 with offsets[0] = 0, non-decreasing, offsets[Q] = nnz; rows [nnz] int64; both device memory).
+ * out_scores / out_ids [Q, k] get the k best rows of each list by cosine similarity, descending, ties to the lower row,
+ * ids as row + row_offset. Rows outside [0, N) are ignored; lists may be in any order and of any length. A query with
+ * fewer than k valid rows gets a (-inf, -1) tail, an empty list k x (-inf, -1). The rows of one list must be distinct:
+ * a row listed twice may come back twice.
+ *
+ * Queries, catalog, D and alignment as icr_cos_topk (int8 catalogs: fp32 queries, D % 16 == 0). cat_inv_norms is
+ * required: the rows' inverse norms (int8: the factors of icr_quantize_rows). Scores:
+ *   ICR_F32   bit for bit those of icr_cos_topk's tensor-core path (its exact fp32 re-scoring, and its query norm)
+ *   ICR_BF16, ICR_F16  fp32 FMAs on the 16-bit values times both inverse norms
+ *   ICR_I8    key = fp32(S) * f_row with S the exact int32 code dot product, score = key * f_query: bit for bit K1's
+ * The cost follows nnz, not N: the entries are cut into fixed chunks, so a long list is split over many warps and many
+ * short lists share one. Two launches on `stream` (query preparation, then the top-k with the merge of split lists in its
+ * tail), no synchronisation, no host copies. Workspace: icr_cos_topk_subset_workspace_bytes (256-byte aligned), about
+ * 2 * ceil(nnz / chunk) * k keys plus a few words per query. */
+size_t icr_cos_topk_subset_workspace_bytes(int64_t Q, int64_t nnz, int64_t D, int dtype, int k);
+int icr_cos_topk_subset(const void* queries, int64_t Q, int64_t ldq,
+                        const void* catalog, int64_t N, int64_t ldc, int64_t D, int dtype,
+                        const float* cat_inv_norms,
+                        const int64_t* offsets, const int64_t* rows, int64_t nnz,
+                        int k, int64_t row_offset, float* out_scores, int64_t* out_ids,
+                        void* workspace, size_t workspace_bytes, void* stream);
+
 /* number of kernel launches the last icr_cos_topk call on this thread enqueued */
 int icr_last_launch_count(void);
 

@@ -12,7 +12,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB_DIR = PKG / "lib"
 LIB_PATH = LIB_DIR / "libicr_b200.so"
-SOURCES = ["api.cu", "prep.cu", "gemv_topk.cu", "select.cu", "select_hist.cu", "dense.cu", "mnrl.cu", "mnrl_tc.cu", "metrics.cu", "exchange.cu", "gemm_topk.cu"]
+SOURCES = ["api.cu", "prep.cu", "gemv_topk.cu", "select.cu", "select_hist.cu", "dense.cu", "mnrl.cu", "mnrl_tc.cu", "metrics.cu", "exchange.cu", "gemm_topk.cu", "subset_topk.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

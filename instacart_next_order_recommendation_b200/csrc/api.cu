@@ -101,6 +101,11 @@ int launch_scale2(const void* x0, const void* x1, int64_t n, int dtype, const fl
 bool mnrl_tc_applies(int64_t B, int64_t Bc, int64_t D);
 size_t mnrl_tc_workspace_bytes(int64_t B, int64_t Bc, int64_t D);
 int launch_mnrl_tc(const MnrlArgs& m, int dtype, int mode, void* ws, size_t ws_bytes, cudaStream_t st);
+// candidate-list top-k (subset_topk.cu)
+size_t subset_workspace_bytes(int64_t Q, int64_t nnz, int64_t D, int dtype, int k);
+int launch_subset_topk(const void* queries, int64_t Q, int64_t ldq, const void* catalog, int64_t N, int64_t ldc, int64_t D, int dtype,
+                       const float* cat_inv_norms, const int64_t* offsets, const int64_t* rows, int64_t nnz, int k, int64_t row_offset,
+                       float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes, cudaStream_t st);
 int launch_query_exclusion_bits(const int64_t* offsets, const int64_t* rows, int64_t Q, int64_t N, uint32_t* bits, cudaStream_t st);
 int launch_ir_metrics(const int64_t* ids, int64_t Q, int K, int64_t ld, const int64_t* rel_offsets, const int64_t* rel_rows,
                       const int32_t* n_relevant, const int32_t* kinds, const int32_t* ks, int M, double* per_query, double* means,
@@ -406,6 +411,52 @@ int icr_cos_topk(const void* queries, int64_t Q, int64_t ldq, const void* catalo
                  void* stream) {
   return icr_cos_topk_excl(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_planes, cat_inv_norms, exclude_mask, nullptr, k, row_offset, path,
                            out_scores, out_ids, workspace, workspace_bytes, stream);
+}
+
+size_t icr_cos_topk_subset_workspace_bytes(int64_t Q, int64_t nnz, int64_t D, int dtype, int k) {
+  if (Q < 0 || nnz < 0 || D <= 0 || k < 1 || k > ICR_MAX_K) return 256;
+  return subset_workspace_bytes(Q, nnz, D, dtype, k);
+}
+
+int icr_cos_topk_subset(const void* queries, int64_t Q, int64_t ldq, const void* catalog, int64_t N, int64_t ldc, int64_t D, int dtype,
+                        const float* cat_inv_norms, const int64_t* offsets, const int64_t* rows, int64_t nnz, int k, int64_t row_offset,
+                        float* out_scores, int64_t* out_ids, void* workspace, size_t workspace_bytes, void* stream) {
+  g_launches = 0;
+  int rc;
+  if (dtype == ICR_I8) {  // fp32 queries, quantised by the call
+    if ((rc = check_matrix("cos_topk_subset.queries", queries, Q, D, ldq, ICR_F32))) return rc;
+    if ((rc = check_codes("cos_topk_subset.catalog", catalog, N, D, ldc))) return rc;
+  } else {
+    if ((rc = check_matrix("cos_topk_subset.queries", queries, Q, D, ldq, dtype))) return rc;
+    if ((rc = check_matrix("cos_topk_subset.catalog", catalog, N, D, ldc, dtype))) return rc;
+  }
+  if (N > 0 && !cat_inv_norms) {
+    set_error("cos_topk_subset: cat_inv_norms is required (icr_row_inv_norms / icr_screen_plane; int8: the factors of icr_quantize_rows)");
+    return ICR_ERR_ARG;
+  }
+  if (k < 1 || k > ICR_MAX_K) {
+    set_error("cos_topk_subset: k=%d outside [1, %d]", k, ICR_MAX_K);
+    return ICR_ERR_K;
+  }
+  if (N >= 0xffffffffll || Q >= (1ll << 31) || nnz < 0) {
+    set_error("cos_topk_subset: bad sizes N=%lld Q=%lld nnz=%lld", (long long)N, (long long)Q, (long long)nnz);
+    return ICR_ERR_ARG;
+  }
+  if ((Q > 0 && !offsets) || (nnz > 0 && !rows)) {
+    set_error("cos_topk_subset: null CSR list (offsets [Q + 1], and rows when nnz > 0, must be device pointers)");
+    return ICR_ERR_ARG;
+  }
+  if (Q > 0 && (!out_scores || !out_ids)) {
+    set_error("cos_topk_subset: null output");
+    return ICR_ERR_ARG;
+  }
+  if ((reinterpret_cast<uintptr_t>(workspace) & 255) != 0) {
+    set_error("cos_topk_subset: workspace must be 256-byte aligned");
+    return ICR_ERR_ALIGN;
+  }
+  if ((rc = check_device())) return rc;
+  return launch_subset_topk(queries, Q, ldq, catalog, N, ldc, D, dtype, cat_inv_norms, offsets, rows, nnz, k, row_offset, out_scores, out_ids,
+                            workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
 }
 
 int icr_query_exclusion_bits(const int64_t* offsets, const int64_t* rows, int64_t Q, int64_t N, uint32_t* bits, void* stream) {

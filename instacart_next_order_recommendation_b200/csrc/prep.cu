@@ -1,36 +1,8 @@
 // K5: row inverse norms and the fp16 (hi|lo) operand planes of the fp32-parity tensor path.
 #include "common.cuh"
+#include "rows.cuh"
 
 namespace icr {
-
-__device__ __forceinline__ float4 ldg_stream_f4(const float* p) {
-  const uint4 v = ldg_stream(p);
-  return make_float4(__uint_as_float(v.x), __uint_as_float(v.y), __uint_as_float(v.z), __uint_as_float(v.w));
-}
-
-// One row's sum of squares, on every lane of the calling warp; its inverse norm is 1 / max(sqrt(ss), eps). Lane l
-// sums, with fmaf in element order, the elements of its vectors l, l + 32, ... and then the elements past the last whole
-// vector; then warp_sum. STREAM: read through the non-coherent streaming path (rows that no kernel writes meanwhile);
-// icr_update_rows reads back the row it has just written and needs coherent loads.
-template <typename T, bool STREAM>
-__device__ __forceinline__ float row_sumsq(const T* __restrict__ row, int nvec, int64_t dim, int lane) {
-  constexpr int VEC = Elem<T>::VEC;
-  float ss = 0.f;
-  for (int v = lane; v < nvec; v += 32) {
-    float f[VEC];
-    if constexpr (STREAM)
-      Elem<T>::unpack(ldg_stream(row + static_cast<int64_t>(v) * VEC), f);
-    else
-      Elem<T>::unpack(*reinterpret_cast<const uint4*>(row + static_cast<int64_t>(v) * VEC), f);
-#pragma unroll
-    for (int i = 0; i < VEC; ++i) ss = fmaf(f[i], f[i], ss);
-  }
-  for (int e = nvec * VEC + lane; e < dim; e += 32) {
-    const float f = Elem<T>::to_f32(row[e]);
-    ss = fmaf(f, f, ss);
-  }
-  return warp_sum(ss);
-}
 
 // one warp per row; 128-bit loads; inv = 1 / max(||x||, eps)   (torch F.normalize semantics)
 // tau_init / ovf_init (optional, query side of a top-k call): the per-query threshold starts at -inf and the overflow flag at 0;
@@ -93,16 +65,7 @@ __global__ void __launch_bounds__(256) split_f16_planes_kernel(const float* __re
 template <bool STREAM, typename OnInv>
 __device__ __forceinline__ void screen_row(const float* __restrict__ row, int nvec, int nvec_pad, __half* __restrict__ plane, int64_t off,
                                            int lane, OnInv on_inv) {
-  float ss = 0.f;
-  for (int v = lane; v < nvec; v += 32) {
-    float4 f;
-    if constexpr (STREAM)
-      f = ldg_stream_f4(row + 4 * v);
-    else
-      f = *reinterpret_cast<const float4*>(row + 4 * v);
-    ss = fmaf(f.x, f.x, fmaf(f.y, f.y, fmaf(f.z, f.z, fmaf(f.w, f.w, ss))));
-  }
-  ss = warp_sum(ss);
+  const float ss = screen_sumsq<STREAM>(row, nvec, lane);
   const float inv = 1.0f / fmaxf(sqrtf(ss), kNormEps);
   on_inv(inv);
   const float sc = 256.0f * inv;

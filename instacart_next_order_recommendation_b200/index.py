@@ -708,7 +708,7 @@ class DeviceCatalog:
     EXCLUSION_BITS_MAX_BYTES = 256 << 20
 
     def topk(self, queries, k: int, *, exclude_mask: torch.Tensor | None = None, exclude_rows=None, path: int = ops.PATH_AUTO,
-             peer=None):
+             peer=None, include_rows=None):
         """(values [Q,k], global ids [Q,k]) of the k most cosine-similar rows per query. With ``peer``
         (``PeerExchange.next_call()``; needs k <= len(self)) the rows are one rank's shard and the result is the global
         top-k over all ranks' shards (``ops.cos_topk``).
@@ -717,7 +717,16 @@ class DeviceCatalog:
         local rows per query (before ``row_offset``; out-of-range rows are ignored) that this query never returns: the
         batch is searched in one fused call per chunk of queries whose exclusion bitmap (``ops.query_exclusion_bits``,
         ceil(len(self)/32) words per query) fits EXCLUSION_BITS_MAX_BYTES. A query with fewer than k eligible rows gets a
-        (-inf, -1) tail."""
+        (-inf, -1) tail.
+
+        ``include_rows`` is the opposite: one candidate list of local rows per query (Q iterables, or an ``(offsets, rows)``
+        CSR pair of int64 tensors with distinct rows per list), and query q ranks only its list (``ops.cos_topk_subset``):
+        the call reads the listed rows, not the catalog. It cannot be combined with ``exclude_rows``, ``exclude_mask`` or
+        ``peer``; out-of-range rows are ignored and a list with fewer than k valid rows gets a (-inf, -1) tail."""
+        if include_rows is not None:
+            if exclude_rows is not None or exclude_mask is not None or peer is not None:
+                raise ValueError("include_rows cannot be combined with exclude_rows, exclude_mask or peer")
+            return self._topk_including(queries, k, include_rows)
         if exclude_rows is not None:
             return self._topk_excluding(queries, k, exclude_rows, exclude_mask, path, peer)
         q = queries
@@ -737,6 +746,22 @@ class DeviceCatalog:
         ws = self._resident_workspace(q.shape[0], k, path, peer is not None) if q.shape[0] <= 8 else None
         return ops.cos_topk(q, self.rows, k, cat_planes=self.planes, cat_inv_norms=self.inv_norms, exclude_mask=exclude_mask,
                             row_offset=self.row_offset, path=path, workspace=ws, peer=peer)
+
+    def _topk_including(self, queries, k: int, include_rows):
+        q = self._device_queries(queries)
+        if q.dim() == 1:
+            q = q.unsqueeze(0)
+        Q = q.shape[0]
+        if int(k) > ops.MAX_K:
+            raise ValueError(f"k={k} outside [1, {ops.MAX_K}]")
+        k = min(int(k), len(self))
+        if k < 1:
+            return (torch.empty(Q, 0, device=self.device), torch.empty(Q, 0, dtype=torch.int64, device=self.device))
+        csr = include_rows if isinstance(include_rows, tuple) and len(include_rows) == 2 and all(
+            isinstance(t, torch.Tensor) for t in include_rows) else list(include_rows)
+        if not isinstance(csr, tuple) and len(csr) != Q:
+            raise ValueError(f"include_rows has {len(csr)} entries for {Q} queries")
+        return ops.cos_topk_subset(q, self.rows, k, csr, cat_inv_norms=self.inv_norms, row_offset=self.row_offset)
 
     def _topk_excluding(self, queries, k: int, exclude_rows, exclude_mask, path: int, peer):
         if peer is not None:

@@ -371,6 +371,101 @@ def cos_topk(
     return vals, ids
 
 
+def candidate_lists(rows_per_query, device=None) -> tuple[torch.Tensor, torch.Tensor]:
+    """Per-query candidate lists as a device CSR pair ``(offsets int64 [Q+1], rows int64 [nnz])`` for ``cos_topk_subset``.
+
+    `rows_per_query` takes the two forms of ``query_exclusion_bits``: Q iterables of local catalog rows, which are
+    deduplicated here, or a CSR pair of int64 tensors, which is validated (offsets[0] = 0, non-decreasing, offsets[Q] =
+    len(rows)) and whose lists must already hold distinct rows. Rows may be in any order; out-of-range rows are kept (the
+    kernel ignores them)."""
+    import numpy as np
+
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    if isinstance(rows_per_query, tuple) and len(rows_per_query) == 2 and all(isinstance(t, torch.Tensor) for t in rows_per_query):
+        offsets, rows = rows_per_query
+        if offsets.dim() != 1 or offsets.numel() < 1 or rows.dim() != 1:
+            raise ValueError("CSR candidate lists must be 1-D offsets [Q+1] and rows tensors")
+        offsets = offsets.to(device=dev, dtype=torch.int64).contiguous()
+        rows = rows.to(device=dev, dtype=torch.int64).contiguous()
+        lens = offsets[1:] - offsets[:-1]
+        if int(offsets[0]) != 0 or int(offsets[-1]) != rows.numel() or bool((lens < 0).any()):
+            raise ValueError("CSR candidate lists need offsets[0] = 0, non-decreasing offsets and offsets[Q] = len(rows)")
+        if rows.numel() > 1:
+            seg = torch.repeat_interleave(torch.arange(lens.numel(), device=dev), lens)
+            o = torch.argsort(rows, stable=True)
+            o = o[torch.argsort(seg[o], stable=True)]
+            rs, ss = rows[o], seg[o]
+            if bool(((rs[1:] == rs[:-1]) & (ss[1:] == ss[:-1])).any()):
+                raise ValueError("a CSR candidate list holds a row twice: the rows of one list must be distinct")
+        return offsets, rows
+    lists = [np.unique(np.asarray(list(r) if not isinstance(r, np.ndarray) else r, dtype=np.int64).reshape(-1)) for r in rows_per_query]
+    off = np.zeros(len(lists) + 1, dtype=np.int64)
+    if lists:
+        np.cumsum([len(r) for r in lists], out=off[1:])
+    flat = np.concatenate(lists) if lists and off[-1] > 0 else np.zeros(0, np.int64)
+    return torch.from_numpy(off).to(dev), torch.from_numpy(flat).to(dev)
+
+
+def cos_topk_subset(
+    queries: torch.Tensor,
+    catalog: torch.Tensor,
+    k: int,
+    rows,
+    *,
+    cat_inv_norms: torch.Tensor | None = None,
+    row_offset: int = 0,
+    out: tuple[torch.Tensor, torch.Tensor] | None = None,
+):
+    """Top-k of each query over its own candidate list: query q ranks only the catalog rows of ``rows[q]``.
+
+    ``rows`` is Q iterables of local rows, or a CSR pair ``(offsets, rows)`` of int64 tensors (``candidate_lists``).
+    Returns (values f32 [Q,k] descending, ids int64 [Q,k] = row + row_offset), ties to the lower row; rows outside [0, N)
+    are ignored, and a list with fewer than k valid rows gets a (-inf, -1) tail. The call reads the listed rows only
+    (``icr_cos_topk_subset``). Scores: fp32 catalogs bit for bit those of ``cos_topk``'s tensor-core path, int8 those of
+    ``cos_topk`` (queries quantised the same way), bf16 / fp16 fp32 arithmetic on the 16-bit values. Missing inverse norms
+    are computed with ``row_inv_norms``; an int8 catalog needs its factors."""
+    _require_cuda("queries", queries)
+    _require_cuda("catalog", catalog)
+    queries, catalog = _rows(_like_catalog(queries, catalog.dtype)), _rows(catalog)
+    if catalog.dtype == torch.int8:
+        if cat_inv_norms is None:
+            raise ValueError("an int8 catalog needs its factors (quantize_rows) as cat_inv_norms")
+        if queries.shape[1] < catalog.shape[1]:
+            queries = _rows(torch.nn.functional.pad(queries, (0, catalog.shape[1] - queries.shape[1])))
+    if queries.shape[1] != catalog.shape[1]:
+        raise ValueError(f"embedding dims differ: {queries.shape[1]} vs {catalog.shape[1]}")
+    if not 1 <= k <= MAX_K:
+        raise ValueError(f"k={k} outside [1, {MAX_K}]")
+    Q, D = queries.shape
+    N = catalog.shape[0]
+    dev = catalog.device
+    offsets, flat = candidate_lists(rows, dev)
+    if offsets.numel() != Q + 1:
+        raise ValueError(f"{offsets.numel() - 1} candidate lists for {Q} queries")
+    if cat_inv_norms is None:
+        cat_inv_norms = row_inv_norms(catalog) if N > 0 else torch.empty(0, dtype=torch.float32, device=dev)
+    if cat_inv_norms.dtype != torch.float32 or cat_inv_norms.shape != (N,) or not cat_inv_norms.is_contiguous():
+        raise ValueError("cat_inv_norms must be the output of row_inv_norms(catalog) (int8: the factors of quantize_rows)")
+    if out is None:
+        vals = torch.empty(Q, k, dtype=torch.float32, device=dev)
+        ids = torch.empty(Q, k, dtype=torch.int64, device=dev)
+    else:
+        vals, ids = out
+    lib = _lib.load()
+    dt = _dtype_code(catalog)
+    nnz = flat.numel()
+    with _on(dev):
+        ws = _workspace(lib.icr_cos_topk_subset_workspace_bytes(Q, nnz, D, dt, k), dev)
+        _lib.check(
+            lib.icr_cos_topk_subset(
+                queries.data_ptr(), Q, _ld(queries), catalog.data_ptr(), N, _ld(catalog), D, dt, _ptr(cat_inv_norms),
+                offsets.data_ptr(), flat.data_ptr() if nnz else None, nnz, k, row_offset, vals.data_ptr(), ids.data_ptr(),
+                ws.data_ptr(), ws.numel(), _stream(dev),
+            )
+        )
+    return vals, ids
+
+
 def peer_exchange_merge(vals: torch.Tensor, ids: torch.Tensor, peer: tuple[int, int, int, int, int]):
     """This rank's [Q,k] candidates (f32 scores, i64 global ids) -> the global top-k of every query on every rank, in ONE kernel
     (``icr_peer_exchange_merge``: NVLink push, flags, wait, merge). ``peer`` as for ``cos_topk``. Collective."""

@@ -224,9 +224,35 @@ class Recommender:
                 break
         return out
 
-    def recommend(self, query: str, top_k: int = 10, exclude_product_ids: set[str] | None = None) -> list[tuple[str, float]]:
-        """Return top-k (product_id, score) sorted by cosine similarity."""
-        return self._rank(self._encode_query(query), top_k, exclude_product_ids)
+    def _rank_candidates(self, query_emb, top_k: int, exclude_product_ids, candidate_product_ids) -> list[tuple[str, float]]:
+        """Equals: sort all rows by score, keep the candidates that are not excluded, keep the first top_k. Only the
+        candidates' rows are read (``DeviceCatalog.topk(..., include_rows=...)``)."""
+        with self._rw.read():
+            if top_k <= 0 or not self.product_ids:
+                return []
+            if top_k > ops.MAX_K:
+                raise ValueError(f"top_k={top_k} exceeds the fused kernel limit {ops.MAX_K} (the reference API caps top_k at 100)")
+            rows = self._candidate_rows(candidate_product_ids, exclude_product_ids)
+            if not rows:
+                return []
+            vals, ids = self.catalog.topk(query_emb, min(top_k, len(rows)), include_rows=[rows])
+            return [(self.product_ids[r], float(s)) for s, r in zip(vals[0].tolist(), ids[0].tolist()) if r >= 0]
+
+    def _candidate_rows(self, candidate_product_ids, exclude_product_ids) -> list[int]:
+        """Catalog rows of the known candidates minus the exclusions, each once."""
+        excluded = set(exclude_product_ids or ())
+        return [self._pid_to_row[p] for p in dict.fromkeys(candidate_product_ids) if p in self._pid_to_row and p not in excluded]
+
+    def recommend(self, query: str, top_k: int = 10, exclude_product_ids: set[str] | None = None, *,
+                  candidate_product_ids=None) -> list[tuple[str, float]]:
+        """Return top-k (product_id, score) sorted by cosine similarity.
+
+        ``candidate_product_ids`` restricts the ranking to those products (a user's previous purchases, the products in
+        stock, one aisle, a candidate set from another stage): the result equals ranking every product and keeping the
+        candidates that are not excluded. Unknown ids are ignored; an empty collection gives []."""
+        if candidate_product_ids is None:
+            return self._rank(self._encode_query(query), top_k, exclude_product_ids)
+        return self._rank_candidates(self._encode_query(query), top_k, exclude_product_ids, candidate_product_ids)
 
     def _encode_queries(self, queries: list[str]):
         if self._query_on_device:
@@ -237,16 +263,22 @@ class Recommender:
         return self.model.encode(queries, normalize_embeddings=True)
 
     def recommend_batch(self, queries: list[str], top_k: int = 10,
-                        exclude_product_ids: list[set[str] | None] | None = None) -> list[list[tuple[str, float]]]:
+                        exclude_product_ids: list[set[str] | None] | None = None, *,
+                        candidate_product_ids: list | None = None) -> list[list[tuple[str, float]]]:
         """``recommend`` for many requests at once: entry i equals ``recommend(queries[i], top_k, exclude_product_ids[i])``.
 
         The queries are encoded in one ``encode`` call and ranked in one fused top-k over the resident catalog, each with
         its own exclusion set applied on the device (``DeviceCatalog.topk(..., exclude_rows=...)``): no per-request
         launches, and no limit on the size of an exclusion set. Unknown product ids are ignored; a request with fewer
-        eligible products than top_k gets a shorter list."""
+        eligible products than top_k gets a shorter list.
+
+        ``candidate_product_ids``: one entry per query, as ``recommend``'s keyword; ``None`` entries rank the whole catalog.
+        The restricted queries run in one candidate-list call, the others in the fused call above."""
         queries = list(queries)
         if exclude_product_ids is not None and len(exclude_product_ids) != len(queries):
             raise ValueError(f"exclude_product_ids has {len(exclude_product_ids)} entries for {len(queries)} queries")
+        if candidate_product_ids is not None:
+            return self._recommend_batch_candidates(queries, top_k, exclude_product_ids, list(candidate_product_ids))
         if not queries:
             return []
         if top_k <= 0 or not self.product_ids:
@@ -263,6 +295,37 @@ class Recommender:
             k = min(top_k, n)
             vals, ids = self.catalog.topk(embs, k, exclude_rows=excluded if any(excluded) else None)
             return [[(self.product_ids[r], float(s)) for s, r in zip(vr, ir) if r >= 0] for vr, ir in zip(vals.tolist(), ids.tolist())]
+
+    def _recommend_batch_candidates(self, queries, top_k, exclude_product_ids, candidates) -> list[list[tuple[str, float]]]:
+        if len(candidates) != len(queries):
+            raise ValueError(f"candidate_product_ids has {len(candidates)} entries for {len(queries)} queries")
+        if not queries:
+            return []
+        if top_k <= 0 or not self.product_ids:
+            return [[] for _ in queries]
+        if top_k > ops.MAX_K:
+            raise ValueError(f"top_k={top_k} exceeds the fused kernel limit {ops.MAX_K} (the reference API caps top_k at 100)")
+        embs = self._encode_queries(queries)
+        exclude = exclude_product_ids or [None] * len(queries)
+        out: list[list[tuple[str, float]]] = [[] for _ in queries]
+        with self._rw.read():
+            n = len(self.product_ids)
+            if n == 0:
+                return out
+            k = min(top_k, n)
+            restricted = [i for i, c in enumerate(candidates) if c is not None]
+            free = [i for i, c in enumerate(candidates) if c is None]
+            if restricted:
+                lists = [self._candidate_rows(candidates[i], exclude[i]) for i in restricted]
+                vals, ids = self.catalog.topk(_pick(embs, restricted), k, include_rows=lists)
+                for i, vr, ir in zip(restricted, vals.tolist(), ids.tolist()):
+                    out[i] = [(self.product_ids[r], float(s)) for s, r in zip(vr, ir) if r >= 0]
+            if free:
+                excluded = [[self._pid_to_row[p] for p in (exclude[i] or ()) if p in self._pid_to_row] for i in free]
+                vals, ids = self.catalog.topk(_pick(embs, free), k, exclude_rows=excluded if any(excluded) else None)
+                for i, vr, ir in zip(free, vals.tolist(), ids.tolist()):
+                    out[i] = [(self.product_ids[r], float(s)) for s, r in zip(vr, ir) if r >= 0]
+        return out
 
     # ---- catalog changes ---------------------------------------------------------------------------------
     def update_products(self, products: dict[str, str]) -> None:
@@ -341,6 +404,11 @@ class Recommender:
         self._pid_to_row = {pid: i for i, pid in enumerate(self.product_ids)}
 
 
+def _pick(embs, idx: list[int]):
+    """Rows `idx` of a batch of query embeddings (an array or tensor, or a list of vectors)."""
+    return embs[idx] if hasattr(embs, "shape") else [embs[i] for i in idx]
+
+
 class MonitoredRecommender(Recommender):
     """Recommender with timing; sets ``last_metrics`` after each ``recommend``."""
 
@@ -350,12 +418,15 @@ class MonitoredRecommender(Recommender):
         self.last_metrics: Optional[RecommendationMetrics] = None
 
     def recommend(self, query: str, top_k: int = 10, user_id: Optional[str] = None,
-                  exclude_product_ids: set[str] | None = None) -> list[tuple[str, float]]:
+                  exclude_product_ids: set[str] | None = None, *, candidate_product_ids=None) -> list[tuple[str, float]]:
         start = time.time()
         query_emb = self._encode_query(query)
         encode_ms = (time.time() - start) * 1000
         sim_start = time.time()
-        results = self._rank(query_emb, top_k, exclude_product_ids)  # includes the host read, so it is complete
+        if candidate_product_ids is None:
+            results = self._rank(query_emb, top_k, exclude_product_ids)  # includes the host read, so it is complete
+        else:
+            results = self._rank_candidates(query_emb, top_k, exclude_product_ids, candidate_product_ids)
         sim_ms = (time.time() - sim_start) * 1000
         total_ms = (time.time() - start) * 1000
         self.last_metrics = RecommendationMetrics(

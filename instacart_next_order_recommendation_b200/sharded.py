@@ -194,13 +194,18 @@ class ShardedCatalog:
         other.exchange, other._peer = exchange, None
         return other
 
-    def local_topk(self, queries, k: int):
-        """[Q,k] candidates of this shard with GLOBAL ids; short shards pad with (-inf, -1)."""
+    def local_topk(self, queries, k: int, include_rows=None):
+        """[Q,k] candidates of this shard with GLOBAL ids; short shards pad with (-inf, -1). ``include_rows``: per-query
+        candidate lists of GLOBAL ids (``topk``); the shard ranks the entries that fall in its block."""
         kk = min(k, self.n_local)
+        local_lists = None if include_rows is None else self._local_lists(include_rows)
         if self._local_topk is not None:
-            vals, ids = self._local_topk(queries, self.local, kk, self.row_offset)
+            if local_lists is None:
+                vals, ids = self._local_topk(queries, self.local, kk, self.row_offset)
+            else:
+                vals, ids = self._local_topk(queries, self.local, kk, self.row_offset, include_rows=local_lists)
         elif kk > 0:
-            vals, ids = self.local.topk(queries, kk)
+            vals, ids = self.local.topk(queries, kk, include_rows=local_lists)
         else:
             Q = queries.shape[0] if hasattr(queries, "shape") and len(queries.shape) == 2 else 1
             vals = torch.empty(Q, 0, dtype=torch.float32, device=self.device)
@@ -211,9 +216,36 @@ class ShardedCatalog:
             ids = torch.cat([ids, torch.full((Q, k - kk), -1, dtype=torch.int64, device=ids.device)], dim=1)
         return vals, ids
 
-    def topk(self, queries, k: int):
-        """Global (values [Q,k'], ids [Q,k']) on every rank, k' = min(k, total rows)."""
+    def _local_lists(self, include_rows):
+        """Global candidate lists -> this shard's local lists (global id - row_offset, ids outside the block dropped): Q
+        arrays for Q iterables, or a CSR pair for a CSR pair."""
+        lo, hi = self.row_offset, self.row_offset + self.n_local
+        if isinstance(include_rows, tuple) and len(include_rows) == 2 and all(isinstance(t, torch.Tensor) for t in include_rows):
+            offsets, rows = (t.to(torch.int64) for t in include_rows)
+            keep = (rows >= lo) & (rows < hi)
+            seg = torch.repeat_interleave(torch.arange(offsets.numel() - 1, device=rows.device), offsets[1:] - offsets[:-1])
+            counts = torch.zeros(offsets.numel() - 1, dtype=torch.int64, device=rows.device).index_add_(0, seg[keep], torch.ones_like(seg[keep]))
+            new_off = torch.zeros_like(offsets)
+            new_off[1:] = torch.cumsum(counts, 0)
+            return new_off, rows[keep] - lo
+        out = []
+        for r in include_rows:
+            g = np.unique(np.asarray(list(r) if not isinstance(r, np.ndarray) else r, dtype=np.int64).reshape(-1))
+            out.append(g[(g >= lo) & (g < hi)] - lo)
+        return out
+
+    def topk(self, queries, k: int, *, include_rows=None):
+        """Global (values [Q,k'], ids [Q,k']) on every rank, k' = min(k, total rows).
+
+        ``include_rows``: one candidate list of GLOBAL ids per query (Q iterables, or an ``(offsets, rows)`` CSR pair with
+        distinct ids per list); query q ranks only its list. Each rank runs the subset search over the ids in its block and
+        the candidates go through the usual exchange. Collective: every rank passes the same lists."""
         k = min(int(k), self.total_rows)
+        if include_rows is not None:
+            if k > ops.MAX_K:
+                raise ValueError(f"k={k} outside [1, {ops.MAX_K}]")
+            vals, ids = self.local_topk(queries, k, include_rows)
+            return self.exchange_merge(vals, ids, k)
         if self.exchange == "peer" and self.world_size > 1 and self._local_topk is None and 1 <= k <= self.n_local:
             # one library call: the shard's search with the exchange and the merge behind it - a single launch for request-sized
             # batches (icr_cos_topk_sharded). Ranks whose shard is shorter than k take the route below; the protocols mix.
